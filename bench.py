@@ -6,6 +6,8 @@
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU arithmetic (oracle port)
     python bench.py --impl library ...                       # the reference's arithmetic as torch library kernels
                                                              # (cuDNN / cuBLAS TF32 + SDPA) on the same B200
+    python bench.py ... --dump-outputs DIR                   # also write the results of the last timed step as
+                                                             # DIR/{emb,dm,mean}.npy (rank 0; inputs are seeded)
 
 One "step" (every N) = one pass of the hot path over one batch per GPU: 256 synthetic 4-second clips -> wav2vec 2.0
 base -> NOMAD embedding -> distance rows + row means against the (M, 256) NMR embeddings resident on every rank
@@ -408,6 +410,7 @@ def run_ours(args):
     n0 = eng.launch_count()
     total_ms = timed(step_dev, args.steps)
     launches = eng.launch_count() - n0
+    dumped = dict(last)  # the last timed step's result tensors (every step allocates new ones)
     e2e_ms = timed(step_host, args.steps)
     # roofline leg: the same K steps again with one CUDA-event pair around every tensor-core GEMM launch (kept out
     # of the `value` region: ~1100 extra event records per 10 steps cost ~5 % of the step)
@@ -491,6 +494,14 @@ def run_ours(args):
         return 0
     sys.stdout.flush()
     os.dup2(saved_stdout, 1)
+
+    if args.dump_outputs:
+        # what a caller of the timed path receives: rank 0's embeddings, and the distance rows + row means of every
+        # rank (256 x 1000 fp32, 256 fp64 per rank)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        dumped["mean"] = dumped["mean"].reshape(-1)  # gathered from N > 1 ranks as an (N * 256, 1) column
+        for name in ("emb", "dm", "mean"):
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), dumped[name].cpu().numpy())
 
     utt_s_per_step = CLIPS * CLIP_SECONDS * world
     ms_per_step = total_ms / args.steps
@@ -580,7 +591,13 @@ def main():
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", type=str, default="ours", choices=["ours", "reference", "library"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the embeddings, distance rows and row means of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     if args.impl == "library":
