@@ -205,6 +205,44 @@ NOMAD_B200_API int64_t nomad_b200_ingest_out_samples(int64_t n_frames, int sr, i
 NOMAD_B200_API int nomad_b200_ingest_pcm16(const int16_t* pcm_dev, int64_t n_frames, int channels, int sr, int target_sr, int trim,
                             float* out_dev, void* stream);
 
+/* Sample formats of the wav files the native reader handles (``torchaudio.load`` decode, nomad.py:196), each decoded to
+ * fp32 exactly as the host path ``nomad_b200.audio.load_wav`` does: U8 (x - 128) / 128; S16 x / 2^15; S24 (packed
+ * 3-byte little-endian) x / 2^23; S32 float32(x) rounded to nearest, then / 2^31; F32 as is; F64 rounded to fp32.  The
+ * container width decides the format (WAVE_FORMAT_EXTENSIBLE's valid-bits field is ignored, as ``wave`` ignores it). */
+#define NOMAD_B200_WAV_U8 1
+#define NOMAD_B200_WAV_S16 2
+#define NOMAD_B200_WAV_S24 3
+#define NOMAD_B200_WAV_S32 4
+#define NOMAD_B200_WAV_F32 5
+#define NOMAD_B200_WAV_F64 6
+
+/* One file of a batched ingest (``load_processing`` of nomad.py:192-212 for n files in one call).  Its raw data bytes
+ * (n_frames x channels interleaved samples of ``format``, as stored in the file) start at src_dev + byte_offset, which
+ * must be aligned to the sample size (1 for U8 and S24).  The first out_samples mono fp32 samples at ``target_sr`` --
+ * mean of the first two channels when channels > 1 (nomad.py:199-200), torchaudio's default Resample when the rates
+ * differ (nomad.py:203-205) -- go to out_dev + out_offset.  out_samples is at most
+ * nomad_b200_ingest_out_samples(n_frames, sample_rate, target_sr, 0); passing
+ * nomad_b200_ingest_out_samples(..., 1) gives the 10 s trim (nomad.py:208-210). */
+typedef struct {
+    int64_t byte_offset;
+    int64_t n_frames;
+    int64_t out_offset;
+    int64_t out_samples;
+    int32_t channels;
+    int32_t format;       /* NOMAD_B200_WAV_* */
+    int32_t sample_rate;
+    int32_t reserved;     /* 0 */
+} nomad_b200_ingest_item;
+
+/* ``load_processing`` for a batch of wav files, still undecoded: src_dev holds the raw data bytes of all of them, items is a
+ * HOST array of n descriptors.  One kernel launch for the items already at target_sr plus one per distinct other
+ * sample rate, whatever n is.  The device copy of the descriptor table lives in the caller's workspace (size from
+ * ``nomad_b200_ingest_workspace_bytes``, 0 = bad descriptors, see ``nomad_b200_last_error``).  S16 items give the
+ * same bits as ``nomad_b200_ingest_pcm16``. */
+NOMAD_B200_API size_t nomad_b200_ingest_workspace_bytes(const nomad_b200_ingest_item* items, int64_t n, int target_sr);
+NOMAD_B200_API int nomad_b200_ingest_batch(const void* src_dev, const nomad_b200_ingest_item* items, int64_t n, int target_sr,
+                                           float* out_dev, void* workspace_dev, size_t workspace_bytes, void* stream);
+
 /* Decode step of ``load_processing`` (``torchaudio.load``, nomad.py:196) for 16-bit PCM RIFF/WAVE files, on `threads` host
  * threads (0 = all cores), no GPU involved.  ``wav_probe`` parses the headers: frames[i] = -1 marks a file that is not
  * plain 16-bit PCM (the caller decodes it some other way).  ``wav_read_pcm16`` then reads n_samples[i] (= frames x channels)
@@ -214,6 +252,18 @@ NOMAD_B200_API int nomad_b200_wav_probe(const char* const* paths, int64_t n, int
                          int64_t* frames, int64_t* data_offset, int threads);
 NOMAD_B200_API int nomad_b200_wav_read_pcm16(const char* const* paths, int64_t n, const int64_t* data_offset,
                               const int64_t* n_samples, const int64_t* dst_offset, int16_t* dst, int threads);
+/* The same for every format above (``torchaudio.load``, nomad.py:196; decoded on the device by
+ * ``nomad_b200_ingest_batch``).  ``wav_probe_format`` accepts format tag 1 (PCM, 8/16/24/32 bits), tag 3 (IEEE float,
+ * 32/64 bits) and WAVE_FORMAT_EXTENSIBLE with the full PCM or IEEE_FLOAT sub-format GUID, with block_align = channels x
+ * sample bytes; format[i] = NOMAD_B200_WAV_*, or frames[i] = -1 and format[i] = 0 for anything else (u-law, A-law,
+ * ADPCM, RIFX, a ``data`` chunk before ``fmt ``, unreadable files).  frames counts the whole frames present (a truncated
+ * ``data`` chunk is cut at the end of the file).  ``wav_probe`` / ``wav_read_pcm16`` above are this parser and reader
+ * restricted to S16.  ``wav_read`` reads n_bytes[i] bytes of file i from byte src_offset[i] to (char*)dst +
+ * dst_offset[i]. */
+NOMAD_B200_API int nomad_b200_wav_probe_format(const char* const* paths, int64_t n, int32_t* sample_rate, int32_t* channels,
+                                               int64_t* frames, int64_t* data_offset, int32_t* format, int threads);
+NOMAD_B200_API int nomad_b200_wav_read(const char* const* paths, int64_t n, const int64_t* src_offset, const int64_t* n_bytes,
+                                       const int64_t* dst_offset, void* dst, int threads);
 
 /* The attention core of one encoder layer, softmax(Q K^T) V per (utterance, head) (fairseq
  * MultiheadAttention inside TransformerSentenceEncoderLayer; mirror torchaudio components.py:237-330).

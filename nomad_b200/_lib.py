@@ -7,12 +7,24 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+from typing import NamedTuple
+
+import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("NOMAD_B200_LIB") or os.path.join(_HERE, "csrc", "libnomad_b200.so")  # override: kernel A/B probes
 
 c_i64 = C.c_int64
 c_vp = C.c_void_p
+
+
+# NOMAD_B200_WAV_* sample formats -> bytes per sample
+WAV_U8, WAV_S16, WAV_S24, WAV_S32, WAV_F32, WAV_F64 = 1, 2, 3, 4, 5, 6
+FORMAT_BYTES = np.array([0, 1, 2, 3, 4, 4, 8], np.int64)
+
+# ``nomad_b200_ingest_item``
+INGEST_ITEM = np.dtype([("byte_offset", "<i8"), ("n_frames", "<i8"), ("out_offset", "<i8"), ("out_samples", "<i8"),
+                        ("channels", "<i4"), ("format", "<i4"), ("sample_rate", "<i4"), ("reserved", "<i4")])
 
 
 class Tensor(C.Structure):
@@ -68,6 +80,10 @@ PROTOTYPES = {
     "nomad_b200_ingest_pcm16": (C.c_int, [c_vp, c_i64, C.c_int, C.c_int, C.c_int, C.c_int, c_vp, c_vp]),
     "nomad_b200_wav_probe": (C.c_int, [C.POINTER(C.c_char_p), c_i64, c_vp, c_vp, c_vp, c_vp, C.c_int]),
     "nomad_b200_wav_read_pcm16": (C.c_int, [C.POINTER(C.c_char_p), c_i64, c_vp, c_vp, c_vp, c_vp, C.c_int]),
+    "nomad_b200_wav_probe_format": (C.c_int, [C.POINTER(C.c_char_p), c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, C.c_int]),
+    "nomad_b200_wav_read": (C.c_int, [C.POINTER(C.c_char_p), c_i64, c_vp, c_vp, c_vp, c_vp, C.c_int]),
+    "nomad_b200_ingest_workspace_bytes": (C.c_size_t, [c_vp, c_i64, C.c_int]),
+    "nomad_b200_ingest_batch": (C.c_int, [c_vp, c_vp, c_i64, C.c_int, c_vp, c_vp, C.c_size_t, c_vp]),
     "nomad_b200_attention_workspace_bytes": (C.c_size_t, [C.POINTER(C.c_int32), C.c_int]),
     "nomad_b200_attention_f16": (C.c_int, [c_vp, c_i64, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.c_int, c_vp, c_vp,
                                             c_vp, C.c_size_t, c_vp]),
@@ -133,6 +149,53 @@ def wav_probe(paths, threads=0):
     check(load().nomad_b200_wav_probe(arr, n, sr.ctypes.data_as(c_vp), ch.ctypes.data_as(c_vp), fr.ctypes.data_as(c_vp),
                                      off.ctypes.data_as(c_vp), int(threads)), "nomad_b200_wav_probe")
     return sr, ch, fr, off
+
+
+class WavProbe(NamedTuple):
+    """Per-file header fields from ``nomad_b200_wav_probe_format``; frames = -1 (format 0): not read natively."""
+    sample_rate: np.ndarray   # int32
+    channels: np.ndarray      # int32
+    frames: np.ndarray        # int64
+    data_offset: np.ndarray   # int64
+    format: np.ndarray        # int32, WAV_*
+
+    def take(self, idx) -> "WavProbe":
+        return WavProbe(*(a[idx] for a in self))
+
+    @staticmethod
+    def unread(n: int) -> "WavProbe":
+        """n files left to the host decoder"""
+        return WavProbe(np.zeros(n, np.int32), np.zeros(n, np.int32), np.full(n, -1, np.int64), np.zeros(n, np.int64),
+                        np.zeros(n, np.int32))
+
+
+def wav_probe_format(paths, threads=0) -> WavProbe:
+    n = len(paths)
+    arr = (C.c_char_p * max(n, 1))(*[str(p).encode("utf-8") for p in paths])
+    p = WavProbe.unread(n)
+    check(load().nomad_b200_wav_probe_format(arr, n, *(a.ctypes.data_as(c_vp) for a in p), int(threads)),
+          "nomad_b200_wav_probe_format")
+    return p
+
+
+def ingest_out_samples(frames, sample_rate, target_sr=16000, trim=False) -> np.ndarray:
+    """``nomad_b200_ingest_out_samples`` per file (-1 where frames < 0)."""
+    frames = np.asarray(frames, np.int64)
+    sample_rate = np.asarray(sample_rate, np.int64)
+    out = np.where(frames >= 0, frames, -1)
+    f = load().nomad_b200_ingest_out_samples
+    for i in np.flatnonzero((frames >= 0) & ((sample_rate != target_sr) | bool(trim))):
+        out[i] = f(int(frames[i]), int(sample_rate[i]), int(target_sr), int(bool(trim)))
+    return out
+
+
+def wav_read(paths, src_offset, n_bytes, dst_offset, dst_ptr, threads=0):
+    """Read n_bytes[i] bytes of file i from byte src_offset[i] to (char*) dst_ptr + dst_offset[i] with host threads."""
+    n = len(paths)
+    arr = (C.c_char_p * max(n, 1))(*[str(p).encode("utf-8") for p in paths])
+    a = [np.ascontiguousarray(x, dtype=np.int64) for x in (src_offset, n_bytes, dst_offset)]
+    check(load().nomad_b200_wav_read(arr, n, *(x.ctypes.data_as(c_vp) for x in a), c_vp(dst_ptr), int(threads)),
+          "nomad_b200_wav_read")
 
 
 def wav_read_pcm16(paths, data_offset, n_samples, dst_offset, dst_ptr, threads=0):

@@ -51,30 +51,21 @@ def load_wav(filepath: str):
         return torchaudio.load(filepath)
 
 
-def read_pcm16(filepath: str):
-    """-> ((n_frames, channels) int16 array, sample_rate) for a 16-bit PCM wav, else None."""
-    try:
-        with wave.open(str(filepath), "rb") as w:
-            if w.getsampwidth() != 2:
-                return None
-            ch, sr, n = w.getnchannels(), w.getframerate(), w.getnframes()
-            raw = w.readframes(n)
-        return np.frombuffer(raw, dtype="<i2").reshape(-1, ch), sr
-    except (wave.Error, EOFError):
-        return None
-
-
 def load_processing_device(engine, filepath, target_sr: int = 16000, trim: bool = False) -> torch.Tensor:
-    """``load_processing`` with the sample conversion, channel mix, resampling and trim on the GPU
-    (``nomad_b200_ingest_pcm16``) for 16-bit PCM wavs -- the 16-bit samples are what crosses PCIe; any other file
-    takes the host path below and is moved to the device.  Returns a (1, N) fp32 CUDA tensor."""
+    """``load_processing`` with the sample decode, channel mix, resampling and trim on the GPU
+    (``Engine.ingest_wav_files``) for every wav file the native reader handles (PCM of 8, 16, 24 or 32 bits, float of
+    32 or 64 bits) -- the file's own data bytes are what crosses PCIe; any other file takes the host path below and is
+    moved to the device.  Returns a (1, N) fp32 CUDA tensor."""
+    from . import _lib
     if isinstance(filepath, np.ndarray):
         filepath = filepath[0]
-    got = read_pcm16(filepath)
-    if got is None:
+    probe = _lib.wav_probe_format([str(filepath)], 1)
+    if probe.frames[0] < 0:
         return load_processing(filepath, target_sr, trim).to(engine.device)
-    pcm, sr = got
-    return engine.ingest_pcm16(pcm, sr, target_sr, trim)
+    n_out = _lib.ingest_out_samples(probe.frames, probe.sample_rate, target_sr, trim)
+    out = torch.empty((1, int(n_out[0])), dtype=torch.float32, device=engine.device)
+    engine.ingest_wav_files([str(filepath)], probe, n_out, out, np.zeros(1, np.int64), 1, target_sr)
+    return out
 
 
 def load_processing(filepath, target_sr: int = 16000, trim: bool = False) -> torch.Tensor:

@@ -210,6 +210,15 @@ def init_from_env(backend: Optional[str] = None):
     return rank, world, local
 
 
+def shard_costs(files, threads: int = 0) -> List[float]:
+    """Work estimate per file for ``shard_by_cost``: the 16 kHz output length for a wav file the native reader handles
+    (the embedding's cost does not depend on the file's encoding), the size in bytes for any other file."""
+    from . import _lib
+    probe = _lib.wav_probe_format(files, threads)
+    n_out = _lib.ingest_out_samples(probe.frames, probe.sample_rate)
+    return [float(n) if n >= 0 else float(os.path.getsize(f)) for f, n in zip(files, n_out)]
+
+
 # above this many matrix bytes the rows stay with the ranks and are written as row-sharded files
 ROOT_MATRIX_LIMIT_BYTES = 8 << 30
 
@@ -244,7 +253,7 @@ def predict_sharded(nomad, mode: str, nmr: str, deg: str, results_path: Optional
 
     # windowed, length-bucketed, device-ingest loader of Nomad.get_embeddings_csv, on this rank's files only
     embed_files = lambda files: (lambda idx: nomad.embed_files([files[i] for i in idx]))
-    cost = lambda files: [float(os.path.getsize(f)) for f in files]
+    cost = lambda files: shard_costs(files, nomad.reader_threads)
     res = score_sharded(cost(nmr_files), embed_files(nmr_files), cost(deg_files), embed_files(deg_files),
                         lambda a, b, wm: nomad.engine.cdist_mean(a, b, wm), device, group, matrix)
     if matrix == "local":

@@ -230,42 +230,54 @@ class Engine:
         ev.record(torch.cuda.current_stream())
         self._ring_ev[self._ring_i] = ev
 
-    def embed_pcm16_mono(self, pcms: Sequence[np.ndarray], out: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """A batch of 16 kHz MONO 16-bit PCM utterances (1-D int16 arrays): packed into ONE pinned buffer, ONE H2D copy
-        of the 16-bit samples, ONE conversion launch (``nomad_b200_ingest_pcm16`` over the concatenation: the
-        conversion is per sample) and one ``nomad_b200_embed`` -- instead of a copy + a launch per file."""
-        lens = [int(p.shape[0]) for p in pcms]
-        total = sum(lens)
-        stage = self.pinned(2 * total)
-        host = stage[: 2 * total].view(torch.int16).numpy()
-        o = 0
-        for p, n in zip(pcms, lens):
-            host[o:o + n] = p
-            o += n
-        dev = stage[: 2 * total].view(torch.int16).to(self.device, non_blocking=True)
+    def ingest_wav_files(self, paths, probe: "_lib.WavProbe", n_out, out: torch.Tensor, out_offset, threads: int = 0,
+                         target_sr: int = 16000):
+        """``load_processing`` on the device for wav files the native reader handles (``probe.frames >= 0``): their data
+        bytes are read by the library's host threads into the pinned staging ring (each file at a 16-byte aligned
+        offset), cross PCIe in ONE copy and are decoded, mixed and resampled by ONE ``nomad_b200_ingest_batch`` call
+        (one launch per source rate) into ``out[out_offset[i]:][:n_out[i]]`` (fp32 CUDA).  Nothing synchronises."""
+        n_bytes = probe.frames * probe.channels * _lib.FORMAT_BYTES[probe.format]
+        staged = (n_bytes + 15) // 16 * 16
+        dst = np.zeros(len(paths), np.int64)
+        np.cumsum(staged[:-1], out=dst[1:])
+        total = int(staged.sum())
+        stage = self.pinned(total)
+        _lib.wav_read(paths, probe.data_offset, n_bytes, dst, stage.data_ptr(), threads)
+        src = stage[:total].to(self.device, non_blocking=True)
         self.pinned_release()
-        wav = torch.empty((total,), dtype=torch.float32, device=self.device)
+        items = np.zeros(len(paths), _lib.INGEST_ITEM)
+        items["byte_offset"], items["n_frames"], items["out_offset"], items["out_samples"] = dst, probe.frames, out_offset, n_out
+        items["channels"], items["format"], items["sample_rate"] = probe.channels, probe.format, probe.sample_rate
+        ip = items.ctypes.data_as(C.c_void_p)
+        need = self.lib.nomad_b200_ingest_workspace_bytes(ip, len(items), int(target_sr))
+        if need == 0:
+            raise _lib.NomadB200Error(self.lib.nomad_b200_last_error().decode())
+        wp, wbytes = self._aligned(self.workspace(need))
+        assert out.is_cuda and out.dtype == torch.float32 and out.is_contiguous()
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.nomad_b200_ingest_pcm16(_ptr(dev), total, 1, 16000, 16000, 0, _ptr(wav), _stream_ptr()),
-                       "nomad_b200_ingest_pcm16")
-        return self.embed_packed(wav, self.offsets(lens), out)
+            _lib.check(self.lib.nomad_b200_ingest_batch(_ptr(src), ip, len(items), int(target_sr), _ptr(out), wp, wbytes,
+                                                        _stream_ptr()), "nomad_b200_ingest_batch")
 
-    def embed_pcm16_mono_files(self, paths, data_offset, frames, threads: int = 0, out: Optional[torch.Tensor] = None):
-        """Same as :meth:`embed_pcm16_mono` with the samples read straight from 16 kHz mono 16-bit wav files into the pinned
-        staging buffer by the library's host threads (``nomad_b200_wav_read_pcm16``): no per-file Python work."""
-        lens = [int(n) for n in frames]
-        total = sum(lens)
-        stage = self.pinned(2 * total)
-        dst = np.zeros(len(lens), dtype=np.int64)
-        np.cumsum(lens[:-1], out=dst[1:])
-        _lib.wav_read_pcm16(paths, data_offset, lens, dst, stage.data_ptr(), threads)
-        dev = stage[: 2 * total].view(torch.int16).to(self.device, non_blocking=True)
-        self.pinned_release()
-        wav = torch.empty((total,), dtype=torch.float32, device=self.device)
-        with torch.cuda.device(self.device):
-            _lib.check(self.lib.nomad_b200_ingest_pcm16(_ptr(dev), total, 1, 16000, 16000, 0, _ptr(wav), _stream_ptr()),
-                       "nomad_b200_ingest_pcm16")
-        return self.embed_packed(wav, self.offsets(lens), out)
+    def embed_wav_files(self, paths, probe: "_lib.WavProbe", threads: int = 0, out: Optional[torch.Tensor] = None,
+                        waves=None) -> torch.Tensor:
+        """Embed one batch of wav files (``load_processing`` + ``model`` of nomad.py:172-186) -> (B, 256) CUDA tensor.
+        Files with ``probe.frames >= 0`` go through :meth:`ingest_wav_files`; the others must come decoded in ``waves``
+        ({position in ``paths``: 1-D or (1, N) fp32 tensor at 16 kHz}) and are copied into the same packed buffer, so
+        the whole batch is one ``nomad_b200_embed`` call."""
+        waves = waves or {}
+        native = np.flatnonzero(probe.frames >= 0)
+        lens = np.zeros(len(paths), np.int64)
+        lens[native] = _lib.ingest_out_samples(probe.frames[native], probe.sample_rate[native])
+        for i, w in waves.items():
+            lens[i] = w.numel()
+        offsets = self.offsets(lens)
+        wav = torch.empty((int(offsets[-1]),), dtype=torch.float32, device=self.device)
+        if len(native):
+            self.ingest_wav_files([paths[i] for i in native], probe.take(native), lens[native], wav, offsets[native],
+                                  threads)
+        for i, w in waves.items():
+            wav[offsets[i]:offsets[i + 1]].copy_(w.reshape(-1), non_blocking=True)
+        return self.embed_packed(wav, offsets, out)
 
     # ------------------------------------------------------------------ ingest
     def ingest_pcm16(self, pcm: np.ndarray, sr: int, target_sr: int = 16000, trim: bool = False) -> torch.Tensor:

@@ -294,29 +294,18 @@ class Nomad():
             out[torch.as_tensor(idx, device=self.engine.device)] = emb
         return out.cpu().numpy()
 
-    def _read_for_embed(self, filepath):
-        """One file of the per-file loop -> ("pcm", int16 (n,)) for the common case (16-bit PCM, mono, 16 kHz: the
-        samples cross PCIe as 16-bit and are converted on the GPU in one launch per batch) or ("wav", (1, N) tensor)."""
-        if isinstance(filepath, np.ndarray):
-            filepath = filepath[0]  # nomad.py:194-195: a DataFrame row
-        if self.device_ingest:
-            got = audio.read_pcm16(filepath)
-            if got is not None:
-                pcm, sr = got
-                if sr == 16000 and pcm.shape[1] == 1:
-                    return "pcm", pcm[:, 0]
-                return "dev", (pcm, sr)   # other rates / stereo: per-file device ingest (mix + resample on the GPU)
-        return "wav", self.load_processing(filepath, trim=False)
-
     def embed_files(self, filepaths: Sequence, root=False) -> torch.Tensor:
         """The reference's per-file loop (``nomad.py:172-186``) restructured for throughput -> (n, 256) CUDA tensor in
         input order.  Files are handled in windows of ``self.window_files`` (bounded memory for 100 k-file corpora).
-        Per window the headers of all files are parsed by the library's host threads (``nomad_b200_wav_probe``); 16 kHz
-        mono 16-bit PCM files -- the common corpus format -- are then read batch by batch straight into a pinned
-        staging buffer (``nomad_b200_wav_read_pcm16``), cross PCIe as 16-bit samples in ONE copy per batch and are
-        converted on the GPU in one launch; everything else takes the per-file path (device resampling for other PCM16
-        wavs, ``load_processing`` for other formats).  Nothing synchronises per batch: the GPU works on batch k while
-        the host reads batch k + 1 (the returned tensor may still be being computed)."""
+        Per window the headers of all files are parsed by the library's host threads (``nomad_b200_wav_probe_format``).
+        Every wav file the native reader handles -- PCM of 8, 16, 24 or 32 bits or float of 32 or 64 bits, any sample
+        rate and channel count -- is then read batch by batch straight into a pinned staging buffer, crosses PCIe as
+        the file's own bytes in ONE copy per batch and is decoded, mixed to mono and resampled to 16 kHz on the GPU
+        (``nomad_b200_ingest_batch``: one launch per batch plus one per distinct other sample rate).  Other files
+        (u-law, A-law, RIFX, non-wav containers) are decoded on the host by ``load_processing`` and packed into the
+        same batch.  Batches are planned on 16 kHz lengths.  ``NOMAD_B200_DEVICE_INGEST=0`` decodes every file on the
+        host.  Nothing synchronises per batch: the GPU works on batch k while the host reads batch k + 1 (the returned
+        tensor may still be being computed)."""
         from concurrent.futures import ThreadPoolExecutor
 
         from . import _lib
@@ -331,39 +320,24 @@ class Nomad():
                     paths.append(os.path.join(root, filename_anchor) if root else filename_anchor)
                 paths = [str(p) for p in paths]
                 if self.device_ingest:
-                    sr, ch, frames, data_off = _lib.wav_probe(paths, self.reader_threads)
-                    fast = (frames >= 0) & (sr == 16000) & (ch == 1)
+                    probe = _lib.wav_probe_format(paths, self.reader_threads)
                 else:
-                    frames = np.full(len(paths), -1, np.int64)
-                    data_off = np.zeros(len(paths), np.int64)
-                    fast = np.zeros(len(paths), bool)
-                slow_idx = [i for i in range(len(paths)) if not fast[i]]
-                items = dict(zip(slow_idx, pool.map(self._read_for_embed, [paths[i] for i in slow_idx])))
-                lengths = []
-                for k in range(len(paths)):
-                    if fast[k]:
-                        n = int(frames[k])
-                    else:
-                        kind, v = items[k]
-                        if kind == "dev":   # 16-bit PCM at another rate / stereo: mix + resample on the GPU, per file
-                            items[k] = (kind, v) = ("wav", self.engine.ingest_pcm16(v[0], v[1], 16000, False))
-                        n = int(v.shape[-1]) if kind == "wav" else int(v.shape[0])
+                    probe = _lib.WavProbe.unread(len(paths))
+                lengths = _lib.ingest_out_samples(probe.frames, probe.sample_rate)
+                host_idx = np.flatnonzero(probe.frames < 0)
+                waves = dict(zip(host_idx.tolist(), pool.map(self.load_processing, [paths[i] for i in host_idx])))
+                for k, w in waves.items():
+                    lengths[k] = w.shape[-1]
+                for n in lengths:
                     if n < MIN_SAMPLES:
                         raise RuntimeError(f"Calculated padded input size per channel: ({n}). Kernel size: (10). "
                                            "Kernel size can't be greater than actual input size")
-                    lengths.append(n)
                 dev_out = torch.empty((len(paths), EMB_DIM), dtype=torch.float32, device=self.engine.device)
                 for idx in plan_batches(lengths, self.max_batch_samples):
                     sel = torch.as_tensor(idx, device=self.engine.device)
-                    if all(fast[i] for i in idx):
-                        dev_out[sel] = self.engine.embed_pcm16_mono_files([paths[i] for i in idx], data_off[idx], frames[idx],
-                                                                          self.reader_threads)
-                        continue
-                    waves = []
-                    for i in idx:   # mixed batch (rare): the fast files take the per-file path too
-                        kind, v = items[i] if i in items else self._read_for_embed(paths[i])
-                        waves.append(v.reshape(-1) if kind == "wav" else torch.from_numpy(v.astype(np.float32) / 32768.0))
-                    dev_out[sel] = self.engine.embed(waves)
+                    pos = {i: j for j, i in enumerate(idx)}
+                    dev_out[sel] = self.engine.embed_wav_files([paths[i] for i in idx], probe.take(idx), self.reader_threads,
+                                                               waves={pos[i]: waves[i] for i in idx if i in waves})
                 parts.append(dev_out)  # still being computed; the host goes on with the next window
         if not parts:
             return torch.zeros((0, EMB_DIM), dtype=torch.float32, device=self.engine.device)
