@@ -115,6 +115,29 @@ NOMAD_B200_API int64_t nomad_b200_num_frames(int64_t n_samples);
 NOMAD_B200_API int nomad_b200_layers_fwd(nomad_b200_handle* h, const float* wav_dev, int B, int64_t N, float* layers_dev,
                           float* emb_dev, void* workspace_dev, size_t workspace_bytes, void* stream);
 
+/* ---- autograd through ``LossNetLayers`` / ``TripletModel`` (nomad.py:224-258 are plain nn.Modules) ------------------
+ * Save-mode forward of the network for B utterances of N samples (fp16 operands, like the loss path).  Writes the 12
+ * post-LayerNorm layer outputs (12 x B x T x 768 fp32, layer major, may be NULL) and the head output (B x 256, may be
+ * NULL).  head: 0 = the NOMAD head (TripletModel), 1 = the loss head set by nomad_b200_set_loss_head (LossNetLayers).
+ * Everything the backward needs goes into ``saved`` (caller-owned, 1024-byte aligned, nomad_b200_layers_saved_bytes
+ * bytes, alive and untouched until the last backward that uses it): the save-mode activations, the pooled features and
+ * a snapshot of the chosen head, so a later nomad_b200_set_loss_head does not change the backward. */
+NOMAD_B200_API size_t nomad_b200_layers_saved_bytes(int B, int64_t N);
+NOMAD_B200_API int nomad_b200_layers_fwd_save(nomad_b200_handle* h, const float* wav_dev, int B, int64_t N, int head,
+                                              float* layers_dev, float* emb_dev, void* saved_dev, size_t saved_bytes,
+                                              void* stream);
+/* d_wav = d(<g_layers, layers> + <g_emb, emb>) / d wav (B x N fp32 device), with fairseq's
+ * GradMultiply(feature_grad_mult) on the conv features.  g_layers: HOST array of 12 device pointers (B x T x 768 fp32
+ * each, 16-byte aligned, NULL = zero gradient) or NULL; g_emb: B x 256 fp32 device or NULL.  ``saved`` comes from
+ * nomad_b200_layers_fwd_save with the same B and N, wav_dev is the waveform given to it.  The power-of-two scale that
+ * keeps the 16-bit gradients in range is chosen on the device from max|g|.  The saved buffer is only read: one forward
+ * may be differentiated more than once.  No weight gradients; no host synchronisation. */
+NOMAD_B200_API size_t nomad_b200_layers_bwd_workspace_bytes(int B, int64_t N);
+NOMAD_B200_API int nomad_b200_layers_bwd(nomad_b200_handle* h, const void* saved_dev, size_t saved_bytes, const float* wav_dev,
+                                         int B, int64_t N, const float* const* g_layers, const float* g_emb,
+                                         float feature_grad_mult, float* d_wav_dev, void* workspace_dev,
+                                         size_t workspace_bytes, void* stream);
+
 /* ---- distance: ``cdist(test, nmr)`` + ``np.mean(axis=1)`` (nomad.py:108,111) ---------------------
  * deg: n x 256, nmr: m x 256 fp32 device.  dm (n x m fp32 device, may be NULL when only the means are
  * wanted) and row_mean (n fp64 device; NaN when m == 0, like np.mean of an empty row).  Row means are summed in a

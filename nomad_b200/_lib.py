@@ -54,6 +54,11 @@ PROTOTYPES = {
     "nomad_b200_layers_workspace_bytes": (C.c_size_t, [C.c_int, c_i64]),
     "nomad_b200_num_frames": (c_i64, [c_i64]),
     "nomad_b200_layers_fwd": (C.c_int, [c_vp, c_vp, C.c_int, c_i64, c_vp, c_vp, c_vp, C.c_size_t, c_vp]),
+    "nomad_b200_layers_saved_bytes": (C.c_size_t, [C.c_int, c_i64]),
+    "nomad_b200_layers_fwd_save": (C.c_int, [c_vp, c_vp, C.c_int, c_i64, C.c_int, c_vp, c_vp, c_vp, C.c_size_t, c_vp]),
+    "nomad_b200_layers_bwd_workspace_bytes": (C.c_size_t, [C.c_int, c_i64]),
+    "nomad_b200_layers_bwd": (C.c_int, [c_vp, c_vp, C.c_size_t, c_vp, C.c_int, c_i64, C.POINTER(c_vp), c_vp, C.c_float, c_vp,
+                                        c_vp, C.c_size_t, c_vp]),
     "nomad_b200_cdist_workspace_bytes": (C.c_size_t, [c_i64, c_i64]),
     "nomad_b200_cdist_mean": (C.c_int, [c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, C.c_size_t, C.c_int, c_vp]),
     "nomad_b200_cdist_mean_host": (C.c_int, [c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, C.c_size_t, c_vp]),

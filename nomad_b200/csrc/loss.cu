@@ -158,6 +158,129 @@ __global__ void __launch_bounds__(256) ln768_bwd_kernel(const float* __restrict_
     store_row768(out, g_out ? g_out + f * EMBED : nullptr, g_out_h ? g_out_h + f * EMBED : nullptr, lane);
 }
 
+// The same backward with caller-given upstream gradients (nomad_b200_layers_bwd): g_user is the gradient wrt this
+// layer's output in the caller's (B, T, 768) layout (row b * user_T + t, may be null); S is read from the device.
+//   g = g_in + S * g_user[b, t] + S * g_pool[utt]
+__global__ void __launch_bounds__(256) ln768_bwd_user_kernel(const float* __restrict__ g_in, const float* __restrict__ pre,
+                                                             const UttMeta* __restrict__ meta, int B, long long frames,
+                                                             const float* __restrict__ gam, const float* __restrict__ g_user,
+                                                             int user_T, const float* __restrict__ g_pool,
+                                                             const float* __restrict__ scale, float* __restrict__ g_out,
+                                                             op_t* __restrict__ g_out_h) {
+    const long long f = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
+    if (f >= frames) return;
+    const int lane = threadIdx.x & 31;
+    const int b = find_utt_by_frame(meta, B, (int)f);
+    const int t = (int)f - meta[b].frame0;
+    Row768f out;
+    if (t >= meta[b].T) {
+#pragma unroll
+        for (int i = 0; i < 24; ++i) out.v[i] = 0.f;
+        store_row768(out, g_out + f * EMBED, g_out_h + f * EMBED, lane);
+        return;
+    }
+    const float S = __ldg(scale);
+    Row768f xh, gg, g;
+    load_row768(xh, pre + f * EMBED, lane);
+    load_vec768(gg, gam, lane);
+    const float rstd = normalise768(xh);
+    if (g_in != nullptr) {
+        load_row768(g, g_in + f * EMBED, lane);
+    } else {
+#pragma unroll
+        for (int i = 0; i < 24; ++i) g.v[i] = 0.f;
+    }
+    if (g_user != nullptr) {
+        Row768f gu;
+        load_row768(gu, g_user + ((long long)b * user_T + t) * EMBED, lane);
+#pragma unroll
+        for (int i = 0; i < 24; ++i) g.v[i] = fmaf(S, gu.v[i], g.v[i]);
+    }
+    if (g_pool != nullptr) {
+        Row768f gp;
+        load_vec768(gp, g_pool + (long long)b * EMBED, lane);
+#pragma unroll
+        for (int i = 0; i < 24; ++i) g.v[i] = fmaf(S, gp.v[i], g.v[i]);
+    }
+    float s1 = 0.f, s2 = 0.f;
+#pragma unroll
+    for (int i = 0; i < 24; ++i) {
+        g.v[i] *= gg.v[i];
+        s1 += g.v[i];
+        s2 = fmaf(g.v[i], xh.v[i], s2);
+    }
+    s1 = warp_sum(s1) * (1.0f / EMBED);
+    s2 = warp_sum(s2) * (1.0f / EMBED);
+#pragma unroll
+    for (int i = 0; i < 24; ++i) out.v[i] = rstd * (g.v[i] - s1 - xh.v[i] * s2);
+    store_row768(out, g_out + f * EMBED, g_out_h + f * EMBED, lane);
+}
+
+// Power-of-two gradient scale of the autograd backward, chosen on the device: S with max|g| * S in [1, 2) over every
+// upstream gradient given (S = 1 when they are all zero or not finite).  state[0] = running max as float bits (|g| >= 0
+// orders like its bits), state[1] = finished blocks; both zeroed by the caller.  The last block writes S.
+struct ScaleSources {
+    const float* p[LAYERS + 1];
+    long long n[LAYERS + 1];
+};
+__global__ void __launch_bounds__(256) grad_scale_kernel(ScaleSources src, unsigned* __restrict__ state, float* __restrict__ scale) {
+    unsigned m = 0;
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    for (int a = 0; a < LAYERS + 1; ++a) {
+        const float* p = src.p[a];
+        if (p == nullptr) continue;
+        for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < src.n[a]; i += stride)
+            m = max(m, __float_as_uint(fabsf(__ldg(p + i))));
+    }
+    m = __reduce_max_sync(0xffffffffu, m);
+    __shared__ unsigned red[8];
+    __shared__ bool last;
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = m;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        for (int w = 1; w < 8; ++w) m = max(m, red[w]);
+        atomicMax(state, m);
+        __threadfence();
+        last = atomicAdd(state + 1, 1u) == gridDim.x - 1;
+    }
+    __syncthreads();
+    if (last && threadIdx.x == 0) {
+        const float mx = __uint_as_float(atomicMax(state, 0u));
+        float S = 1.f;
+        if (mx > 0.f && mx <= 3.402823466e38f) S = ldexpf(1.f, min(max(-ilogbf(mx), -126), 127));
+        *scale = S;
+    }
+}
+
+// Head backward from an explicit upstream gradient g_emb of e = normalize(W relu(pooled) + b) (the forward's snapshot of
+// the head): gy[b] = d<g_emb, e> / d y, unscaled.  y is recomputed in the forward kernel's order.
+__global__ void __launch_bounds__(256) head_emb_bwd_kernel(const float* __restrict__ pooled, const float* __restrict__ head_wt,
+                                                           const float* __restrict__ head_b, const float* __restrict__ g_emb,
+                                                           float* __restrict__ gy) {
+    const int b = blockIdx.x, tid = threadIdx.x;
+    __shared__ float pr[EMBED];
+    __shared__ float red[2][8];
+    for (int k = tid; k < EMBED; k += 256) pr[k] = fmaxf(pooled[(long long)b * EMBED + k], 0.f);
+    __syncthreads();
+    float y = head_b[tid];
+    for (int k = 0; k < EMBED; ++k) y = fmaf(pr[k], __ldg(head_wt + k * EMB + tid), y);
+    const float sq = warp_sum(y * y);
+    if ((tid & 31) == 0) red[0][tid >> 5] = sq;
+    __syncthreads();
+    float n = 0.f;
+#pragma unroll
+    for (int w = 0; w < 8; ++w) n += red[0][w];
+    n = fmaxf(sqrtf(n), 1e-12f);
+    const float e = y / n, ge = g_emb[(long long)b * EMB + tid];
+    const float dp = warp_sum(ge * e);
+    if ((tid & 31) == 0) red[1][tid >> 5] = dp;
+    __syncthreads();
+    float dot = 0.f;
+#pragma unroll
+    for (int w = 0; w < 8; ++w) dot += red[1][w];
+    gy[(long long)b * EMB + tid] = (ge - e * dot) / n;  // backward of y / max(||y||, eps)
+}
+
 // ---------------------------------------------------------------------------------------------
 // Head term: e = normalize(W relu(pooled) + b) for both halves; acc += sum |e_est - e_clean|;
 // g_pool[b][k] = d(term) / d x[t, k] for every valid frame t of estimate b (already divided by T).
@@ -431,10 +554,12 @@ __global__ void __launch_bounds__(128) conv0_bwd_consts_kernel(const double* __r
     consts[(long long)b * 112 + tid] = (float)a;
 }
 
-// Overlap-add of the 10 taps (stride 5) into the waveform gradient, times out_scale (= 1 / S).
+// Overlap-add of the 10 taps (stride 5) into the waveform gradient, times out_scale (= 1 / S), or times 1 / *scale_dev
+// when the scale was chosen on the device (scale_dev non-null).
 __global__ void __launch_bounds__(256) conv0_bwd_finish_kernel(const float* __restrict__ V, const float* __restrict__ wav,
                                                                const UttMeta* __restrict__ meta, const float* __restrict__ consts,
-                                                               long long n_per_utt, float out_scale, float* __restrict__ d_wav) {
+                                                               long long n_per_utt, float out_scale,
+                                                               const float* __restrict__ scale_dev, float* __restrict__ d_wav) {
     const int b = blockIdx.y;
     const long long s = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= n_per_utt) return;
@@ -455,7 +580,7 @@ __global__ void __launch_bounds__(256) conv0_bwd_finish_kernel(const float* __re
             acc += v;
         }
     }
-    d_wav[(long long)b * n_per_utt + s] = acc * out_scale;
+    d_wav[(long long)b * n_per_utt + s] = acc * (scale_dev != nullptr ? 1.0f / __ldg(scale_dev) : out_scale);
 }
 
 __global__ void loss_finalize_kernel(const double* __restrict__ acc, double inv_layer, double inv_head, float* __restrict__ loss) {
@@ -568,8 +693,16 @@ size_t nomad_b200_loss_workspace_bytes(int B, int64_t N, int with_grad) {
 // to the waveform (dgrad chain).  `seed_layer`: L1 seed of every layer output against the second half of the batch (the
 // loss path; 0 = none); L.g_pool: per-utterance gradient of the mean-pooled top layer.  `tc` (triplet fine-tuning,
 // triplet section below): also produce the parameter gradients of everything after the (frozen) conv feature encoder and
-// stop there.
+// stop there.  `ug` (autograd path, nomad_b200_layers_bwd): caller-given upstream gradients of the layer outputs and the
+// pooled head instead of the L1 seeds, under a scale S that lives on the device.
 struct TrainCtx;
+struct UserGrads {
+    const float* g_layers[LAYERS];  // gradient wrt layer l's output, B x T x 768 (caller layout), or null
+    int T;                          // frames per utterance of that layout
+    const float* g_pool;            // [B][768] unscaled pooled-feature gradient of the head, or null
+    const float* scale;             // device: S
+    int top;                        // highest layer that receives a gradient; the layers above it are skipped
+};
 static int train_hook_layer(Handle* h, const Workspace& ws, const LossBufs& L, TrainCtx* tc, int l, int stage, int B,
                             long long Fe, const float* g_running, cudaStream_t st);
 static int train_hook_front(Handle* h, const Workspace& ws, const LossBufs& L, TrainCtx* tc, int stage, int B, long long Fe,
@@ -577,7 +710,8 @@ static int train_hook_front(Handle* h, const Workspace& ws, const LossBufs& L, T
 
 static int backward_chain(Handle* h, const Workspace& ws, const LossBufs& L, int B, long long Fe, long long R0e,
                           long long pos_rows_e, int T, float seed_layer, float feature_grad_mult, float S,
-                          const float* est_dev, int64_t N, float* d_est_dev, cudaStream_t st, TrainCtx* tc) {
+                          const float* est_dev, int64_t N, float* d_est_dev, cudaStream_t st, TrainCtx* tc,
+                          const UserGrads* ug = nullptr) {
     const Weights& w = h->w;
     const int impl = h->gemm_impl;
     const unsigned row_blocks = (unsigned)((Fe + 7) / 8);
@@ -588,12 +722,18 @@ static int backward_chain(Handle* h, const Workspace& ws, const LossBufs& L, int
     };
     NB_CUDA(cudaMemsetAsync(L.g_qkv, 0, 2ull * 3 * EMBED * Fe, st));
     const float* g_running = nullptr;  // gradient wrt the current layer's output from the layers above
-    for (int l = LAYERS - 1; l >= 0; --l) {
+    for (int l = ug != nullptr ? ug->top : LAYERS - 1; l >= 0; --l) {
         const LayerWeights& W = w.layer[l];
         const LayerBufs& Lb = ws.layer[l];
         // final_layer_norm backward (+ L1 seed of this layer's output, + pooled-head gradient on the top layer)
-        ln768_bwd_kernel<<<row_blocks, 256, 0, st>>>(g_running, Lb.pre2, ws.meta, B, Fe, W.ln2_g, seed_layer,
-                                                     l == LAYERS - 1 ? L.g_pool : nullptr, L.g_b, L.g_bh);
+        if (ug != nullptr) {
+            ln768_bwd_user_kernel<<<row_blocks, 256, 0, st>>>(g_running, Lb.pre2, ws.meta, B, Fe, W.ln2_g, ug->g_layers[l],
+                                                              ug->T, l == LAYERS - 1 ? ug->g_pool : nullptr, ug->scale,
+                                                              L.g_b, L.g_bh);
+        } else {
+            ln768_bwd_kernel<<<row_blocks, 256, 0, st>>>(g_running, Lb.pre2, ws.meta, B, Fe, W.ln2_g, seed_layer,
+                                                         l == LAYERS - 1 ? L.g_pool : nullptr, L.g_b, L.g_bh);
+        }
         NB_LAUNCHED();
         if (tc) NB_TRY(train_hook_layer(h, ws, L, tc, l, 0, B, Fe, g_running, st));  // LN2 params, fc2 weight + bias
         {   // fc2 dgrad, times gelu'(fc1 pre-activation)
@@ -702,7 +842,8 @@ static int backward_chain(Handle* h, const Workspace& ws, const LossBufs& L, int
         NB_TRY(gemm_h16(st, A, Bw, (int)R0e, 16, CONV_DIM, 1, e, impl));
     }
     dim3 fgrid((unsigned)((N + 255) / 256), B);
-    conv0_bwd_finish_kernel<<<fgrid, 256, 0, st>>>(L.c0_V, est_dev, ws.meta, L.c0_consts, N, 1.0f / S, d_est_dev);
+    conv0_bwd_finish_kernel<<<fgrid, 256, 0, st>>>(L.c0_V, est_dev, ws.meta, L.c0_consts, N, 1.0f / S,
+                                                   ug != nullptr ? ug->scale : nullptr, d_est_dev);
     NB_LAUNCHED();
     return 0;
 }
@@ -1368,6 +1509,159 @@ int nomad_b200_triplet_fwd_bwd(nomad_b200_handle* hh, const float* wav_dev, int 
     NB_LAUNCHED();
     *grad_scale_out = S;
     return backward_chain(h, ws, L, U, F, R0, pos_rows, p.max_T, 0.f, 1.0f, S, wav_dev, N, nullptr, st, &tc);
+}
+
+}  // extern "C"
+
+// ---- autograd through LossNetLayers / TripletModel: save-mode forward + backward from arbitrary upstream gradients ----
+// The saved buffer is [save-mode Workspace | pooled features B x 768 | head output B x 256 | head snapshot: transposed
+// weight 768 x 256, bias 256].  The backward re-derives the Plan from (B, N) and re-carves the same Workspace over it, so
+// every pointer (metadata included) comes back as the forward left it; the backward only reads it.
+struct SavedTail {
+    float* pooled;
+    float* emb;
+    float* head_wt;
+    float* head_b;
+};
+
+static int layers_plan(int B, int64_t N, Plan* p) {
+    NB_CHECK(B > 0, "layers: need B > 0 utterances");
+    NB_CHECK(N >= NOMAD_B200_MIN_SAMPLES,
+             "layers: N = %lld samples; the conv feature encoder needs at least %d (kernel size can't be greater than "
+             "actual input size)", (long long)N, NOMAD_B200_MIN_SAMPLES);
+    std::vector<int64_t> off((size_t)B + 1);
+    for (int b = 0; b <= B; ++b) off[b] = (int64_t)b * N;
+    return make_plan(off.data(), B, p);
+}
+
+static size_t carve_saved(const Plan& p, void* base, Workspace* ws, SavedTail* tail) {
+    size_t o = carve_workspace(p, base, ws, true);
+    auto take = [&](size_t bytes) {
+        size_t at = o;
+        o = (o + bytes + 1023) / 1024 * 1024;
+        return base ? (float*)((char*)base + at) : nullptr;
+    };
+    SavedTail t;
+    t.pooled = take(4ull * EMBED * p.B);
+    t.emb = take(4ull * EMB * p.B);
+    t.head_wt = take(4ull * EMBED * EMB);
+    t.head_b = take(4ull * EMB);
+    if (tail) *tail = t;
+    return o;
+}
+
+// backward scratch: [LossBufs | gy B x 256 | scale state: max bits, block counter, S]
+static size_t carve_layers_bwd(const Plan& p, void* base, LossBufs* L, float** gy, unsigned** state) {
+    const size_t lb = carve_loss(p, p.B, p.frames, p.rows0, p.pos_rows, true, base, L);
+    const size_t gy_bytes = (4ull * EMB * p.B + 1023) / 1024 * 1024;
+    if (base) {
+        *gy = (float*)((char*)base + lb);
+        *state = (unsigned*)((char*)base + lb + gy_bytes);
+    }
+    return lb + gy_bytes + 1024;
+}
+
+extern "C" {
+
+size_t nomad_b200_layers_saved_bytes(int B, int64_t N) {
+    Plan p;
+    if (layers_plan(B, N, &p)) return 0;
+    return carve_saved(p, nullptr, nullptr, nullptr);
+}
+
+size_t nomad_b200_layers_bwd_workspace_bytes(int B, int64_t N) {
+    Plan p;
+    if (layers_plan(B, N, &p)) return 0;
+    return carve_layers_bwd(p, nullptr, nullptr, nullptr, nullptr);
+}
+
+int nomad_b200_layers_fwd_save(nomad_b200_handle* hh, const float* wav_dev, int B, int64_t N, int head, float* layers_dev,
+                               float* emb_dev, void* saved_dev, size_t saved_bytes, void* stream) {
+    NB_CHECK(hh != nullptr, "null nomad_b200 handle");
+    Handle* h = &hh->h;
+    NB_CHECK(wav_dev && saved_dev, "layers_fwd_save: null pointer");
+    NB_CHECK(head == 0 || head == 1, "layers_fwd_save: head must be 0 (NOMAD head) or 1 (loss head)");
+    NB_CHECK(head == 0 || h->has_loss_head, "layers_fwd_save: head 1 needs nomad_b200_set_loss_head first");
+    NB_CHECK(((uintptr_t)wav_dev & 3) == 0, "layers_fwd_save: waveform pointer must be 4-byte aligned");
+    NB_CHECK(((uintptr_t)saved_dev & 1023) == 0, "layers_fwd_save: saved buffer must be 1024-byte aligned");
+    NB_CUDA(cudaSetDevice(h->device));
+    Plan p;
+    NB_TRY(layers_plan(B, N, &p));
+    Workspace ws;
+    SavedTail t;
+    const size_t need = carve_saved(p, saved_dev, &ws, &t);
+    NB_CHECK(saved_bytes >= need, "layers_fwd_save: saved buffer too small (%zu < %zu bytes)", saved_bytes, need);
+    cudaStream_t st = (cudaStream_t)stream;
+    const Weights& w = h->w;
+    NB_CUDA(cudaMemcpyAsync(t.head_wt, head ? w.loss_head_wt : w.head_wt, 4ull * EMBED * EMB, cudaMemcpyDeviceToDevice, st));
+    NB_CUDA(cudaMemcpyAsync(t.head_b, head ? w.loss_head_b : w.head_b, 4ull * EMB, cudaMemcpyDeviceToDevice, st));
+    NB_TRY(upload_meta(h, p, ws, st));
+    NB_TRY(forward_encoder(h, p, ws, wav_dev, st, layers_dev, p.max_T));
+    NB_TRY(launch_pool_head(st, ws.x, ws.meta, p.B, t.head_wt, t.head_b, emb_dev ? emb_dev : t.emb, t.pooled));
+    return 0;
+}
+
+int nomad_b200_layers_bwd(nomad_b200_handle* hh, const void* saved_dev, size_t saved_bytes, const float* wav_dev, int B,
+                          int64_t N, const float* const* g_layers, const float* g_emb, float feature_grad_mult,
+                          float* d_wav_dev, void* workspace_dev, size_t workspace_bytes, void* stream) {
+    NB_CHECK(hh != nullptr, "null nomad_b200 handle");
+    Handle* h = &hh->h;
+    NB_CHECK(saved_dev && wav_dev && d_wav_dev && workspace_dev, "layers_bwd: null pointer");
+    NB_CHECK(((uintptr_t)saved_dev & 1023) == 0 && ((uintptr_t)workspace_dev & 1023) == 0,
+             "layers_bwd: saved buffer and workspace must be 1024-byte aligned");
+    NB_CHECK(((uintptr_t)wav_dev & 3) == 0 && ((uintptr_t)d_wav_dev & 3) == 0, "layers_bwd: waveform pointers must be 4-byte aligned");
+    NB_CHECK(((uintptr_t)g_emb & 15) == 0, "layers_bwd: g_emb must be 16-byte aligned");
+    for (int l = 0; g_layers != nullptr && l < LAYERS; ++l)
+        NB_CHECK(((uintptr_t)g_layers[l] & 15) == 0, "layers_bwd: g_layers[%d] must be 16-byte aligned", l);
+    NB_CUDA(cudaSetDevice(h->device));
+    Plan p;
+    NB_TRY(layers_plan(B, N, &p));
+    Workspace ws;
+    SavedTail t;
+    const size_t need_saved = carve_saved(p, (void*)saved_dev, &ws, &t);
+    NB_CHECK(saved_bytes >= need_saved, "layers_bwd: saved buffer too small (%zu < %zu bytes): not from a forward of this B x N?",
+             saved_bytes, need_saved);
+    LossBufs L;
+    float* gy = nullptr;
+    unsigned* state = nullptr;
+    const size_t need = carve_layers_bwd(p, workspace_dev, &L, &gy, &state);
+    NB_CHECK(workspace_bytes >= need, "layers_bwd: workspace too small (%zu < %zu bytes)", workspace_bytes, need);
+    cudaStream_t st = (cudaStream_t)stream;
+
+    UserGrads ug;
+    memset(&ug, 0, sizeof(ug));
+    ug.T = p.max_T;
+    ug.top = -1;
+    ScaleSources src;
+    memset(&src, 0, sizeof(src));
+    const long long layer_n = (long long)B * p.max_T * EMBED;
+    for (int l = 0; l < LAYERS; ++l) {
+        ug.g_layers[l] = g_layers != nullptr ? g_layers[l] : nullptr;
+        src.p[l] = ug.g_layers[l];
+        src.n[l] = layer_n;
+        if (ug.g_layers[l] != nullptr) ug.top = l;
+    }
+    if (ug.top < 0 && g_emb == nullptr) {  // no output is used: the gradient is zero
+        NB_CUDA(cudaMemsetAsync(d_wav_dev, 0, 4ull * B * N, st));
+        return 0;
+    }
+    if (g_emb != nullptr) {  // head: g_emb -> gy -> pooled-feature gradient (ReLU mask, / T), with the snapshotted head
+        head_emb_bwd_kernel<<<B, 256, 0, st>>>(t.pooled, t.head_wt, t.head_b, g_emb, gy);
+        NB_LAUNCHED();
+        head_pool_grad_kernel<<<B, 256, 0, st>>>(gy, t.pooled, ws.meta, t.head_wt, L.g_pool);
+        NB_LAUNCHED();
+        ug.g_pool = L.g_pool;
+        ug.top = LAYERS - 1;
+        src.p[LAYERS] = L.g_pool;
+        src.n[LAYERS] = (long long)B * EMBED;
+    }
+    float* scale = (float*)(state + 2);
+    ug.scale = scale;
+    NB_CUDA(cudaMemsetAsync(state, 0, 2 * sizeof(unsigned), st));
+    grad_scale_kernel<<<2 * 148, 256, 0, st>>>(src, state, scale);
+    NB_LAUNCHED();
+    return backward_chain(h, ws, L, B, p.frames, p.rows0, p.pos_rows, p.max_T, 0.f, feature_grad_mult, 1.f, wav_dev, N,
+                          d_wav_dev, st, nullptr, &ug);
 }
 
 }  // extern "C"

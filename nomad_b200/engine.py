@@ -319,6 +319,53 @@ class Engine:
                                                       _stream_ptr()), "nomad_b200_layers_fwd")
         return layers, emb
 
+    def layers_fwd_save(self, wav: torch.Tensor, head: int, want_layers: bool = True):
+        """Save-mode forward of a (B, N) CUDA batch for autograd (``nomad_b200_layers_fwd_save``; fp16 operands whatever
+        the engine's precision).  ``head``: 0 = NOMAD head, 1 = loss head.  -> ((12, B, T, 768) | None, (B, 256), saved):
+        ``saved`` is a uint8 CUDA tensor owned by the caller that :meth:`layers_bwd` needs; keep it until then."""
+        wav = wav.to(self.device, torch.float32).contiguous()
+        B, N = wav.shape
+        T = self.num_frames(N)
+        nbytes = self.lib.nomad_b200_layers_saved_bytes(B, N)
+        if nbytes == 0:
+            raise _lib.NomadB200Error(self.lib.nomad_b200_last_error().decode())
+        saved = torch.empty(nbytes + 1024, dtype=torch.uint8, device=self.device)
+        sp, sbytes = self._aligned(saved)
+        layers = torch.empty((NUM_LAYERS, B, T, SSL_OUT_DIM), dtype=torch.float32, device=self.device) if want_layers else None
+        emb = torch.empty((B, EMB_DIM), dtype=torch.float32, device=self.device)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.nomad_b200_layers_fwd_save(self.handle, _ptr(wav), B, N, int(head), _ptr(layers), _ptr(emb),
+                                                           sp, sbytes, _stream_ptr()), "nomad_b200_layers_fwd_save")
+        return layers, emb, saved
+
+    def layers_bwd(self, saved: torch.Tensor, wav: torch.Tensor, g_layers: Sequence[Optional[torch.Tensor]],
+                   g_emb: Optional[torch.Tensor], feature_grad_mult: float) -> torch.Tensor:
+        """d(<g_layers, layers> + <g_emb, emb>) / d wav for the forward that filled ``saved`` (``nomad_b200_layers_bwd``):
+        ``g_layers``: 12 entries of (B, T, 768) or None, ``g_emb``: (B, 256) or None.  -> (B, N) fp32 CUDA tensor."""
+        wav = wav.to(self.device, torch.float32).contiguous()
+        B, N = wav.shape
+
+        def dev(g):  # fp32, contiguous, 16-byte aligned (the kernels read rows as float4)
+            if g is None:
+                return None
+            g = g.to(self.device, torch.float32).contiguous()
+            return g if g.data_ptr() % 16 == 0 else g.clone()
+
+        gl = [dev(g) for g in g_layers]
+        ge = dev(g_emb)
+        need = self.lib.nomad_b200_layers_bwd_workspace_bytes(B, N)
+        if need == 0:
+            raise _lib.NomadB200Error(self.lib.nomad_b200_last_error().decode())
+        wp, wbytes = self._aligned(self.workspace(need))
+        sp, sbytes = self._aligned(saved)
+        ptrs = (C.c_void_p * NUM_LAYERS)(*[None if g is None else g.data_ptr() for g in gl])
+        d_wav = torch.empty((B, N), dtype=torch.float32, device=self.device)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.nomad_b200_layers_bwd(self.handle, sp, sbytes, _ptr(wav), B, N, ptrs, _ptr(ge),
+                                                      C.c_float(feature_grad_mult), _ptr(d_wav), wp, wbytes, _stream_ptr()),
+                       "nomad_b200_layers_bwd")
+        return d_wav
+
     def loss_fwd_bwd(self, est: torch.Tensor, clean: torch.Tensor, feature_grad_mult: float, with_grad: bool = True):
         if est.dim() == 3:
             est = est.squeeze(1)

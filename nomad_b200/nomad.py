@@ -9,8 +9,10 @@ backward) runs in ``libnomad_b200.so`` on a B200.  Differences that are delibera
 * there is no CPU path: ``device='cpu'`` raises;
 * weights come from ``pt-models/nomad_best_model.pt`` (or ``$NOMAD_B200_CHECKPOINT``) when present,
   else seeded random-init of the identical architecture -- nothing is downloaded at import;
-* ``forward`` back-propagates to ``estimate`` only (dgrad chain, wheel 0.0.8 semantics: the NOMAD
-  network's own parameters receive no ``.grad``).
+* gradients reach the input waveforms only (dgrad chain, wheel 0.0.8 semantics: the NOMAD network's own
+  parameters receive no ``.grad``);
+* the differentiable calls (``model``, ``lossnet_layers`` and ``forward`` with grad on) always run fp16 tensor-core
+  operands: with ``precision='fp32'`` only the no-grad path is fp32-class.
 """
 from __future__ import annotations
 
@@ -26,7 +28,7 @@ import torch.nn.functional as F
 
 from . import audio
 from .engine import Engine, MIN_SAMPLES
-from .weights import EMB_DIM, SSL_OUT_DIM, load_state_dict
+from .weights import EMB_DIM, NUM_LAYERS, SSL_OUT_DIM, load_state_dict
 
 w2v_path = 'pt-models/wav2vec_small.pt'        # kept for API compatibility (nomad.py:21); unused
 nomad_path = 'pt-models/nomad_best_model.pt'   # nomad.py:29
@@ -49,12 +51,42 @@ def plan_batches(lengths: Sequence[int], max_samples: int) -> List[List[int]]:
     return batches
 
 
-class TripletModel:
-    """``TripletModel`` (``nomad.py:214-231``): ``model(wav, lengths=None) -> (B, 256)`` unit-norm."""
+class _NetworkFn(torch.autograd.Function):
+    """The network as an autograd node: save-mode forward (``nomad_b200_layers_fwd_save``) of a (B, N) batch, backward
+    from whichever outputs were used (``nomad_b200_layers_bwd``; unused outputs reach it as NULL).  ``head``: 0 = NOMAD
+    head, outputs (emb,); 1 = loss head, outputs (12 layer outputs..., emb).  Only ``wav`` gets a gradient."""
 
-    def __init__(self, engine: Engine):
+    @staticmethod
+    def forward(ctx, wav, engine, head, feature_grad_mult):
+        ctx.set_materialize_grads(False)
+        ctx.engine, ctx.fgm, ctx.want_layers = engine, float(feature_grad_mult), head == 1
+        ctx.in_shape, ctx.in_device, ctx.in_dtype = wav.shape, wav.device, wav.dtype
+        flat = wav.detach().reshape(-1, wav.shape[-1]).to(engine.device, torch.float32).contiguous()
+        layers, emb, saved = engine.layers_fwd_save(flat, head, want_layers=ctx.want_layers)
+        ctx.save_for_backward(flat, saved)  # released after the backward (unless the graph is retained)
+        return (*layers.unbind(0), emb) if ctx.want_layers else emb
+
+    @staticmethod
+    def backward(ctx, *grads):
+        flat, saved = ctx.saved_tensors
+        g_layers = list(grads[:-1]) if ctx.want_layers else [None] * NUM_LAYERS
+        d = ctx.engine.layers_bwd(saved, flat, g_layers, grads[-1], ctx.fgm)
+        return d.reshape(ctx.in_shape).to(ctx.in_device, ctx.in_dtype), None, None, None
+
+
+def _differentiable(wav) -> bool:
+    return torch.is_grad_enabled() and torch.is_tensor(wav) and wav.requires_grad
+
+
+class TripletModel:
+    """``TripletModel`` (``nomad.py:214-231``): ``model(wav, lengths=None) -> (B, 256)`` unit-norm.  With grad enabled
+    and ``wav.requires_grad`` the call is differentiable wrt ``wav`` (fp16 operands, fairseq's GradMultiply of
+    ``feature_grad_mult()`` on the conv features)."""
+
+    def __init__(self, engine: Engine, feature_grad_mult=lambda: 0.1):
         self.engine = engine
         self.ssl_features = SSL_OUT_DIM
+        self.feature_grad_mult = feature_grad_mult  # zero-argument callable, read at each differentiable call
 
     def eval(self):
         return self
@@ -65,23 +97,29 @@ class TripletModel:
     def __call__(self, wav, lengths=None):  # ``lengths`` accepted and ignored, as in the reference
         return self.forward(wav, lengths)
 
-    @torch.no_grad()
     def forward(self, wav: torch.Tensor, lengths=None) -> torch.Tensor:
         if wav.dim() == 3:
             wav = wav.squeeze(1)  # nomad.py:225
         if wav.dim() == 1:
             wav = wav.unsqueeze(0)
-        B, N = wav.shape
-        flat = wav.to(self.engine.device, torch.float32).contiguous().reshape(-1)
-        return self.engine.embed_packed(flat, np.arange(B + 1, dtype=np.int64) * N)
+        if _differentiable(wav):
+            return _NetworkFn.apply(wav, self.engine, 0, self.feature_grad_mult())
+        with torch.no_grad():
+            B, N = wav.shape
+            flat = wav.to(self.engine.device, torch.float32).contiguous().reshape(-1)
+            return self.engine.embed_packed(flat, np.arange(B + 1, dtype=np.int64) * N)
 
 
 class LossNetLayers:
-    """``LossNetLayers`` (``nomad.py:233-258``): 12 transformer-layer outputs + the head output."""
+    """``LossNetLayers`` (``nomad.py:233-258``): 12 transformer-layer outputs + the head output.  With grad enabled and
+    ``wav.requires_grad`` the call is differentiable wrt ``wav`` through any use of the 13 outputs (fp16 operands,
+    fairseq's GradMultiply of ``feature_grad_mult()`` on the conv features); the backward uses the head as it was at
+    the forward."""
 
-    def __init__(self, engine: Engine):
+    def __init__(self, engine: Engine, feature_grad_mult=lambda: 0.1):
         self.engine = engine
         self.ssl_features = SSL_OUT_DIM
+        self.feature_grad_mult = feature_grad_mult  # zero-argument callable, read at each differentiable call
         # freshly initialised head, exactly like the reference (nomad.py:238-241)
         self.embedding_layer = nn.Sequential(nn.ReLU(), nn.Linear(SSL_OUT_DIM, EMB_DIM))
         self._synced = None
@@ -99,11 +137,13 @@ class LossNetLayers:
     def __call__(self, wav):
         return self.forward(wav)
 
-    @torch.no_grad()
     def forward(self, wav: torch.Tensor) -> List[torch.Tensor]:
         self.sync_head()
-        layers, emb = self.engine.layers(wav)
-        return [layers[i] for i in range(layers.shape[0])] + [emb]
+        if _differentiable(wav):
+            return list(_NetworkFn.apply(wav, self.engine, 1, self.feature_grad_mult()))
+        with torch.no_grad():
+            layers, emb = self.engine.layers(wav)
+            return [layers[i] for i in range(layers.shape[0])] + [emb]
 
 
 class NomadLoss(nn.Module):
@@ -172,9 +212,9 @@ class Nomad():
         self.precision = precision or os.environ.get("NOMAD_B200_PRECISION", "fp16")
         self.engine = Engine(state_dict, index, self.precision)
         self.state_dict_ref = state_dict if keep_state_dict else None   # fine-tuning (triplet.py) needs the fp32 tensors
-        self.model = TripletModel(self.engine)
+        self.model = TripletModel(self.engine, lambda: self.feature_grad_mult)
         # NOMAD loss model shares the same network (nomad.py:70-72)
-        self.lossnet_layers = LossNetLayers(self.engine)
+        self.lossnet_layers = LossNetLayers(self.engine, lambda: self.feature_grad_mult)
         self.nomad_loss = NomadLoss()
         # fairseq applies GradMultiply(feature_grad_mult) to the conv features (wav2vec 2.0 base: 0.1)
         self.feature_grad_mult = float(feature_grad_mult)
@@ -263,7 +303,11 @@ class Nomad():
         return dm.cpu().numpy().astype(np.float64), mean.cpu().numpy()
 
     def forward(self, estimate, clean):
-        """Differentiable NOMAD loss (``nomad.py:142-146``): 0-dim tensor, grad flows to ``estimate``."""
+        """Differentiable NOMAD loss (``nomad.py:142-146``): 0-dim tensor, grad flows to ``estimate``.  When ``clean``
+        requires grad too (grad enabled), the reference's own composition runs instead of the fused CUDA-graph step,
+        so both inputs get their gradient."""
+        if _differentiable(clean):
+            return self.nomad_loss(self.lossnet_layers(clean), self.lossnet_layers(estimate))
         self.lossnet_layers.sync_head()
         return _NomadLossFn.apply(estimate, clean, self)
 
