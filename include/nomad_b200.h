@@ -179,7 +179,7 @@ NOMAD_B200_API int nomad_b200_write_scores_csv(const char* path, const char* ind
 NOMAD_B200_API int nomad_b200_paired_dist(const float* a_dev, const float* b_dev, int64_t n, double* out_dev, void* stream);
 
 /* ---- triplet fine-tuning step (reference src/training/train_triplet.py:112-133; conv feature encoder frozen as in
- * src/config/train_triplet.yaml `freeze_convnet: True`) ---------------------------------------------------------------
+ * src/config/train_triplet.yaml `freeze_convnet: True`, or trained with it: nomad_b200_triplet_conv_fwd_bwd) ----------
  * wav: 3B x N fp32 device rows: B anchors, then B positives, then B negatives (the zero-padded batches of the
  * reference's collate_fn).  Computes the embeddings of all three, loss = nn.TripletMarginLoss(margin)(A, P, N) and the
  * gradient of the loss wrt EVERY trainable parameter: LayerNorm(512), feature projection, positional conv (as the
@@ -189,11 +189,18 @@ NOMAD_B200_API int nomad_b200_paired_dist(const float* a_dev, const float* b_dev
  * values laid out as nomad_b200_triplet_grad_segment enumerates, all multiplied by *grad_scale_out (a power of two
  * that keeps 16-bit activation gradients in range; divide it out).  The optimiser step itself (Adam, train_triplet.py:
  * 92-107) is host plumbing: see nomad_b200/triplet.py. */
-/* After the optimiser step (train_triplet.py:129-130): rebuild the kernel-ready weights of everything trainable (16-bit
- * copies, fused q|k|v with the q scale, transposes for the dgrad GEMMs, LayerNorm folds, weight-norm fold of the positional
- * conv, head) from fp32 master tensors that live on the DEVICE -- same names as nomad_b200_create, `data` = device pointers.
- * A few bandwidth-bound kernels on `stream`; the frozen conv feature encoder is not touched. */
+/* After the optimiser step (train_triplet.py:129-130): rebuild the kernel-ready weights of everything after the conv
+ * feature encoder (16-bit copies, fused q|k|v with the q scale, transposes for the dgrad GEMMs, LayerNorm folds,
+ * weight-norm fold of the positional conv, head) from fp32 master tensors that live on the DEVICE -- same names as
+ * nomad_b200_create, `data` = device pointers.  A few bandwidth-bound kernels on `stream`; the conv feature encoder is
+ * rebuilt by nomad_b200_refresh_conv_weights (only needed when it is trained). */
 NOMAD_B200_API int nomad_b200_refresh_weights(nomad_b200_handle* h, const nomad_b200_tensor* tensors_dev, int n_tensors, void* stream);
+/* The same for the conv feature encoder (freeze_convnet: False): conv0 and GroupNorm weights and every 16-bit / transposed
+ * conv1-6 copy are rewritten IN PLACE from the device tensors `ssl_model.feature_extractor.conv_layers.*`, with the bits
+ * nomad_b200_create gives, so pointers captured by loss-step CUDA graphs stay valid.  Refused while the fp32-class planes
+ * are built and active (fine-tuning runs the fp16-operand path). */
+NOMAD_B200_API int nomad_b200_refresh_conv_weights(nomad_b200_handle* h, const nomad_b200_tensor* tensors_dev, int n_tensors,
+                                                   void* stream);
 /* Test hook for the refresh path: copy one kernel-ready weight buffer to the host (see refresh.cu for the names). */
 NOMAD_B200_API int nomad_b200_debug_read_weight(nomad_b200_handle* h, const char* which, void* dst_host, size_t bytes);
 NOMAD_B200_API int64_t nomad_b200_triplet_grad_floats(void);
@@ -202,6 +209,19 @@ NOMAD_B200_API size_t nomad_b200_triplet_workspace_bytes(int B, int64_t N);
 NOMAD_B200_API int nomad_b200_triplet_fwd_bwd(nomad_b200_handle* h, const float* wav_dev, int B, int64_t N, float margin,
                                float* loss_dev, float* grads_dev, float* grad_scale_out, void* workspace_dev,
                                size_t workspace_bytes, void* stream);
+/* Triplet step with the conv feature encoder trained too (freeze_convnet: False).  loss and grads exactly as
+ * nomad_b200_triplet_fwd_bwd; conv_grads (16-byte aligned): nomad_b200_triplet_conv_grad_floats() fp32 values, the
+ * gradients of conv0, the GroupNorm affine pair and conv1-6 under their fairseq state-dict names, each in the
+ * checkpoint's (out, in, tap) order (nomad_b200_triplet_conv_grad_segment), times the same *grad_scale_out.  fairseq's
+ * GradMultiply(feature_grad_mult) on the conv features scales every conv gradient (and not the LayerNorm(512) ones).
+ * conv1-6 weight gradients are split-K tensor-core GEMMs over the tokens; conv0 / GroupNorm reduce to per-channel sums. */
+NOMAD_B200_API size_t nomad_b200_triplet_conv_workspace_bytes(int B, int64_t N);
+NOMAD_B200_API int64_t nomad_b200_triplet_conv_grad_floats(void);
+NOMAD_B200_API int nomad_b200_triplet_conv_grad_segment(int i, char* name, int name_cap, int64_t* offset, int64_t* numel);
+NOMAD_B200_API int nomad_b200_triplet_conv_fwd_bwd(nomad_b200_handle* h, const float* wav_dev, int B, int64_t N, float margin,
+                                                   float feature_grad_mult, float* loss_dev, float* grads_dev,
+                                                   float* conv_grads_dev, float* grad_scale_out, void* workspace_dev,
+                                                   size_t workspace_bytes, void* stream);
 
 /* ---- building block exposed for the parity tests --------------------------------------------------
  * C (m x n, ldc) = epilogue(A (m x k op_t, row stride lda elements, may overlap) * B^T (n x k op_t)).

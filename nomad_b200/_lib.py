@@ -76,6 +76,12 @@ PROTOTYPES = {
     "nomad_b200_triplet_workspace_bytes": (C.c_size_t, [C.c_int, c_i64]),
     "nomad_b200_triplet_fwd_bwd": (C.c_int, [c_vp, c_vp, C.c_int, c_i64, C.c_float, c_vp, c_vp, C.POINTER(C.c_float), c_vp,
                                              C.c_size_t, c_vp]),
+    "nomad_b200_refresh_conv_weights": (C.c_int, [c_vp, C.POINTER(Tensor), C.c_int, c_vp]),
+    "nomad_b200_triplet_conv_grad_floats": (c_i64, []),
+    "nomad_b200_triplet_conv_grad_segment": (C.c_int, [C.c_int, C.c_char_p, C.c_int, C.POINTER(c_i64), C.POINTER(c_i64)]),
+    "nomad_b200_triplet_conv_workspace_bytes": (C.c_size_t, [C.c_int, c_i64]),
+    "nomad_b200_triplet_conv_fwd_bwd": (C.c_int, [c_vp, c_vp, C.c_int, c_i64, C.c_float, C.c_float, c_vp, c_vp, c_vp,
+                                                  C.POINTER(C.c_float), c_vp, C.c_size_t, c_vp]),
     "nomad_b200_gemm_split": (C.c_int, [c_vp, c_vp, c_i64, c_vp, c_vp, C.c_int, C.c_int, C.c_int, C.c_float, c_vp, c_vp, c_vp,
                                         c_vp, c_i64, C.c_int, c_vp]),
     "nomad_b200_write_scores_csv": (C.c_int, [C.c_char_p, C.c_char_p, C.POINTER(C.c_char_p), c_i64, C.POINTER(C.c_char_p),

@@ -541,6 +541,7 @@ int forward_encoder(Handle* h, const Plan& p, const Workspace& ws, const float* 
             NB_TRY(launch_wave_stats(st, wav, ws.meta, b0, nb, p.max_chunks, ws.stat_part));
             NB_TRY(launch_gn_fold(st, ws.stat_part, ws.meta, b0, nb, p.max_chunks, w.conv0_w, w.gn_g, w.gn_b, ws.c0_fold,
                                   ws.gn_stat, ws.c0_fold_h));
+            if (ws.aux0_raw) NB_TRY(launch_fold_unit_dgelu_gain(st, ws.c0_fold, b0, nb));
             NB_TRY(launch_conv0_apply(st, wav, ws.meta, p.B, row_of(b0), row_of(b0 + nb), ws.c0_fold,
                                       impl == 0 ? ws.c0_fold_h : nullptr, ws.y[0], ws.aux[0]));
         }

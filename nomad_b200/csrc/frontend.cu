@@ -150,6 +150,16 @@ int launch_gn_fold(cudaStream_t st, const double* part, const UttMeta* meta, int
     return 0;
 }
 
+__global__ void __launch_bounds__(512) fold_unit_dgelu_gain_kernel(float* __restrict__ fold, int b0) {
+    fold[((long long)(b0 + blockIdx.x) * CONV_DIM + threadIdx.x) * 12 + 11] = 1.f;
+}
+
+int launch_fold_unit_dgelu_gain(cudaStream_t st, float* fold, int b0, int nb) {
+    fold_unit_dgelu_gain_kernel<<<nb, CONV_DIM, 0, st>>>(fold, b0);
+    NB_LAUNCHED();
+    return 0;
+}
+
 // ---------------------------------------------------------------------------------------------
 // One block = 64 consecutive level-0 rows (always inside one utterance: rows0 is a multiple of 64),
 // 256 threads x 2 channels.  out[row][c] = GELU(sum_j fold[c][j] x[5 t + j] + shift[c]) as op_t,

@@ -12,6 +12,8 @@ int launch_gn_fold(cudaStream_t st, const double* part, const UttMeta* meta, int
                    const float* conv0_w, const float* gn_g, const float* gn_b, float* fold, float* stat_out,
                    op_t* fold_h);
 // level-0 rows [row_begin, row_end) (multiples of 64, utterance boundaries)
+// fold[b][c][11] := 1 for utterances [b0, b0 + nb): conv0's saved GELU gradient is then gelu' itself
+int launch_fold_unit_dgelu_gain(cudaStream_t st, float* fold, int b0, int nb);
 int launch_conv0_apply(cudaStream_t st, const float* wav, const UttMeta* meta, int B, long long row_begin,
                        long long row_end, const float* fold, const op_t* fold_h, op_t* out, op_t* aux_out);
 // zero rows [T_l, rows_l) of every utterance at conv level l (so masked rows carry no gradient)

@@ -692,8 +692,9 @@ size_t nomad_b200_loss_workspace_bytes(int B, int64_t N, int with_grad) {
 // Backward of the encoder for the first B utterances of the batch (frames [0, Fe)): gradient wrt every layer input down
 // to the waveform (dgrad chain).  `seed_layer`: L1 seed of every layer output against the second half of the batch (the
 // loss path; 0 = none); L.g_pool: per-utterance gradient of the mean-pooled top layer.  `tc` (triplet fine-tuning,
-// triplet section below): also produce the parameter gradients of everything after the (frozen) conv feature encoder and
-// stop there.  `ug` (autograd path, nomad_b200_layers_bwd): caller-given upstream gradients of the layer outputs and the
+// triplet section below): also produce the parameter gradients of everything after the conv feature encoder, and stop
+// there when the encoder is frozen; when it is trained, go on through conv layers 6..1 (weight gradients from each
+// level's pre-GELU gradient) and stop at conv0 + GroupNorm, whose parameter gradients replace the waveform gradient.  `ug` (autograd path, nomad_b200_layers_bwd): caller-given upstream gradients of the layer outputs and the
 // pooled head instead of the L1 seeds, under a scale S that lives on the device.
 struct TrainCtx;
 struct UserGrads {
@@ -707,6 +708,10 @@ static int train_hook_layer(Handle* h, const Workspace& ws, const LossBufs& L, T
                             long long Fe, const float* g_running, cudaStream_t st);
 static int train_hook_front(Handle* h, const Workspace& ws, const LossBufs& L, TrainCtx* tc, int stage, int B, long long Fe,
                             long long pos_rows_e, cudaStream_t st);
+static bool train_conv(const TrainCtx* tc);
+static int train_hook_conv(TrainCtx* tc, int l, const op_t* gu, const op_t* y_in, long long y_rows, long long M, cudaStream_t st);
+static int train_hook_conv0(TrainCtx* tc, const Workspace& ws, const op_t* D0, const float* wav, int B, long long R0,
+                            const Weights& w, cudaStream_t st);
 
 static int backward_chain(Handle* h, const Workspace& ws, const LossBufs& L, int B, long long Fe, long long R0e,
                           long long pos_rows_e, int T, float seed_layer, float feature_grad_mult, float S,
@@ -797,7 +802,10 @@ static int backward_chain(Handle* h, const Workspace& ws, const LossBufs& L, int
         GemmEpilogue e = epi_grad(EPI_OUT_F32, nullptr, L.g_ln0, nullptr, nullptr, CONV_DIM);
         NB_TRY(gemm_h16(st, A, Bw, (int)Fe, CONV_DIM, EMBED, 1, e, impl));
     }
-    if (tc) return train_hook_front(h, ws, L, tc, 3, B, Fe, pos_rows_e, st);  // LayerNorm(512) params; conv encoder frozen
+    if (tc) {
+        NB_TRY(train_hook_front(h, ws, L, tc, 3, B, Fe, pos_rows_e, st));  // LayerNorm(512) params
+        if (!train_conv(tc)) return 0;                                      // conv feature encoder frozen
+    }
     // conv stack backward.  Gradient buffers start 8 rows into their allocation so that "row -1" reads zeros.
     NB_CUDA(cudaMemsetAsync(L.gu_a, 0, 2ull * CONV_DIM * 8, st));
     NB_CUDA(cudaMemsetAsync(L.gu_b, 0, 2ull * CONV_DIM * 8, st));
@@ -807,6 +815,7 @@ static int backward_chain(Handle* h, const Workspace& ws, const LossBufs& L, int
     NB_LAUNCHED();
     for (int l = 6; l >= 1; --l) {
         const long long M = R0e >> l;  // rows at level l (estimate half)
+        if (tc) NB_TRY(train_hook_conv(tc, l, gu[l], ws.y[l - 1], (R0e >> (l - 1)) + 8, M, st));  // before gu[l] is reused
         if (CONV_KERNEL[l] == 2) {
             // rows 2m and 2m+1 of level l-1 in one GEMM: N = 1024 = (tap, cin)
             GemmOperand A{gu[l], M, CONV_DIM, 0, 0};
@@ -829,6 +838,7 @@ static int backward_chain(Handle* h, const Workspace& ws, const LossBufs& L, int
             }
         }
     }
+    if (tc) return train_hook_conv0(tc, ws, gu[0], est_dev, B, R0e, h->w, st);  // gu[0] = dL/du0: no waveform gradient
     // conv0 + GroupNorm backward: gu[0] = G0
     NB_CUDA(cudaMemsetAsync(L.c0_sums, 0, 8ull * 2 * CONV_DIM * B, st));
     conv0_bwd_stats_kernel<<<(unsigned)(R0e / 64), 256, 0, st>>>(gu[0], est_dev, ws.meta, B, w.conv0_w, ws.gn_stat, L.c0_sums);
@@ -855,7 +865,9 @@ static int backward_chain(Handle* h, const Workspace& ws, const LossBufs& L, int
 // projection, positional conv, encoder LayerNorm, the 12 transformer layers, the embedding head).  The activation
 // gradients are the dgrad chain above; each weight gradient dW = dY^T X is a tensor-core GEMM over the token dimension
 // (both operands transposed into K-major first: two bandwidth-trivial passes), bias / LayerNorm gradients are column
-// reductions.  All gradients carry the power-of-two scale S of the chain; the caller divides it out.
+// reductions.  All gradients carry the power-of-two scale S of the chain; the caller divides it out.  With
+// `freeze_convnet: False` (nomad_b200_triplet_conv_fwd_bwd) the conv feature encoder's gradients follow as well (split-K
+// GEMMs for conv1-6, per-channel sums for conv0 + GroupNorm; see the conv section below).
 
 // flat gradient buffer (fp32): per layer [qkv_w 2304x768 | qkv_b | o_w | o_b | fc1_w | fc1_b | fc2_w | fc2_b | ln1_g | ln1_b |
 // ln2_g | ln2_b], then [enc_ln_g | enc_ln_b | pos_w 16x48x6144 (folded weight, layout [g][n][tap*48+c]) | pos_b |
@@ -879,7 +891,30 @@ struct TrainCtx {
     float* x_tmp;     // F x 768 fp32 scratch for the recomputation kernels
     float* gy;        // [3B][256] gradient wrt the un-normalised head output
     long long Fp;     // tokens rounded up to 8 (K of the weight-gradient GEMMs)
+    // conv feature encoder training (nomad_b200_triplet_conv_fwd_bwd); conv_grads == nullptr: encoder frozen
+    float* conv_grads;  // ConvLayout::TOTAL floats
+    op_t* ctA;          // [splits][512][Ks]: a level's pre-GELU gradient, transposed (K = rows, split into K slices)
+    op_t* ctB;          // [splits][k * 512][Ks]: the overlapping-row view of the level's input, transposed the same way
+    float* part;        // [splits][512][k * 512] fp32 partial weight gradients of the K slices
+    double* c0_sums;    // [3B][512][12] per (utterance, channel): sum D, sum D uhat, sum D x[5t + j]
+    int max_chunks;     // wave-stats chunks per utterance (Plan::max_chunks)
 };
+
+// flat conv-encoder gradient buffer (fp32), each tensor in the checkpoint's (out, in, tap) order:
+// [conv0 512x1x10 | GroupNorm weight 512 | GroupNorm bias 512 | conv1..6 512x512xk]
+struct ConvLayout {
+    static constexpr long long C0_W = 0, GN_G = C0_W + 512 * 10, GN_B = GN_G + 512, L1 = GN_B + 512,
+                               TOTAL = L1 + 4 * 512LL * 512 * 3 + 2 * 512LL * 512 * 2;
+    static long long level(int l) { return L1 + 512LL * 512 * 3 * std::min(l - 1, 4) + 512LL * 512 * 2 * std::max(l - 5, 0); }
+};
+// K slices of a conv weight-gradient GEMM: M (512) x N (512 k) is only 16-24 output tiles, while K = rows of the level
+// reaches ~4e5 at 8 triplets x 10 s; the slices run as the GEMM's batch and one pass sums their fp32 partials
+static constexpr int CONV_SPLIT_MAX = 24;
+static int conv_splits(long long M, long long* Ks) {
+    const int s = (int)std::min<long long>(CONV_SPLIT_MAX, std::max<long long>(1, (M + 4095) / 4096));
+    *Ks = ((M + s - 1) / s + 63) / 64 * 64;
+    return s;
+}
 
 // in [rows][cols] (16-bit) -> out[z][cols][rows_p] with out[z][c][r] = in[r + z][c] (zero past the end): copy z is the
 // transpose shifted by z rows (copies = 1: the plain transpose, columns rows..rows_p-1 zero)
@@ -1179,7 +1214,207 @@ __global__ void triplet_loss_finalize_kernel(const double* __restrict__ acc, dou
     *loss = (float)(acc[0] * inv_b);
 }
 
+// ---- conv feature encoder (trained only with nomad_b200_triplet_conv_fwd_bwd) ----------------------------------------
+// K-major operands of the conv weight gradient dW_l[n][tap * 512 + c] = sum_m gu[m][n] y[2m + tap][c]:
+// out[s][z * 512 + c][r] = in[stride * m + z][c] with m = s * Ks + r (zero for m >= M or past in_rows), z < gridDim.z.
+// stride 1, one tap: the transposed gradient; stride 2, k taps: the overlapping-row view of the level's input.
+__global__ void __launch_bounds__(256) conv_wgrad_transpose_kernel(const op_t* __restrict__ in, long long in_rows, int stride,
+                                                                   long long M, long long Ks, op_t* __restrict__ out) {
+    __shared__ op_t tile[64][66];
+    const long long m0 = (long long)blockIdx.x * 64;
+    const int c0 = blockIdx.y * 64, z = blockIdx.z, taps = gridDim.z;
+    for (int i = threadIdx.x; i < 64 * 64; i += 256) {
+        const int r = i >> 6, c = i & 63;
+        const long long m = m0 + r, src = stride * m + z;
+        tile[r][c] = (m < M && src < in_rows) ? in[src * CONV_DIM + c0 + c] : f2op(0.f);
+    }
+    __syncthreads();
+    const long long s = m0 / Ks, r0 = m0 - s * Ks;  // Ks % 64 == 0: the 64 rows stay in one slice
+    op_t* o = out + (s * taps * CONV_DIM + (long long)z * CONV_DIM) * Ks + r0;
+    for (int i = threadIdx.x; i < 64 * 64; i += 256) {
+        const int c = i >> 6, r = i & 63;
+        o[(long long)(c0 + c) * Ks + r] = tile[r][c];
+    }
+}
+// dW[o][c][tap] (checkpoint order) = sum over slices of part[s][o][tap * 512 + c]
+__global__ void __launch_bounds__(256) conv_wgrad_reduce_kernel(const float* __restrict__ part, int splits, int k,
+                                                                float* __restrict__ dw) {
+    const long long n = (long long)CONV_DIM * k * CONV_DIM;
+    const long long i = (long long)blockIdx.x * 256 + threadIdx.x;
+    if (i >= n) return;
+    float a = 0.f;
+    for (int s = 0; s < splits; ++s) a += part[s * n + i];
+    const int o = (int)(i / (k * CONV_DIM)), rem = (int)(i % (k * CONV_DIM)), tap = rem / CONV_DIM, c = rem % CONV_DIM;
+    dw[((long long)o * CONV_DIM + c) * k + tap] = a;
+}
+
+// conv0 + GroupNorm parameter gradients, pass 1.  D = dL/du0 (u0 = GroupNorm output; the forward saved gelu' itself for
+// level 0, so the level-1 dgrad wrote D), uhat = (conv0 - mean) * rstd:  per (utt, channel) fp64 sums of D, D * uhat and
+// D * x[5t + j] (j < 10).  One block = 4 x 64 level-0 rows (a 64-row group never straddles two utterances).
+static constexpr int C0W_SUMS = 12;
+__global__ void __launch_bounds__(256) conv0_wgrad_stats_kernel(const op_t* __restrict__ D, const float* __restrict__ wav,
+                                                                const UttMeta* __restrict__ meta, int B, long long groups,
+                                                                const float* __restrict__ w0, const float* __restrict__ stat,
+                                                                double* __restrict__ sums) {
+    __shared__ float xs[64 * 5 + 8];
+    const int c = 2 * threadIdx.x;
+    float wa[10], wb[10];
+#pragma unroll
+    for (int j = 0; j < 10; ++j) { wa[j] = __ldg(w0 + c * 10 + j); wb[j] = __ldg(w0 + (c + 1) * 10 + j); }
+    float acc[2][C0W_SUMS];
+    int cur = -1;
+    float mean_a = 0.f, rstd_a = 0.f, mean_b = 0.f, rstd_b = 0.f;
+    auto flush = [&]() {
+        if (cur < 0) return;
+        double* o = sums + ((long long)cur * CONV_DIM + c) * C0W_SUMS;
+#pragma unroll
+        for (int i = 0; i < C0W_SUMS; ++i) {
+            atomicAdd(o + i, (double)acc[0][i]);
+            atomicAdd(o + C0W_SUMS + i, (double)acc[1][i]);
+        }
+    };
+    for (int q = 0; q < 4; ++q) {
+        const long long grp = (long long)blockIdx.x * 4 + q;
+        if (grp >= groups) break;
+        const int b = find_utt_by_frame(meta, B, (int)grp);
+        const UttMeta m = meta[b];
+        const int t_base = (int)(grp * 64) - m.row0;
+        const int valid = min(64, m.T0 - t_base);
+        if (valid <= 0) continue;
+        if (b != cur) {
+            flush();
+            cur = b;
+#pragma unroll
+            for (int i = 0; i < C0W_SUMS; ++i) { acc[0][i] = 0.f; acc[1][i] = 0.f; }
+            mean_a = stat[((long long)b * CONV_DIM + c) * 2]; rstd_a = stat[((long long)b * CONV_DIM + c) * 2 + 1];
+            mean_b = stat[((long long)b * CONV_DIM + c + 1) * 2]; rstd_b = stat[((long long)b * CONV_DIM + c + 1) * 2 + 1];
+        }
+        __syncthreads();
+        const float* x = wav + m.wav_off;
+        for (int i = threadIdx.x; i < 64 * 5 + 5; i += blockDim.x) {
+            const long long s = (long long)t_base * 5 + i;
+            xs[i] = (s < m.n) ? __ldg(x + s) : 0.f;
+        }
+        __syncthreads();
+        const uint32_t* gp = reinterpret_cast<const uint32_t*>(D + grp * 64 * CONV_DIM + c);
+        for (int t = 0; t < valid; ++t) {
+            const float2 g = unpack_op(gp[(long long)t * (CONV_DIM / 2)]);
+            float ua = 0.f, ub = 0.f;
+#pragma unroll
+            for (int j = 0; j < 10; ++j) {
+                const float xv = xs[5 * t + j];
+                ua = fmaf(wa[j], xv, ua);
+                ub = fmaf(wb[j], xv, ub);
+                acc[0][2 + j] = fmaf(g.x, xv, acc[0][2 + j]);
+                acc[1][2 + j] = fmaf(g.y, xv, acc[1][2 + j]);
+            }
+            ua = (ua - mean_a) * rstd_a;
+            ub = (ub - mean_b) * rstd_b;
+            acc[0][0] += g.x; acc[0][1] = fmaf(g.x, ua, acc[0][1]);
+            acc[1][0] += g.y; acc[1][1] = fmaf(g.y, ub, acc[1][1]);
+        }
+    }
+    flush();
+}
+
+// pass 2 (one thread per channel, fp64): with a = gamma rstd, G0 = a D, m1 = mean_t G0, m2 = mean_t G0 uhat and the
+// waveform's tap sums S_j / cross-products C_kj (the forward's wave-stats partials):
+//   dW0[c][j] = sum_b  a P_j - m1 S_j - m2 rstd (sum_k w_k C_kj - mean S_j),  P_j = sum_t D x[5t + j]
+//   d gamma_c = sum_b sum_t D uhat,  d beta_c = sum_b sum_t D
+// (dL/dconv0 = G0 - m1 - uhat m2, times x[5t + j] summed over t; sum_t uhat x[5t + j] = rstd (sum_k w_k C_kj - mean S_j)).
+__global__ void __launch_bounds__(512) conv0_param_grad_kernel(const double* __restrict__ sums, const double* __restrict__ part,
+                                                               const UttMeta* __restrict__ meta, int B, int max_chunks,
+                                                               const float* __restrict__ w0, const float* __restrict__ gn_g,
+                                                               float* __restrict__ dw0, float* __restrict__ d_gamma,
+                                                               float* __restrict__ d_beta) {
+    const int c = threadIdx.x;
+    __shared__ double st[NSTAT], cr[10][10];
+    double w[10], dw[10], dg = 0.0, db = 0.0;
+#pragma unroll
+    for (int j = 0; j < 10; ++j) { w[j] = (double)w0[c * 10 + j]; dw[j] = 0.0; }
+    for (int b = 0; b < B; ++b) {
+        const UttMeta m = meta[b];
+        __syncthreads();
+        if (c < NSTAT) {
+            const int chunks = (m.T0 + STAT_CHUNK - 1) / STAT_CHUNK;
+            double a = 0.0;
+            for (int k = 0; k < chunks; ++k) a += part[((long long)b * max_chunks + k) * NSTAT + c];
+            st[c] = a;
+        }
+        __syncthreads();
+        if (c < 100) {  // C_jk from the upper triangle (wave_stats_kernel's order)
+            const int j = c / 10, k = c % 10, lo = min(j, k), hi = max(j, k);
+            cr[j][k] = st[10 + lo * 10 - lo * (lo - 1) / 2 + (hi - lo)];
+        }
+        __syncthreads();
+        // GroupNorm statistics (gn_fold_kernel's arithmetic up to the summation order): wc_j = sum_k w_k C_kj
+        double wc[10], sum = 0.0, sq = 0.0;
+#pragma unroll
+        for (int j = 0; j < 10; ++j) {
+            double a = 0.0;
+            for (int k = 0; k < 10; ++k) a += w[k] * cr[k][j];
+            wc[j] = a;
+            sum += w[j] * st[j];
+            sq += w[j] * a;
+        }
+        const double inv_n = 1.0 / (double)m.T0;
+        const double mean = sum * inv_n;
+        double var = sq * inv_n - mean * mean;
+        var = var > 0.0 ? var : 0.0;
+        const double rstd = 1.0 / sqrt(var + 1e-5);
+        const double a = (double)gn_g[c] * rstd;
+        const double* q = sums + ((long long)b * CONV_DIM + c) * C0W_SUMS;
+        db += q[0];
+        dg += q[1];
+        const double m1 = a * q[0] * inv_n, m2 = a * q[1] * inv_n;
+#pragma unroll
+        for (int j = 0; j < 10; ++j) dw[j] += a * q[2 + j] - m1 * st[j] - m2 * rstd * (wc[j] - mean * st[j]);
+    }
+#pragma unroll
+    for (int j = 0; j < 10; ++j) dw0[c * 10 + j] = (float)dw[j];
+    d_gamma[c] = (float)dg;
+    d_beta[c] = (float)db;
+}
+
 // ---- hooks called from backward_chain --------------------------------------------------------------------------
+static bool train_conv(const TrainCtx* tc) { return tc->conv_grads != nullptr; }
+
+// weight gradient of conv level l (1..6) from its pre-GELU gradient gu (M rows) and its input y_in (y_rows rows)
+static int train_hook_conv(TrainCtx* tc, int l, const op_t* gu, const op_t* y_in, long long y_rows, long long M, cudaStream_t st) {
+    const int k = CONV_KERNEL[l];
+    long long Ks;
+    const int splits = conv_splits(M, &Ks);
+    const unsigned tiles = (unsigned)(splits * Ks / 64);
+    conv_wgrad_transpose_kernel<<<dim3(tiles, CONV_DIM / 64, 1), 256, 0, st>>>(gu, M, 1, M, Ks, tc->ctA);
+    NB_LAUNCHED();
+    conv_wgrad_transpose_kernel<<<dim3(tiles, CONV_DIM / 64, k), 256, 0, st>>>(y_in, y_rows, 2, M, Ks, tc->ctB);
+    NB_LAUNCHED();
+    const int Ki = k * CONV_DIM;
+    GemmOperand A{tc->ctA, CONV_DIM, Ks, CONV_DIM * Ks, 0};
+    GemmOperand Bw{tc->ctB, Ki, Ks, Ki * Ks, 0};
+    GemmEpilogue e = epi_linear(EPI_OUT_F32, nullptr, nullptr, tc->part, nullptr, Ki);
+    e.out_bstride = (long long)CONV_DIM * Ki;
+    NB_TRY(gemm_h16(st, A, Bw, CONV_DIM, Ki, (int)Ks, splits, e, 0));
+    conv_wgrad_reduce_kernel<<<(unsigned)((CONV_DIM * Ki + 255) / 256), 256, 0, st>>>(tc->part, splits, k,
+                                                                                     tc->conv_grads + ConvLayout::level(l));
+    NB_LAUNCHED();
+    return 0;
+}
+
+static int train_hook_conv0(TrainCtx* tc, const Workspace& ws, const op_t* D0, const float* wav, int B, long long R0,
+                            const Weights& w, cudaStream_t st) {
+    NB_CUDA(cudaMemsetAsync(tc->c0_sums, 0, 8ull * C0W_SUMS * CONV_DIM * B, st));
+    const long long groups = R0 / 64;
+    conv0_wgrad_stats_kernel<<<(unsigned)((groups + 3) / 4), 256, 0, st>>>(D0, wav, ws.meta, B, groups, w.conv0_w, ws.gn_stat,
+                                                                         tc->c0_sums);
+    NB_LAUNCHED();
+    float* G = tc->conv_grads;
+    conv0_param_grad_kernel<<<1, CONV_DIM, 0, st>>>(tc->c0_sums, ws.stat_part, ws.meta, B, tc->max_chunks, w.conv0_w, w.gn_g,
+                                                    G + ConvLayout::C0_W, G + ConvLayout::GN_G, G + ConvLayout::GN_B);
+    NB_LAUNCHED();
+    return 0;
+}
+
 static int train_hook_layer(Handle* h, const Workspace& ws, const LossBufs& L, TrainCtx* tc, int l, int stage, int B,
                             long long Fe, const float* g_running, cudaStream_t st) {
     const Weights& w = h->w;
@@ -1456,10 +1691,36 @@ size_t nomad_b200_triplet_workspace_bytes(int B, int64_t N) {
     return fwd + carve_loss(p, 3 * B, p.frames, p.rows0, pos_rows, true, nullptr, nullptr) + train_extra_bytes(p.frames, 3 * B) + 4096;
 }
 
+}  // extern "C"
+
+// extra scratch of the conv-encoder step: [ctA | ctB | part | c0_sums], carved from `base` (sizes only when null)
+static size_t carve_conv_train(long long R0, int U, void* base, TrainCtx* tc) {
+    const long long rows = R0 / 2 + 64LL * CONV_SPLIT_MAX;  // level 1 (the largest) plus the slices' padding
+    size_t o = 0;
+    auto take = [&](size_t bytes) {
+        size_t at = o;
+        o = (o + bytes + 1023) / 1024 * 1024;
+        return base ? (void*)((char*)base + at) : nullptr;
+    };
+    void* a = take(2ull * CONV_DIM * rows);
+    void* b = take(2ull * 3 * CONV_DIM * rows);
+    void* part = take(4ull * CONV_SPLIT_MAX * CONV_DIM * 3 * CONV_DIM);
+    void* sums = take(8ull * C0W_SUMS * CONV_DIM * U);
+    if (tc) {
+        tc->ctA = (op_t*)a;
+        tc->ctB = (op_t*)b;
+        tc->part = (float*)part;
+        tc->c0_sums = (double*)sums;
+    }
+    return o;
+}
+
 // wav_dev: 3B x N fp32 (anchors, then positives, then negatives); loss_dev: 1 float; grads_dev:
-// nomad_b200_triplet_grad_floats() floats (zeroed here) = grad_scale_out[0] * d loss / d parameter.
-int nomad_b200_triplet_fwd_bwd(nomad_b200_handle* hh, const float* wav_dev, int B, int64_t N, float margin, float* loss_dev,
-                               float* grads_dev, float* grad_scale_out, void* workspace_dev, size_t workspace_bytes, void* stream) {
+// nomad_b200_triplet_grad_floats() floats (zeroed here) = grad_scale_out[0] * d loss / d parameter.  conv_grads_dev non-null:
+// the conv feature encoder is trained too (its gradients, times fgm, go there) and the workspace holds the conv scratch.
+static int triplet_run(nomad_b200_handle* hh, const float* wav_dev, int B, int64_t N, float margin, float fgm, float* loss_dev,
+                       float* grads_dev, float* conv_grads_dev, float* grad_scale_out, void* workspace_dev, size_t workspace_bytes,
+                       void* stream) {
     NB_CHECK(hh != nullptr, "null nomad_b200 handle");
     Handle* h = &hh->h;
     NB_CHECK(wav_dev && loss_dev && grads_dev && grad_scale_out && workspace_dev, "triplet: null pointer");
@@ -1478,9 +1739,11 @@ int nomad_b200_triplet_fwd_bwd(nomad_b200_handle* hh, const float* wav_dev, int 
     LossBufs L;
     const size_t loss_bytes = carve_loss(p, U, F, R0, pos_rows, true, (char*)workspace_dev + fwd_bytes, &L);
     const size_t extra = train_extra_bytes(F, U);
-    NB_CHECK(workspace_bytes >= fwd_bytes + loss_bytes + extra, "triplet: workspace too small (%zu < %zu bytes)", workspace_bytes,
-             fwd_bytes + loss_bytes + extra);
+    const size_t conv_bytes = conv_grads_dev != nullptr ? carve_conv_train(R0, U, nullptr, nullptr) : 0;
+    NB_CHECK(workspace_bytes >= fwd_bytes + loss_bytes + extra + conv_bytes, "triplet: workspace too small (%zu < %zu bytes)",
+             workspace_bytes, fwd_bytes + loss_bytes + extra + conv_bytes);
     TrainCtx tc;
+    memset(&tc, 0, sizeof(tc));
     {
         auto al = [](size_t v) { return (v + 1023) / 1024 * 1024; };
         char* q = (char*)workspace_dev + fwd_bytes + loss_bytes;
@@ -1491,6 +1754,13 @@ int nomad_b200_triplet_fwd_bwd(nomad_b200_handle* hh, const float* wav_dev, int 
         tc.x_tmp = (float*)q; q += al(4ull * EMBED * F);
         tc.gy = (float*)q;
         tc.grads = grads_dev;
+    }
+    if (conv_grads_dev != nullptr) {
+        NB_CHECK(((uintptr_t)conv_grads_dev & 15) == 0, "triplet: conv gradient buffer must be 16-byte aligned");
+        carve_conv_train(R0, U, (char*)workspace_dev + fwd_bytes + loss_bytes + extra, &tc);
+        tc.conv_grads = conv_grads_dev;
+        tc.max_chunks = p.max_chunks;
+        ws.aux0_raw = true;
     }
     NB_TRY(upload_meta(h, p, ws, st));
     NB_CUDA(cudaMemsetAsync(grads_dev, 0, sizeof(float) * TrainLayout::TOTAL, st));
@@ -1508,7 +1778,52 @@ int nomad_b200_triplet_fwd_bwd(nomad_b200_handle* hh, const float* wav_dev, int 
     head_pool_grad_kernel<<<U, 256, 0, st>>>(tc.gy, L.pooled, ws.meta, w.head_wt, L.g_pool);
     NB_LAUNCHED();
     *grad_scale_out = S;
-    return backward_chain(h, ws, L, U, F, R0, pos_rows, p.max_T, 0.f, 1.0f, S, wav_dev, N, nullptr, st, &tc);
+    return backward_chain(h, ws, L, U, F, R0, pos_rows, p.max_T, 0.f, conv_grads_dev != nullptr ? fgm : 1.0f, S, wav_dev, N,
+                          nullptr, st, &tc);
+}
+
+extern "C" {
+
+int nomad_b200_triplet_fwd_bwd(nomad_b200_handle* hh, const float* wav_dev, int B, int64_t N, float margin, float* loss_dev,
+                               float* grads_dev, float* grad_scale_out, void* workspace_dev, size_t workspace_bytes, void* stream) {
+    return triplet_run(hh, wav_dev, B, N, margin, 1.0f, loss_dev, grads_dev, nullptr, grad_scale_out, workspace_dev,
+                       workspace_bytes, stream);
+}
+
+int64_t nomad_b200_triplet_conv_grad_floats(void) { return ConvLayout::TOTAL; }
+
+int nomad_b200_triplet_conv_grad_segment(int i, char* name, int name_cap, int64_t* offset, int64_t* numel) {
+    if (i < 0 || i >= 9 || name == nullptr || offset == nullptr || numel == nullptr) return 1;
+    const char* P = "ssl_model.feature_extractor.conv_layers.";
+    if (i < 3) {
+        static const char* leaf[3] = {"0.0.weight", "0.2.weight", "0.2.bias"};
+        static const long long off[3] = {ConvLayout::C0_W, ConvLayout::GN_G, ConvLayout::GN_B}, cnt[3] = {512 * 10, 512, 512};
+        snprintf(name, name_cap, "%s%s", P, leaf[i]);
+        *offset = off[i];
+        *numel = cnt[i];
+        return 0;
+    }
+    const int l = i - 2;
+    snprintf(name, name_cap, "%s%d.0.weight", P, l);
+    *offset = ConvLayout::level(l);
+    *numel = 512LL * 512 * CONV_KERNEL[l];
+    return 0;
+}
+
+size_t nomad_b200_triplet_conv_workspace_bytes(int B, int64_t N) {
+    const size_t base = nomad_b200_triplet_workspace_bytes(B, N);
+    if (base == 0) return 0;
+    Plan p;
+    if (triplet_plan(B, N, &p)) return 0;
+    return base + carve_conv_train(p.rows0, 3 * B, nullptr, nullptr);
+}
+
+int nomad_b200_triplet_conv_fwd_bwd(nomad_b200_handle* hh, const float* wav_dev, int B, int64_t N, float margin,
+                                    float feature_grad_mult, float* loss_dev, float* grads_dev, float* conv_grads_dev,
+                                    float* grad_scale_out, void* workspace_dev, size_t workspace_bytes, void* stream) {
+    NB_CHECK(conv_grads_dev != nullptr, "triplet_conv: null conv gradient buffer");
+    return triplet_run(hh, wav_dev, B, N, margin, feature_grad_mult, loss_dev, grads_dev, conv_grads_dev, grad_scale_out,
+                       workspace_dev, workspace_bytes, stream);
 }
 
 }  // extern "C"

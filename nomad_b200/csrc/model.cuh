@@ -118,6 +118,8 @@ struct LayerBufs {
 struct Workspace {
     bool save;
     bool train;          // save mode + what the parameter gradients need (per-layer FFN activations)
+    bool aux0_raw;       // save mode, conv encoder training: aux[0] holds gelu' itself (the GroupNorm affine
+                         // gradients need dL/du0 without the gamma * rstd factor, and gamma may be 0)
     UttMeta* meta;       // [B]
     uint32_t* attn_items;  // [Plan::attn_items.size()] work list of the attention kernel
     double* stat_part;   // [B][max_chunks][65]
@@ -125,7 +127,7 @@ struct Workspace {
     op_t* c0_fold_h;     // [B][512][32]: the folded taps as 16-bit hi | lo halves, K padded to 16 (tensor-core conv0)
     float* gn_stat;      // save mode: [B][512][2] mean and rstd of the raw conv0 output per (utt, channel)
     op_t* y[7];          // conv level outputs, level l: (rows0 >> l) + 8 rows x 512
-    op_t* aux[7];        // save mode: gelu'(pre-activation) per level (level 0: times gamma * rstd)
+    op_t* aux[7];        // save mode: gelu'(pre-activation) per level (level 0: times gamma * rstd unless aux0_raw)
     op_t* ln0_out;       // LayerNorm(512) output, frames x 512
     float* x0;           // feature projection output, frames x 768 fp32
     op_t* pos_g;         // [16][pos_rows + 128][48]

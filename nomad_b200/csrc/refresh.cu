@@ -3,8 +3,10 @@
 // nomad_b200_create does the same preparation on the host from host tensors (api.cu: build_weights: fp16 conversion, q-scale,
 // q/k/v fusion, transposes for the dgrad GEMMs, LayerNorm folds, weight-norm fold of the positional conv); repeating that per
 // training step would cost seconds.  Here it is a handful of bandwidth-bound kernels (~190 MB of fp32 read, ~0.5 GB written).
-// The conv feature encoder is frozen in the reference's configuration (`freeze_convnet: True`) and is not touched; the
-// fp32-class weight planes (precision_mode 1) are not rebuilt either: fine-tuning runs the fp16-operand path.
+// nomad_b200_refresh_weights rebuilds everything after the conv feature encoder, which the reference's default
+// configuration freezes (`freeze_convnet: True`); with `freeze_convnet: False` nomad_b200_refresh_conv_weights rebuilds the
+// encoder's buffers too.  The fp32-class weight planes (precision_mode 1) are not rebuilt: fine-tuning runs the fp16-operand
+// path.
 #include <cstdlib>
 #include <cstring>
 #include <string>
@@ -98,6 +100,24 @@ __global__ void __launch_bounds__(256) rf_pos_fold_kernel(const float* __restric
     const op_t q = f2op((float)((double)v[i] * scale[k]));
     fw[(long long)on * (POS_K * POS_GC) + (long long)k * POS_GC + c] = q;
     bw[(long long)(g * POS_GC + c) * (POS_K * POS_GC) + (long long)(POS_K - 1 - k) * POS_GC + n] = q;
+}
+
+// conv layer with k taps: W (cout, cin, tap) fp32 -> conv_w [cout][tap * 512 + cin], conv_wt [tap][cin][cout] and, for
+// k = 3, conv_wte [cin][tap 2: cout | tap 0: cout] (api.cu: build_weights)
+__global__ void __launch_bounds__(256) rf_conv_kernel(const float* __restrict__ W, int k, op_t* __restrict__ fw,
+                                                      op_t* __restrict__ bw, op_t* __restrict__ ew) {
+    const long long i = (long long)blockIdx.x * 256 + threadIdx.x;
+    if (i >= 512LL * 512 * k) return;
+    const int j = (int)(i % k), c = (int)((i / k) % 512), o = (int)(i / (512LL * k));
+    const op_t v = f2op(W[i]);
+    fw[(long long)o * (k * 512) + j * 512 + c] = v;
+    bw[((long long)j * 512 + c) * 512 + o] = v;
+    if (ew != nullptr && j != 1) ew[(long long)c * 1024 + (j == 2 ? 0 : 512) + o] = v;
+}
+// conv0 taps w[c][j] -> conv0_wh [16][512] (rows 10..15 stay zero)
+__global__ void rf_conv0_kernel(const float* __restrict__ W, op_t* __restrict__ wh) {
+    const int i = blockIdx.x * 256 + threadIdx.x;
+    if (i < 512 * 10) wh[(i % 10) * 512 + i / 10] = f2op(W[i]);
 }
 
 static int convert(cudaStream_t st, const float* src, int R, int C, float scale, int scaled_rows, op_t* dst, op_t* dst_t,
@@ -207,8 +227,47 @@ extern "C" int nomad_b200_refresh_weights(nomad_b200_handle* hh, const nomad_b20
     return 0;
 }
 
+extern "C" int nomad_b200_refresh_conv_weights(nomad_b200_handle* hh, const nomad_b200_tensor* tensors_dev, int n_tensors,
+                                               void* stream) {
+    NB_CHECK(hh != nullptr && tensors_dev != nullptr && n_tensors > 0, "refresh_conv_weights: bad arguments");
+    Handle* h = &hh->h;
+    NB_CHECK(!h->pw.built || h->precision == NOMAD_B200_PRECISION_FP16,
+             "refresh_conv_weights: the fp32-class weight planes are not rebuilt; switch the handle to precision_mode 0 for fine-tuning");
+    NB_CUDA(cudaSetDevice(h->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    std::unordered_map<std::string, const nomad_b200_tensor*> map;
+    for (int i = 0; i < n_tensors; ++i)
+        if (tensors_dev[i].name && tensors_dev[i].data) map[tensors_dev[i].name] = &tensors_dev[i];
+    const std::string P = "ssl_model.feature_extractor.conv_layers.";
+    const float* src[9];
+    const char* leaf[3] = {"0.0.weight", "0.2.weight", "0.2.bias"};
+    for (int i = 0; i < 9; ++i) {
+        const std::string name = i < 3 ? P + leaf[i] : P + std::to_string(i - 2) + ".0.weight";
+        const long long numel = i == 0 ? 512 * 10 : i < 3 ? 512 : 512LL * 512 * CONV_KERNEL[i - 2];
+        auto it = map.find(name);
+        NB_CHECK(it != map.end(), "refresh_conv_weights: missing tensor %s", name.c_str());
+        NB_CHECK(it->second->numel == numel, "refresh_conv_weights: tensor %s has %lld elements, expected %lld", name.c_str(),
+                 (long long)it->second->numel, numel);
+        src[i] = it->second->data;
+    }
+    Weights& w = h->w;
+    NB_TRY(copy_f32(st, src[0], 512 * 10, 1.f, w.conv0_w));
+    NB_TRY(copy_f32(st, src[1], 512, 1.f, w.gn_g));
+    NB_TRY(copy_f32(st, src[2], 512, 1.f, w.gn_b));
+    rf_conv0_kernel<<<(512 * 10 + 255) / 256, 256, 0, st>>>(src[0], w.conv0_wh);
+    NB_LAUNCHED();
+    for (int l = 1; l < 7; ++l) {
+        const int k = CONV_KERNEL[l];
+        rf_conv_kernel<<<(unsigned)((512LL * 512 * k + 255) / 256), 256, 0, st>>>(src[l + 2], k, w.conv_w[l], w.conv_wt[l],
+                                                                                  k == 3 ? w.conv_wte[l] : nullptr);
+        NB_LAUNCHED();
+    }
+    return 0;
+}
+
 // Test hook: copy one kernel-ready weight buffer to the host (synchronous).  which: "pos_w" | "pos_wt" | "l<k>.w_fc1_f" |
-// "l<k>.s_fc1" | "l<k>.c_fc1" | "l<k>.w_qkv_f" | "l<k>.s_qkv" | "l<k>.c_qkv" | "l<k>.w_qkv" | "l<k>.wt_fc2" | "head_wt"
+// "l<k>.s_fc1" | "l<k>.c_fc1" | "l<k>.w_qkv_f" | "l<k>.s_qkv" | "l<k>.c_qkv" | "l<k>.w_qkv" | "l<k>.wt_fc2" | "head_wt" |
+// conv encoder: "conv0_w" | "gn_g" | "gn_b" | "conv0_wh" | "c<l>.w" | "c<l>.wt" | "c<l>.wte" (l = 1..6; wte for k = 3)
 extern "C" int nomad_b200_debug_read_weight(nomad_b200_handle* hh, const char* which, void* dst_host, size_t bytes) {
     NB_CHECK(hh && which && dst_host, "debug_read_weight: bad arguments");
     Weights& w = hh->h.w;
@@ -217,6 +276,15 @@ extern "C" int nomad_b200_debug_read_weight(nomad_b200_handle* hh, const char* w
     if (s == "pos_w") src = w.pos_w;
     else if (s == "pos_wt") src = w.pos_wt;
     else if (s == "head_wt") src = w.head_wt;
+    else if (s == "conv0_w") src = w.conv0_w;
+    else if (s == "gn_g") src = w.gn_g;
+    else if (s == "gn_b") src = w.gn_b;
+    else if (s == "conv0_wh") src = w.conv0_wh;
+    else if (s.size() > 2 && s[0] == 'c' && s[1] >= '1' && s[1] <= '6' && s[2] == '.') {
+        const int l = s[1] - '0';
+        const std::string f = s.substr(3);
+        if (f == "w") src = w.conv_w[l]; else if (f == "wt") src = w.conv_wt[l]; else if (f == "wte") src = w.conv_wte[l];
+    }
     else if (s.size() > 2 && s[0] == 'l') {
         const size_t dot = s.find('.');
         NB_CHECK(dot != std::string::npos, "debug_read_weight: bad name %s", which);

@@ -86,10 +86,19 @@ class Engine:
 
     def refresh_weights(self, state_dict_dev):
         """Rebuild the kernel-ready weights from fp32 master tensors on THIS device (``nomad_b200_refresh_weights``): the step
-        after an optimiser update.  ``state_dict_dev``: {state_dict key: contiguous fp32 CUDA tensor}; conv encoder frozen."""
+        after an optimiser update.  ``state_dict_dev``: {state_dict key: contiguous fp32 CUDA tensor}.  Everything after
+        the conv feature encoder; ``refresh_conv_weights`` rebuilds the encoder."""
+        self._refresh(state_dict_dev, False)
+
+    def refresh_conv_weights(self, state_dict_dev):
+        """The same for the conv feature encoder (``nomad_b200_refresh_conv_weights``), in place: pointers captured by
+        loss-step CUDA graphs stay valid."""
+        self._refresh(state_dict_dev, True)
+
+    def _refresh(self, state_dict_dev, conv: bool):
         names, ptrs, keep = [], [], []
         for k, v in state_dict_dev.items():
-            if not torch.is_tensor(v) or k.endswith("mask_emb") or "feature_extractor" in k:
+            if not torch.is_tensor(v) or k.endswith("mask_emb") or ("feature_extractor" in k) != conv:
                 continue
             t = v.detach()
             assert t.is_cuda and t.device == self.device and t.dtype == torch.float32 and t.is_contiguous(), k
@@ -100,7 +109,8 @@ class Engine:
             tens[i].data = C.c_void_p(p_)
             tens[i].numel = t.numel()
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.nomad_b200_refresh_weights(self.handle, tens, len(names), _stream_ptr()), "nomad_b200_refresh_weights")
+            fn = "nomad_b200_refresh_conv_weights" if conv else "nomad_b200_refresh_weights"
+            _lib.check(getattr(self.lib, fn)(self.handle, tens, len(names), _stream_ptr()), fn)
 
     def set_loss_head(self, weight: torch.Tensor, bias: torch.Tensor):
         w = np.ascontiguousarray(weight.detach().to(torch.float32).cpu().numpy())

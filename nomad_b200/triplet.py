@@ -1,12 +1,14 @@
 """Triplet fine-tuning step of the reference (``src/training/train_triplet.py:92-133``) on the B200 path.
 
 ``Training.train`` runs, per batch of (anchor, positive, negative) waveforms: three forwards of ``TripletModel``,
-``nn.TripletMarginLoss(margin)``, ``loss.backward()`` and an Adam step over everything but the frozen conv feature
-encoder (``freeze_convnet: True``), with lr 1e-5 for the pre-trained network and ``lr`` for the embedding head
-(``:96-104``).  Here the three forwards, the loss and ALL parameter gradients come from one C-ABI call
-(``nomad_b200_triplet_fwd_bwd``: tensor-core forward, dgrad chain, weight-gradient GEMMs); the optimiser state and the
-update are host plumbing (``torch.optim.Adam`` on fp32 master tensors on the GPU), after which the kernel-ready
-weights are rebuilt on the device from those tensors (``nomad_b200_refresh_weights``).
+``nn.TripletMarginLoss(margin)``, ``loss.backward()`` and an Adam step with lr 1e-5 for the pre-trained network and
+``lr`` for the embedding head (``:96-104``), over everything but the conv feature encoder when ``freeze_convnet: True``
+(the default of ``src/config/train_triplet.yaml``) and over the encoder too when it is ``False``.  Here the three
+forwards, the loss and ALL parameter gradients come from one C-ABI call (``nomad_b200_triplet_fwd_bwd``, or
+``nomad_b200_triplet_conv_fwd_bwd`` with the encoder trained: tensor-core forward, dgrad chain, weight-gradient GEMMs);
+the optimiser state and the update are host plumbing (``torch.optim.Adam`` on fp32 master tensors on the GPU), after
+which the kernel-ready weights are rebuilt on the device from those tensors (``nomad_b200_refresh_weights``, plus
+``nomad_b200_refresh_conv_weights`` for a trained encoder).
 
 Deliberate difference from the reference: the network runs in evaluation mode (no dropout / LayerDrop: fairseq's
 ``Wav2Vec2Model`` applies dropout 0.1 and layerdrop 0.05 under ``model.train()``, which makes the reference's step
@@ -24,13 +26,15 @@ from . import _lib
 from .engine import Engine, _ptr, _stream_ptr
 
 
-def grad_segments():
-    """[(name, offset, numel)] of the flat gradient buffer, as the library lays it out."""
+def grad_segments(conv: bool = False):
+    """[(name, offset, numel)] of the flat gradient buffer (``conv``: of the conv-encoder buffer), as the library lays it
+    out."""
     lib = _lib.load()
+    seg = lib.nomad_b200_triplet_conv_grad_segment if conv else lib.nomad_b200_triplet_grad_segment
     out, i = [], 0
     name = C.create_string_buffer(128)
     off, cnt = C.c_int64(), C.c_int64()
-    while lib.nomad_b200_triplet_grad_segment(i, name, 128, C.byref(off), C.byref(cnt)) == 0:
+    while seg(i, name, 128, C.byref(off), C.byref(cnt)) == 0:
         out.append((name.value.decode(), int(off.value), int(cnt.value)))
         i += 1
     return out
@@ -57,14 +61,17 @@ SHAPES = {"qkv.weight": (2304, 768), "self_attn.out_proj.weight": (768, 768), "f
 
 
 def triplet_loss_and_grads(engine: Engine, state_dict, anchor: torch.Tensor, positive: torch.Tensor, negative: torch.Tensor,
-                           margin: float = 0.2) -> Tuple[torch.Tensor, "OrderedDict[str, torch.Tensor]"]:
-    """loss (0-dim CUDA tensor) and {state_dict key: gradient} for every trainable tensor (conv encoder frozen).
+                           margin: float = 0.2, freeze_convnet: bool = True,
+                           feature_grad_mult: float = 0.1) -> Tuple[torch.Tensor, "OrderedDict[str, torch.Tensor]"]:
+    """loss (0-dim CUDA tensor) and {state_dict key: gradient} for every trainable tensor.  ``freeze_convnet=False``
+    trains the conv feature encoder too: its 9 tensors join the result, with fairseq's GradMultiply of
+    ``feature_grad_mult`` on the conv features (the frozen step has no gradient below the conv features for it to scale).
     ``anchor`` / ``positive`` / ``negative``: (B, N) or (B, 1, N) waveforms of one common length."""
     lib = engine.lib
     sq = lambda t: (t.squeeze(1) if t.dim() == 3 else t).to(engine.device, torch.float32)
     wav = torch.cat([sq(anchor), sq(positive), sq(negative)]).contiguous()
     B, N = wav.shape[0] // 3, wav.shape[1]
-    need = lib.nomad_b200_triplet_workspace_bytes(B, N)
+    need = (lib.nomad_b200_triplet_workspace_bytes if freeze_convnet else lib.nomad_b200_triplet_conv_workspace_bytes)(B, N)
     if need == 0:
         raise _lib.NomadB200Error(lib.nomad_b200_last_error().decode())
     wp, wbytes = engine._aligned(engine.workspace(need))
@@ -73,8 +80,15 @@ def triplet_loss_and_grads(engine: Engine, state_dict, anchor: torch.Tensor, pos
     loss = torch.empty((), dtype=torch.float32, device=engine.device)
     scale = C.c_float()
     with torch.cuda.device(engine.device):
-        _lib.check(lib.nomad_b200_triplet_fwd_bwd(engine.handle, _ptr(wav), B, N, C.c_float(margin), _ptr(loss), _ptr(flat),
-                                                  C.byref(scale), wp, wbytes, _stream_ptr()), "nomad_b200_triplet_fwd_bwd")
+        if freeze_convnet:
+            _lib.check(lib.nomad_b200_triplet_fwd_bwd(engine.handle, _ptr(wav), B, N, C.c_float(margin), _ptr(loss), _ptr(flat),
+                                                      C.byref(scale), wp, wbytes, _stream_ptr()), "nomad_b200_triplet_fwd_bwd")
+        else:
+            conv_flat = torch.empty((int(lib.nomad_b200_triplet_conv_grad_floats()),), dtype=torch.float32, device=engine.device)
+            _lib.check(lib.nomad_b200_triplet_conv_fwd_bwd(engine.handle, _ptr(wav), B, N, C.c_float(margin),
+                                                           C.c_float(feature_grad_mult), _ptr(loss), _ptr(flat), _ptr(conv_flat),
+                                                           C.byref(scale), wp, wbytes, _stream_ptr()),
+                       "nomad_b200_triplet_conv_fwd_bwd")
     flat = flat / scale.value
     grads: "OrderedDict[str, torch.Tensor]" = OrderedDict()
     for name, off, cnt in grad_segments():
@@ -100,19 +114,27 @@ def triplet_loss_and_grads(engine: Engine, state_dict, anchor: torch.Tensor, pos
             grads["ssl_model.encoder.pos_conv.0.weight_g"] = gg.grad
         else:
             grads[name] = g
+    if not freeze_convnet:
+        conv_flat = conv_flat / scale.value
+        for name, off, cnt in grad_segments(conv=True):   # already in the checkpoint's (out, in, tap) order
+            grads[name] = conv_flat[off:off + cnt].view(state_dict[name].shape)
     return loss, grads
 
 
 class TripletTrainer:
-    """``Training.train``'s inner step (``train_triplet.py:112-133``) with the optimiser of ``:92-107``."""
+    """``Training.train``'s inner step (``train_triplet.py:112-133``) with the optimiser of ``:92-107``.
+    ``freeze_convnet=False`` trains the conv feature encoder as well (its tensors are part of ``ssl_model`` and take
+    ``lr_pretrained``), with ``nomad.feature_grad_mult`` on the conv features as fairseq applies it."""
 
-    def __init__(self, nomad, lr: float = 1e-4, margin: float = 0.2, lr_pretrained: float = 1e-5):
+    def __init__(self, nomad, lr: float = 1e-4, margin: float = 0.2, lr_pretrained: float = 1e-5,
+                 freeze_convnet: bool = True):
         self.nomad = nomad
         self.margin = margin
+        self.freeze_convnet = freeze_convnet
         dev = nomad.engine.device
         self.master = OrderedDict((k, v.detach().to(dev, torch.float32).clone()) for k, v in self._state_dict(nomad).items())
         head = ["embedding_layer.1.weight", "embedding_layer.1.bias"]
-        train = [k for k in self.master if "feature_extractor" not in k and not k.endswith("mask_emb")]
+        train = [k for k in self.master if not k.endswith("mask_emb") and not (freeze_convnet and "feature_extractor" in k)]
         for k in train:
             self.master[k].requires_grad_(True)
         self.optim = torch.optim.Adam([{"params": [self.master[k] for k in train if k not in head], "lr": lr_pretrained},
@@ -126,7 +148,8 @@ class TripletTrainer:
         return sd
 
     def step(self, anchor, positive, negative) -> float:
-        loss, grads = triplet_loss_and_grads(self.nomad.engine, self.master, anchor, positive, negative, self.margin)
+        loss, grads = triplet_loss_and_grads(self.nomad.engine, self.master, anchor, positive, negative, self.margin,
+                                             self.freeze_convnet, self.nomad.feature_grad_mult)
         self.optim.zero_grad(set_to_none=True)
         for k, g in grads.items():
             self.master[k].grad = g.reshape(self.master[k].shape).contiguous()
@@ -134,4 +157,6 @@ class TripletTrainer:
         # rebuild the kernel-ready weights (16-bit copies, q|k|v fusion, transposes, LayerNorm folds, weight-norm fold) from
         # the updated master tensors, on the device
         self.nomad.engine.refresh_weights(self.master)
+        if not self.freeze_convnet:
+            self.nomad.engine.refresh_conv_weights(self.master)
         return float(loss.item())
