@@ -138,6 +138,35 @@ NOMAD_B200_API int nomad_b200_layers_bwd(nomad_b200_handle* h, const void* saved
                                          float feature_grad_mult, float* d_wav_dev, void* workspace_dev,
                                          size_t workspace_bytes, void* stream);
 
+/* ---- parameter gradients through the same autograd forward (fine-tuning with any loss on the outputs) -------------
+ * nomad_b200_layers_fwd_save_ex is nomad_b200_layers_fwd_save plus `flags`: NOMAD_B200_SAVE_PARAMS also keeps what the
+ * weight gradients need (each layer's GELU(fc1) activations); NOMAD_B200_SAVE_CONV saves the conv0 GELU gradient without
+ * the GroupNorm gamma * rstd factor, as the conv-encoder gradients need it.  The flags are recorded in the saved buffer
+ * (size: nomad_b200_layers_saved_bytes_ex; flags 0 = nomad_b200_layers_saved_bytes).  A buffer saved with flags != 0 goes
+ * to nomad_b200_layers_bwd_params only.
+ * nomad_b200_layers_bwd_params: from the same g_layers / g_emb as nomad_b200_layers_bwd, the waveform gradient (d_wav,
+ * B x N, or NULL) and the gradient of every trainable parameter: grads (NULL, or nomad_b200_triplet_grad_floats() fp32
+ * values laid out as nomad_b200_triplet_grad_segment enumerates; needs SAVE_PARAMS), conv_grads (NULL = conv encoder
+ * frozen, or nomad_b200_triplet_conv_grad_floats() values as nomad_b200_triplet_conv_grad_segment; needs SAVE_CONV and
+ * grads).  The embedding-head slots hold the NOMAD head's gradient for a head-0 forward and zeros for head 1.  Every
+ * output is multiplied by the power-of-two scale S chosen on the device, which is written to *grad_scale_dev (device
+ * float): divide it out on the device.  The call reads the saved buffer's 16-byte record back before launching anything
+ * (one stream synchronisation) and refuses gradients the forward did not save for.  With d_wav NULL and the conv
+ * encoder frozen the conv-stack backward is skipped.  Workspace: nomad_b200_layers_bwd_params_workspace_bytes with the
+ * forward's flags.  grads / conv_grads / g_emb / g_layers[l]: 16-byte aligned. */
+#define NOMAD_B200_SAVE_PARAMS 1
+#define NOMAD_B200_SAVE_CONV 2
+NOMAD_B200_API size_t nomad_b200_layers_saved_bytes_ex(int B, int64_t N, int flags);
+NOMAD_B200_API int nomad_b200_layers_fwd_save_ex(nomad_b200_handle* h, const float* wav_dev, int B, int64_t N, int head,
+                                                 float* layers_dev, float* emb_dev, void* saved_dev, size_t saved_bytes,
+                                                 int flags, void* stream);
+NOMAD_B200_API size_t nomad_b200_layers_bwd_params_workspace_bytes(int B, int64_t N, int flags);
+NOMAD_B200_API int nomad_b200_layers_bwd_params(nomad_b200_handle* h, const void* saved_dev, size_t saved_bytes,
+                                                const float* wav_dev, int B, int64_t N, const float* const* g_layers,
+                                                const float* g_emb, float feature_grad_mult, float* d_wav_dev,
+                                                float* grads_dev, float* conv_grads_dev, float* grad_scale_dev,
+                                                void* workspace_dev, size_t workspace_bytes, void* stream);
+
 /* ---- distance: ``cdist(test, nmr)`` + ``np.mean(axis=1)`` (nomad.py:108,111) ---------------------
  * deg: n x 256, nmr: m x 256 fp32 device.  dm (n x m fp32 device, may be NULL when only the means are
  * wanted) and row_mean (n fp64 device; NaN when m == 0, like np.mean of an empty row).  Row means are summed in a

@@ -20,6 +20,8 @@ c_vp = C.c_void_p
 
 # NOMAD_B200_WAV_* sample formats -> bytes per sample
 WAV_U8, WAV_S16, WAV_S24, WAV_S32, WAV_F32, WAV_F64 = 1, 2, 3, 4, 5, 6
+# NOMAD_B200_SAVE_* flags of nomad_b200_layers_fwd_save_ex
+SAVE_PARAMS, SAVE_CONV = 1, 2
 FORMAT_BYTES = np.array([0, 1, 2, 3, 4, 4, 8], np.int64)
 
 # ``nomad_b200_ingest_item``
@@ -59,7 +61,13 @@ PROTOTYPES = {
     "nomad_b200_layers_bwd_workspace_bytes": (C.c_size_t, [C.c_int, c_i64]),
     "nomad_b200_layers_bwd": (C.c_int, [c_vp, c_vp, C.c_size_t, c_vp, C.c_int, c_i64, C.POINTER(c_vp), c_vp, C.c_float, c_vp,
                                         c_vp, C.c_size_t, c_vp]),
-    "nomad_b200_cdist_workspace_bytes": (C.c_size_t, [c_i64, c_i64]),
+    "nomad_b200_layers_saved_bytes_ex": (C.c_size_t, [C.c_int, c_i64, C.c_int]),
+    "nomad_b200_layers_fwd_save_ex": (C.c_int, [c_vp, c_vp, C.c_int, c_i64, C.c_int, c_vp, c_vp, c_vp, C.c_size_t, C.c_int,
+                                                c_vp]),
+    "nomad_b200_layers_bwd_params_workspace_bytes": (C.c_size_t, [C.c_int, c_i64, C.c_int]),
+    "nomad_b200_layers_bwd_params": (C.c_int, [c_vp, c_vp, C.c_size_t, c_vp, C.c_int, c_i64, C.POINTER(c_vp), c_vp, C.c_float,
+                                               c_vp, c_vp, c_vp, c_vp, c_vp, C.c_size_t, c_vp]),
+    "nomad_b200_cdist_workspace_bytes":(C.c_size_t, [c_i64, c_i64]),
     "nomad_b200_cdist_mean": (C.c_int, [c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, C.c_size_t, C.c_int, c_vp]),
     "nomad_b200_cdist_mean_host": (C.c_int, [c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, C.c_size_t, c_vp]),
     "nomad_b200_score_workspace_bytes": (C.c_size_t, [C.POINTER(c_i64), C.c_int, c_i64]),

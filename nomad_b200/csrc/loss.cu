@@ -526,6 +526,24 @@ __global__ void __launch_bounds__(256) conv0_bwd_stats_kernel(const op_t* __rest
     atomicAdd(o + 3, (double)s2b);
 }
 
+// With the conv encoder's forward saved for its parameter gradients (aux0 = gelu' alone), the level-1 dgrad wrote
+// dL/du0; G0 = dL/du0 * gamma_c * rstd_c per (utterance, channel), in place.  One block per 64 level-0 rows.
+__global__ void __launch_bounds__(256) conv0_gain_fold_kernel(op_t* __restrict__ G0, const UttMeta* __restrict__ meta, int B,
+                                                              const float* __restrict__ gn_g, const float* __restrict__ stat) {
+    const int b = find_utt_by_frame(meta, B, blockIdx.x);
+    const UttMeta m = meta[b];
+    const int t_base = blockIdx.x * 64 - m.row0;
+    const int valid = min(64, m.T0 - t_base);
+    const int c = 2 * threadIdx.x;
+    const float ga = __ldg(gn_g + c) * stat[((long long)b * CONV_DIM + c) * 2 + 1];
+    const float gb = __ldg(gn_g + c + 1) * stat[((long long)b * CONV_DIM + c + 1) * 2 + 1];
+    uint32_t* gp = reinterpret_cast<uint32_t*>(G0 + (long long)blockIdx.x * 64 * CONV_DIM + c);
+    for (int t = 0; t < valid; ++t) {
+        const float2 g = unpack_op(gp[(long long)t * (CONV_DIM / 2)]);
+        gp[(long long)t * (CONV_DIM / 2)] = pack_op(g.x * ga, g.y * gb);
+    }
+}
+
 // Per-utterance constants of the dgrad:  val(t, j) = V[t, j] - c1[j] + c2[j] - sum_j' x[5t + j'] Q[j'][j]
 //   c1[j] = sum_c m1_c w[c,j];  c2[j] = sum_c mean_c rstd_c m2_c w[c,j];  Q[j'][j] = sum_c w[c,j'] rstd_c m2_c w[c,j]
 // consts[b] = { cc[10] = c2 - c1, Q[100] }
@@ -695,7 +713,8 @@ size_t nomad_b200_loss_workspace_bytes(int B, int64_t N, int with_grad) {
 // triplet section below): also produce the parameter gradients of everything after the conv feature encoder, and stop
 // there when the encoder is frozen; when it is trained, go on through conv layers 6..1 (weight gradients from each
 // level's pre-GELU gradient) and stop at conv0 + GroupNorm, whose parameter gradients replace the waveform gradient.  `ug` (autograd path, nomad_b200_layers_bwd): caller-given upstream gradients of the layer outputs and the
-// pooled head instead of the L1 seeds, under a scale S that lives on the device.
+// pooled head instead of the L1 seeds, under a scale S that lives on the device.  Both (nomad_b200_layers_bwd_params):
+// the parameter gradients from the caller's gradients, and the waveform gradient too when d_est_dev is non-null.
 struct TrainCtx;
 struct UserGrads {
     const float* g_layers[LAYERS];  // gradient wrt layer l's output, B x T x 768 (caller layout), or null
@@ -703,6 +722,7 @@ struct UserGrads {
     const float* g_pool;            // [B][768] unscaled pooled-feature gradient of the head, or null
     const float* scale;             // device: S
     int top;                        // highest layer that receives a gradient; the layers above it are skipped
+    bool scaled_out;                // the waveform gradient keeps S (parameter path: every output carries S)
 };
 static int train_hook_layer(Handle* h, const Workspace& ws, const LossBufs& L, TrainCtx* tc, int l, int stage, int B,
                             long long Fe, const float* g_running, cudaStream_t st);
@@ -804,7 +824,7 @@ static int backward_chain(Handle* h, const Workspace& ws, const LossBufs& L, int
     }
     if (tc) {
         NB_TRY(train_hook_front(h, ws, L, tc, 3, B, Fe, pos_rows_e, st));  // LayerNorm(512) params
-        if (!train_conv(tc)) return 0;                                      // conv feature encoder frozen
+        if (!train_conv(tc) && d_est_dev == nullptr) return 0;              // conv encoder frozen, no waveform gradient
     }
     // conv stack backward.  Gradient buffers start 8 rows into their allocation so that "row -1" reads zeros.
     NB_CUDA(cudaMemsetAsync(L.gu_a, 0, 2ull * CONV_DIM * 8, st));
@@ -815,7 +835,7 @@ static int backward_chain(Handle* h, const Workspace& ws, const LossBufs& L, int
     NB_LAUNCHED();
     for (int l = 6; l >= 1; --l) {
         const long long M = R0e >> l;  // rows at level l (estimate half)
-        if (tc) NB_TRY(train_hook_conv(tc, l, gu[l], ws.y[l - 1], (R0e >> (l - 1)) + 8, M, st));  // before gu[l] is reused
+        if (tc && train_conv(tc)) NB_TRY(train_hook_conv(tc, l, gu[l], ws.y[l - 1], (R0e >> (l - 1)) + 8, M, st));  // before gu[l] is reused
         if (CONV_KERNEL[l] == 2) {
             // rows 2m and 2m+1 of level l-1 in one GEMM: N = 1024 = (tap, cin)
             GemmOperand A{gu[l], M, CONV_DIM, 0, 0};
@@ -838,7 +858,14 @@ static int backward_chain(Handle* h, const Workspace& ws, const LossBufs& L, int
             }
         }
     }
-    if (tc) return train_hook_conv0(tc, ws, gu[0], est_dev, B, R0e, h->w, st);  // gu[0] = dL/du0: no waveform gradient
+    if (tc && train_conv(tc)) {
+        NB_TRY(train_hook_conv0(tc, ws, gu[0], est_dev, B, R0e, h->w, st));  // reads gu[0] = dL/du0 (aux0_raw)
+        if (d_est_dev == nullptr) return 0;
+    }
+    if (ws.aux0_raw) {  // gu[0] = dL/du0 without the GroupNorm gamma * rstd that the waveform backward expects
+        conv0_gain_fold_kernel<<<(unsigned)(R0e / 64), 256, 0, st>>>(gu[0], ws.meta, B, w.gn_g, ws.gn_stat);
+        NB_LAUNCHED();
+    }
     // conv0 + GroupNorm backward: gu[0] = G0
     NB_CUDA(cudaMemsetAsync(L.c0_sums, 0, 8ull * 2 * CONV_DIM * B, st));
     conv0_bwd_stats_kernel<<<(unsigned)(R0e / 64), 256, 0, st>>>(gu[0], est_dev, ws.meta, B, w.conv0_w, ws.gn_stat, L.c0_sums);
@@ -853,7 +880,7 @@ static int backward_chain(Handle* h, const Workspace& ws, const LossBufs& L, int
     }
     dim3 fgrid((unsigned)((N + 255) / 256), B);
     conv0_bwd_finish_kernel<<<fgrid, 256, 0, st>>>(L.c0_V, est_dev, ws.meta, L.c0_consts, N, 1.0f / S,
-                                                   ug != nullptr ? ug->scale : nullptr, d_est_dev);
+                                                   ug != nullptr && !ug->scaled_out ? ug->scale : nullptr, d_est_dev);
     NB_LAUNCHED();
     return 0;
 }
@@ -898,6 +925,7 @@ struct TrainCtx {
     float* part;        // [splits][512][k * 512] fp32 partial weight gradients of the K slices
     double* c0_sums;    // [3B][512][12] per (utterance, channel): sum D, sum D uhat, sum D x[5t + j]
     int max_chunks;     // wave-stats chunks per utterance (Plan::max_chunks)
+    const UserGrads* ug;  // autograd parameter path (nomad_b200_layers_bwd_params): the caller's output gradients, or null
 };
 
 // flat conv-encoder gradient buffer (fp32), each tensor in the checkpoint's (out, in, tap) order:
@@ -971,11 +999,16 @@ static int launch_colsum(cudaStream_t st, const T* in, long long rows, int cols,
 }
 // LayerNorm(768) parameter gradients: with g = gradient wrt the LayerNorm OUTPUT (g_in rows + g_pool[utt] broadcast, either
 // may be null) and xhat the normalised input: d_gamma += g * xhat, d_beta += g.  `pos_y` non-null: the input row is
-// x[f] + pos_y[pos row of f] (the encoder LayerNorm).
+// x[f] + pos_y[pos row of f] (the encoder LayerNorm).  USER (autograd parameter path): the incoming gradient is
+// g_in + S * g_user[b, t] + S * g_pool[utt] as ln768_bwd_user_kernel forms it (g_user in the caller's layout, row
+// b * user_T + t, may be null; S read from the device).
+template <bool USER>
 __global__ void __launch_bounds__(256) ln768_param_grad_kernel(const float* __restrict__ g_in, const float* __restrict__ g_pool,
                                                                const float* __restrict__ pre, const op_t* __restrict__ pos_y,
                                                                const UttMeta* __restrict__ meta, int B, long long frames,
-                                                               float* __restrict__ d_gamma, float* __restrict__ d_beta) {
+                                                               float* __restrict__ d_gamma, float* __restrict__ d_beta,
+                                                               const float* __restrict__ g_user, int user_T,
+                                                               const float* __restrict__ scale) {
     __shared__ float sg[EMBED], sb[EMBED];
     for (int i = threadIdx.x; i < EMBED; i += 256) { sg[i] = 0.f; sb[i] = 0.f; }
     __syncthreads();
@@ -1006,7 +1039,21 @@ __global__ void __launch_bounds__(256) ln768_param_grad_kernel(const float* __re
 #pragma unroll
             for (int i = 0; i < 24; ++i) g.v[i] = 0.f;
         }
-        if (g_pool != nullptr) {
+        if (USER) {
+            const float S = __ldg(scale);
+            if (g_user != nullptr) {
+                Row768f gu;
+                load_row768(gu, g_user + ((long long)b * user_T + t) * EMBED, lane);
+#pragma unroll
+                for (int i = 0; i < 24; ++i) g.v[i] = fmaf(S, gu.v[i], g.v[i]);
+            }
+            if (g_pool != nullptr) {
+                Row768f gp;
+                load_vec768(gp, g_pool + (long long)b * EMBED, lane);
+#pragma unroll
+                for (int i = 0; i < 24; ++i) g.v[i] = fmaf(S, gp.v[i], g.v[i]);
+            }
+        } else if (g_pool != nullptr) {
             Row768f gp;
             load_vec768(gp, g_pool + (long long)b * EMBED, lane);
 #pragma unroll
@@ -1028,7 +1075,16 @@ __global__ void __launch_bounds__(256) ln768_param_grad_kernel(const float* __re
 static int launch_ln768_param_grad(cudaStream_t st, const float* g_in, const float* g_pool, const float* pre, const op_t* pos_y,
                                    const UttMeta* meta, int B, long long frames, float* dg, float* db) {
     const unsigned blocks = (unsigned)std::min<long long>((frames + 7) / 8, 296);
-    ln768_param_grad_kernel<<<blocks, 256, 0, st>>>(g_in, g_pool, pre, pos_y, meta, B, frames, dg, db);
+    ln768_param_grad_kernel<false><<<blocks, 256, 0, st>>>(g_in, g_pool, pre, pos_y, meta, B, frames, dg, db, nullptr, 0, nullptr);
+    NB_LAUNCHED();
+    return 0;
+}
+static int launch_ln768_param_grad_user(cudaStream_t st, const float* g_in, const float* g_user, int user_T, const float* g_pool,
+                                        const float* scale, const float* pre, const UttMeta* meta, int B, long long frames,
+                                        float* dg, float* db) {
+    const unsigned blocks = (unsigned)std::min<long long>((frames + 7) / 8, 296);
+    ln768_param_grad_kernel<true><<<blocks, 256, 0, st>>>(g_in, g_pool, pre, nullptr, meta, B, frames, dg, db, g_user, user_T,
+                                                          scale);
     NB_LAUNCHED();
     return 0;
 }
@@ -1181,19 +1237,23 @@ __global__ void __launch_bounds__(256) triplet_head_kernel(const float* __restri
         gy[((long long)u * B + i) * EMB + tid] = (ge[u] - e[u] * dot) / nrm[u];  // backward of y / max(||y||, eps)
     }
 }
-// head parameter gradients and the pooled-feature gradient from gy
+// head parameter gradients and the pooled-feature gradient from gy; DEV_SCALE: times the scale S on the device (the
+// autograd parameter path, whose gy is unscaled)
+template <bool DEV_SCALE>
 __global__ void __launch_bounds__(256) head_param_grad_kernel(const float* __restrict__ gy, const float* __restrict__ pooled, int n_utt,
-                                                              float* __restrict__ dW, float* __restrict__ db) {
+                                                              float* __restrict__ dW, float* __restrict__ db,
+                                                              const float* __restrict__ scale) {
     const int o = blockIdx.x;  // output row of the head
+    const float S = DEV_SCALE ? __ldg(scale) : 1.f;
     float bsum = 0.f;
     for (int k = threadIdx.x; k < EMBED; k += 256) {
         float a = 0.f;
         for (int u = 0; u < n_utt; ++u) a = fmaf(gy[(long long)u * EMB + o], fmaxf(pooled[(long long)u * EMBED + k], 0.f), a);
-        dW[(long long)o * EMBED + k] = a;
+        dW[(long long)o * EMBED + k] = DEV_SCALE ? a * S : a;
     }
     if (threadIdx.x == 0) {
         for (int u = 0; u < n_utt; ++u) bsum += gy[(long long)u * EMB + o];
-        db[o] = bsum;
+        db[o] = DEV_SCALE ? bsum * S : bsum;
     }
 }
 __global__ void __launch_bounds__(256) head_pool_grad_kernel(const float* __restrict__ gy, const float* __restrict__ pooled,
@@ -1422,8 +1482,14 @@ static int train_hook_layer(Handle* h, const Workspace& ws, const LossBufs& L, T
     const LayerBufs& Lb = ws.layer[l];
     float* G = tc->grads + TrainLayout::LAYER * l;
     if (stage == 0) {  // final_layer_norm params (incoming: g_running + pooled gradient on the top layer); fc2
-        NB_TRY(launch_ln768_param_grad(st, g_running, l == LAYERS - 1 ? L.g_pool : nullptr, Lb.pre2, nullptr, ws.meta, B, Fe,
-                                       G + TrainLayout::LN2_G, G + TrainLayout::LN2_B));
+        if (tc->ug != nullptr) {  // + the caller's gradient of this layer's output, both under S
+            const UserGrads& ug = *tc->ug;
+            NB_TRY(launch_ln768_param_grad_user(st, g_running, ug.g_layers[l], ug.T, l == LAYERS - 1 ? ug.g_pool : nullptr,
+                                                ug.scale, Lb.pre2, ws.meta, B, Fe, G + TrainLayout::LN2_G, G + TrainLayout::LN2_B));
+        } else {
+            NB_TRY(launch_ln768_param_grad(st, g_running, l == LAYERS - 1 ? L.g_pool : nullptr, Lb.pre2, nullptr, ws.meta, B, Fe,
+                                           G + TrainLayout::LN2_G, G + TrainLayout::LN2_B));
+        }
         NB_TRY(wgrad(st, tc, L.g_bh, EMBED, Lb.ffn_h, FFN, Fe, G + TrainLayout::FC2_W));
         NB_TRY(launch_colsum<float>(st, L.g_b, Fe, EMBED, G + TrainLayout::FC2_B));
     } else if (stage == 1) {  // fc1: input = LayerNorm1(pre1), recomputed
@@ -1773,7 +1839,8 @@ static int triplet_run(nomad_b200_handle* hh, const float* wav_dev, int B, int64
     NB_LAUNCHED();
     triplet_loss_finalize_kernel<<<1, 1, 0, st>>>(L.acc, 1.0 / (double)B, loss_dev);
     NB_LAUNCHED();
-    head_param_grad_kernel<<<EMB, 256, 0, st>>>(tc.gy, L.pooled, U, grads_dev + TrainLayout::HEAD_W, grads_dev + TrainLayout::HEAD_B);
+    head_param_grad_kernel<false><<<EMB, 256, 0, st>>>(tc.gy, L.pooled, U, grads_dev + TrainLayout::HEAD_W,
+                                                       grads_dev + TrainLayout::HEAD_B, nullptr);
     NB_LAUNCHED();
     head_pool_grad_kernel<<<U, 256, 0, st>>>(tc.gy, L.pooled, ws.meta, w.head_wt, L.g_pool);
     NB_LAUNCHED();
@@ -1829,15 +1896,24 @@ int nomad_b200_triplet_conv_fwd_bwd(nomad_b200_handle* hh, const float* wav_dev,
 }  // extern "C"
 
 // ---- autograd through LossNetLayers / TripletModel: save-mode forward + backward from arbitrary upstream gradients ----
-// The saved buffer is [save-mode Workspace | pooled features B x 768 | head output B x 256 | head snapshot: transposed
-// weight 768 x 256, bias 256].  The backward re-derives the Plan from (B, N) and re-carves the same Workspace over it, so
-// every pointer (metadata included) comes back as the forward left it; the backward only reads it.
+// The saved buffer is [record | save-mode Workspace | pooled features B x 768 | head output B x 256 | head snapshot:
+// transposed weight 768 x 256, bias 256].  The backward re-derives the Plan from (B, N) and re-carves the same Workspace
+// over it, so every pointer (metadata included) comes back as the forward left it; the backward only reads it.  The
+// record holds what the forward saved for (NOMAD_B200_SAVE_* flags; PARAMS makes the Workspace larger): the parameter
+// backward reads it back first and refuses what the forward did not save for.
 struct SavedTail {
     float* pooled;
     float* emb;
     float* head_wt;
     float* head_b;
 };
+struct SavedRecord {
+    uint32_t magic;
+    int32_t flags, head, B;
+    int64_t N;
+};
+static constexpr uint32_t SAVED_MAGIC = 0x4e425356u;
+static constexpr size_t SAVED_RECORD_BYTES = 1024;
 
 static int layers_plan(int B, int64_t N, Plan* p) {
     NB_CHECK(B > 0, "layers: need B > 0 utterances");
@@ -1849,8 +1925,10 @@ static int layers_plan(int B, int64_t N, Plan* p) {
     return make_plan(off.data(), B, p);
 }
 
-static size_t carve_saved(const Plan& p, void* base, Workspace* ws, SavedTail* tail) {
-    size_t o = carve_workspace(p, base, ws, true);
+static size_t carve_saved(const Plan& p, int flags, void* base, Workspace* ws, SavedTail* tail) {
+    size_t o = SAVED_RECORD_BYTES + carve_workspace(p, base ? (char*)base + SAVED_RECORD_BYTES : nullptr, ws, true,
+                                                    (flags & NOMAD_B200_SAVE_PARAMS) != 0);
+    if (ws) ws->aux0_raw = (flags & NOMAD_B200_SAVE_CONV) != 0;
     auto take = [&](size_t bytes) {
         size_t at = o;
         o = (o + bytes + 1023) / 1024 * 1024;
@@ -1876,12 +1954,32 @@ static size_t carve_layers_bwd(const Plan& p, void* base, LossBufs* L, float** g
     return lb + gy_bytes + 1024;
 }
 
+// parameter backward scratch: [carve_layers_bwd | TrainCtx buffers (train_extra_bytes) | conv scratch when CONV]
+static size_t carve_params_bwd(const Plan& p, int flags, void* base, LossBufs* L, float** gy, unsigned** state, TrainCtx* tc) {
+    const size_t lb = carve_layers_bwd(p, base, L, gy, state);
+    const size_t extra = train_extra_bytes(p.frames, p.B);
+    if (base) {
+        auto al = [](size_t v) { return (v + 1023) / 1024 * 1024; };
+        char* q = (char*)base + lb;
+        tc->Fp = (p.frames + 7) / 8 * 8;
+        tc->tA = (op_t*)q; q += al(2ull * FFN * tc->Fp);
+        tc->tB = (op_t*)q; q += al(2ull * FFN * tc->Fp);
+        tc->xh_tmp = (op_t*)q; q += al(2ull * EMBED * p.frames);
+        tc->x_tmp = (float*)q; q += al(4ull * EMBED * p.frames);
+        tc->gy = (float*)q;
+    }
+    const size_t conv = (flags & NOMAD_B200_SAVE_CONV) ? carve_conv_train(p.rows0, p.B, base ? (char*)base + lb + extra : nullptr, tc) : 0;
+    return lb + extra + conv;
+}
+
 extern "C" {
 
-size_t nomad_b200_layers_saved_bytes(int B, int64_t N) {
+size_t nomad_b200_layers_saved_bytes(int B, int64_t N) { return nomad_b200_layers_saved_bytes_ex(B, N, 0); }
+
+size_t nomad_b200_layers_saved_bytes_ex(int B, int64_t N, int flags) {
     Plan p;
     if (layers_plan(B, N, &p)) return 0;
-    return carve_saved(p, nullptr, nullptr, nullptr);
+    return carve_saved(p, flags, nullptr, nullptr, nullptr);
 }
 
 size_t nomad_b200_layers_bwd_workspace_bytes(int B, int64_t N) {
@@ -1890,13 +1988,25 @@ size_t nomad_b200_layers_bwd_workspace_bytes(int B, int64_t N) {
     return carve_layers_bwd(p, nullptr, nullptr, nullptr, nullptr);
 }
 
+size_t nomad_b200_layers_bwd_params_workspace_bytes(int B, int64_t N, int flags) {
+    Plan p;
+    if (layers_plan(B, N, &p)) return 0;
+    return carve_params_bwd(p, flags, nullptr, nullptr, nullptr, nullptr, nullptr);
+}
+
 int nomad_b200_layers_fwd_save(nomad_b200_handle* hh, const float* wav_dev, int B, int64_t N, int head, float* layers_dev,
                                float* emb_dev, void* saved_dev, size_t saved_bytes, void* stream) {
+    return nomad_b200_layers_fwd_save_ex(hh, wav_dev, B, N, head, layers_dev, emb_dev, saved_dev, saved_bytes, 0, stream);
+}
+
+int nomad_b200_layers_fwd_save_ex(nomad_b200_handle* hh, const float* wav_dev, int B, int64_t N, int head, float* layers_dev,
+                                  float* emb_dev, void* saved_dev, size_t saved_bytes, int flags, void* stream) {
     NB_CHECK(hh != nullptr, "null nomad_b200 handle");
     Handle* h = &hh->h;
     NB_CHECK(wav_dev && saved_dev, "layers_fwd_save: null pointer");
     NB_CHECK(head == 0 || head == 1, "layers_fwd_save: head must be 0 (NOMAD head) or 1 (loss head)");
     NB_CHECK(head == 0 || h->has_loss_head, "layers_fwd_save: head 1 needs nomad_b200_set_loss_head first");
+    NB_CHECK((flags & ~(NOMAD_B200_SAVE_PARAMS | NOMAD_B200_SAVE_CONV)) == 0, "layers_fwd_save: unknown flags %d", flags);
     NB_CHECK(((uintptr_t)wav_dev & 3) == 0, "layers_fwd_save: waveform pointer must be 4-byte aligned");
     NB_CHECK(((uintptr_t)saved_dev & 1023) == 0, "layers_fwd_save: saved buffer must be 1024-byte aligned");
     NB_CUDA(cudaSetDevice(h->device));
@@ -1904,10 +2014,13 @@ int nomad_b200_layers_fwd_save(nomad_b200_handle* hh, const float* wav_dev, int 
     NB_TRY(layers_plan(B, N, &p));
     Workspace ws;
     SavedTail t;
-    const size_t need = carve_saved(p, saved_dev, &ws, &t);
+    const size_t need = carve_saved(p, flags, saved_dev, &ws, &t);
     NB_CHECK(saved_bytes >= need, "layers_fwd_save: saved buffer too small (%zu < %zu bytes)", saved_bytes, need);
     cudaStream_t st = (cudaStream_t)stream;
     const Weights& w = h->w;
+    // pageable source: staged by the call itself, nothing to keep alive
+    const SavedRecord rec{SAVED_MAGIC, flags, head, B, (int64_t)N};
+    NB_CUDA(cudaMemcpyAsync(saved_dev, &rec, sizeof(rec), cudaMemcpyHostToDevice, st));
     NB_CUDA(cudaMemcpyAsync(t.head_wt, head ? w.loss_head_wt : w.head_wt, 4ull * EMBED * EMB, cudaMemcpyDeviceToDevice, st));
     NB_CUDA(cudaMemcpyAsync(t.head_b, head ? w.loss_head_b : w.head_b, 4ull * EMB, cudaMemcpyDeviceToDevice, st));
     NB_TRY(upload_meta(h, p, ws, st));
@@ -1915,6 +2028,88 @@ int nomad_b200_layers_fwd_save(nomad_b200_handle* hh, const float* wav_dev, int 
     NB_TRY(launch_pool_head(st, ws.x, ws.meta, p.B, t.head_wt, t.head_b, emb_dev ? emb_dev : t.emb, t.pooled));
     return 0;
 }
+
+}  // extern "C"
+
+// Backward of one saved forward from the caller's output gradients.  grads_dev null (nomad_b200_layers_bwd): the waveform
+// gradient only, S divided out.  grads_dev non-null (nomad_b200_layers_bwd_params): every parameter gradient as well
+// (TrainLayout; conv_grads_dev: ConvLayout, which needs a CONV forward), the waveform gradient only when d_wav_dev is
+// non-null; every output is multiplied by S and S goes to scale_out.
+static int layers_backward(Handle* h, const Plan& p, int flags, int head, const void* saved_dev, const float* wav_dev, int64_t N,
+                           const float* const* g_layers, const float* g_emb, float feature_grad_mult, float* d_wav_dev,
+                           float* grads_dev, float* conv_grads_dev, float* scale_out, void* workspace_dev,
+                           size_t workspace_bytes, cudaStream_t st) {
+    const int B = p.B;
+    const bool params = grads_dev != nullptr;
+    Workspace ws;
+    SavedTail t;
+    carve_saved(p, flags, (void*)saved_dev, &ws, &t);
+    LossBufs L;
+    float* gy = nullptr;
+    unsigned* state = nullptr;
+    TrainCtx tc;
+    memset(&tc, 0, sizeof(tc));
+    const size_t need = params ? carve_params_bwd(p, flags, workspace_dev, &L, &gy, &state, &tc)
+                               : carve_layers_bwd(p, workspace_dev, &L, &gy, &state);
+    NB_CHECK(workspace_bytes >= need, "layers_bwd: workspace too small (%zu < %zu bytes)", workspace_bytes, need);
+
+    UserGrads ug;
+    memset(&ug, 0, sizeof(ug));
+    ug.T = p.max_T;
+    ug.top = -1;
+    ug.scaled_out = params;
+    ScaleSources src;
+    memset(&src, 0, sizeof(src));
+    const long long layer_n = (long long)B * p.max_T * EMBED;
+    for (int l = 0; l < LAYERS; ++l) {
+        ug.g_layers[l] = g_layers != nullptr ? g_layers[l] : nullptr;
+        src.p[l] = ug.g_layers[l];
+        src.n[l] = layer_n;
+        if (ug.g_layers[l] != nullptr) ug.top = l;
+    }
+    float* scale = scale_out != nullptr ? scale_out : (float*)(state + 2);
+    ug.scale = scale;
+    if (ug.top < 0 && g_emb == nullptr) {  // no output is used: the gradient is zero
+        if (d_wav_dev != nullptr) NB_CUDA(cudaMemsetAsync(d_wav_dev, 0, 4ull * B * N, st));
+        if (!params) return 0;
+        NB_CUDA(cudaMemsetAsync(grads_dev, 0, sizeof(float) * TrainLayout::TOTAL, st));
+        if (conv_grads_dev != nullptr) NB_CUDA(cudaMemsetAsync(conv_grads_dev, 0, sizeof(float) * ConvLayout::TOTAL, st));
+        NB_CUDA(cudaMemsetAsync(state, 0, 2 * sizeof(unsigned), st));
+        grad_scale_kernel<<<1, 256, 0, st>>>(src, state, scale);  // no sources: S = 1
+        NB_LAUNCHED();
+        return 0;
+    }
+    if (params) NB_CUDA(cudaMemsetAsync(grads_dev, 0, sizeof(float) * TrainLayout::TOTAL, st));
+    if (g_emb != nullptr) {  // head: g_emb -> gy -> pooled-feature gradient (ReLU mask, / T), with the snapshotted head
+        head_emb_bwd_kernel<<<B, 256, 0, st>>>(t.pooled, t.head_wt, t.head_b, g_emb, gy);
+        NB_LAUNCHED();
+        head_pool_grad_kernel<<<B, 256, 0, st>>>(gy, t.pooled, ws.meta, t.head_wt, L.g_pool);
+        NB_LAUNCHED();
+        ug.g_pool = L.g_pool;
+        ug.top = LAYERS - 1;
+        src.p[LAYERS] = L.g_pool;
+        src.n[LAYERS] = (long long)B * EMBED;
+    }
+    NB_CUDA(cudaMemsetAsync(state, 0, 2 * sizeof(unsigned), st));
+    grad_scale_kernel<<<2 * 148, 256, 0, st>>>(src, state, scale);
+    NB_LAUNCHED();
+    if (params) {
+        // the NOMAD head's own gradient (gy is unscaled: S from the device); the loss head (head 1) is not trained here
+        if (g_emb != nullptr && head == 0) {
+            head_param_grad_kernel<true><<<EMB, 256, 0, st>>>(gy, t.pooled, B, grads_dev + TrainLayout::HEAD_W,
+                                                              grads_dev + TrainLayout::HEAD_B, scale);
+            NB_LAUNCHED();
+        }
+        tc.grads = grads_dev;
+        tc.conv_grads = conv_grads_dev;
+        tc.max_chunks = p.max_chunks;
+        tc.ug = &ug;
+    }
+    return backward_chain(h, ws, L, B, p.frames, p.rows0, p.pos_rows, p.max_T, 0.f, feature_grad_mult, 1.f, wav_dev, N,
+                          d_wav_dev, st, params ? &tc : nullptr, &ug);
+}
+
+extern "C" {
 
 int nomad_b200_layers_bwd(nomad_b200_handle* hh, const void* saved_dev, size_t saved_bytes, const float* wav_dev, int B,
                           int64_t N, const float* const* g_layers, const float* g_emb, float feature_grad_mult,
@@ -1931,52 +2126,48 @@ int nomad_b200_layers_bwd(nomad_b200_handle* hh, const void* saved_dev, size_t s
     NB_CUDA(cudaSetDevice(h->device));
     Plan p;
     NB_TRY(layers_plan(B, N, &p));
-    Workspace ws;
-    SavedTail t;
-    const size_t need_saved = carve_saved(p, (void*)saved_dev, &ws, &t);
+    const size_t need_saved = carve_saved(p, 0, nullptr, nullptr, nullptr);
     NB_CHECK(saved_bytes >= need_saved, "layers_bwd: saved buffer too small (%zu < %zu bytes): not from a forward of this B x N?",
              saved_bytes, need_saved);
-    LossBufs L;
-    float* gy = nullptr;
-    unsigned* state = nullptr;
-    const size_t need = carve_layers_bwd(p, workspace_dev, &L, &gy, &state);
-    NB_CHECK(workspace_bytes >= need, "layers_bwd: workspace too small (%zu < %zu bytes)", workspace_bytes, need);
-    cudaStream_t st = (cudaStream_t)stream;
+    return layers_backward(h, p, 0, 0, saved_dev, wav_dev, N, g_layers, g_emb, feature_grad_mult, d_wav_dev, nullptr, nullptr,
+                           nullptr, workspace_dev, workspace_bytes, (cudaStream_t)stream);
+}
 
-    UserGrads ug;
-    memset(&ug, 0, sizeof(ug));
-    ug.T = p.max_T;
-    ug.top = -1;
-    ScaleSources src;
-    memset(&src, 0, sizeof(src));
-    const long long layer_n = (long long)B * p.max_T * EMBED;
-    for (int l = 0; l < LAYERS; ++l) {
-        ug.g_layers[l] = g_layers != nullptr ? g_layers[l] : nullptr;
-        src.p[l] = ug.g_layers[l];
-        src.n[l] = layer_n;
-        if (ug.g_layers[l] != nullptr) ug.top = l;
-    }
-    if (ug.top < 0 && g_emb == nullptr) {  // no output is used: the gradient is zero
-        NB_CUDA(cudaMemsetAsync(d_wav_dev, 0, 4ull * B * N, st));
-        return 0;
-    }
-    if (g_emb != nullptr) {  // head: g_emb -> gy -> pooled-feature gradient (ReLU mask, / T), with the snapshotted head
-        head_emb_bwd_kernel<<<B, 256, 0, st>>>(t.pooled, t.head_wt, t.head_b, g_emb, gy);
-        NB_LAUNCHED();
-        head_pool_grad_kernel<<<B, 256, 0, st>>>(gy, t.pooled, ws.meta, t.head_wt, L.g_pool);
-        NB_LAUNCHED();
-        ug.g_pool = L.g_pool;
-        ug.top = LAYERS - 1;
-        src.p[LAYERS] = L.g_pool;
-        src.n[LAYERS] = (long long)B * EMBED;
-    }
-    float* scale = (float*)(state + 2);
-    ug.scale = scale;
-    NB_CUDA(cudaMemsetAsync(state, 0, 2 * sizeof(unsigned), st));
-    grad_scale_kernel<<<2 * 148, 256, 0, st>>>(src, state, scale);
-    NB_LAUNCHED();
-    return backward_chain(h, ws, L, B, p.frames, p.rows0, p.pos_rows, p.max_T, 0.f, feature_grad_mult, 1.f, wav_dev, N,
-                          d_wav_dev, st, nullptr, &ug);
+int nomad_b200_layers_bwd_params(nomad_b200_handle* hh, const void* saved_dev, size_t saved_bytes, const float* wav_dev, int B,
+                                 int64_t N, const float* const* g_layers, const float* g_emb, float feature_grad_mult,
+                                 float* d_wav_dev, float* grads_dev, float* conv_grads_dev, float* grad_scale_dev,
+                                 void* workspace_dev, size_t workspace_bytes, void* stream) {
+    NB_CHECK(hh != nullptr, "null nomad_b200 handle");
+    Handle* h = &hh->h;
+    NB_CHECK(saved_dev && wav_dev && grad_scale_dev && workspace_dev, "layers_bwd_params: null pointer");
+    NB_CHECK(d_wav_dev != nullptr || grads_dev != nullptr, "layers_bwd_params: nothing to compute (d_wav and grads both NULL)");
+    NB_CHECK(conv_grads_dev == nullptr || grads_dev != nullptr, "layers_bwd_params: conv_grads needs grads too");
+    NB_CHECK(((uintptr_t)saved_dev & 1023) == 0 && ((uintptr_t)workspace_dev & 1023) == 0,
+             "layers_bwd_params: saved buffer and workspace must be 1024-byte aligned");
+    NB_CHECK(((uintptr_t)wav_dev & 3) == 0 && ((uintptr_t)d_wav_dev & 3) == 0 && ((uintptr_t)grad_scale_dev & 3) == 0,
+             "layers_bwd_params: waveform and scale pointers must be 4-byte aligned");
+    NB_CHECK((((uintptr_t)g_emb | (uintptr_t)grads_dev | (uintptr_t)conv_grads_dev) & 15) == 0,
+             "layers_bwd_params: g_emb, grads and conv_grads must be 16-byte aligned");
+    for (int l = 0; g_layers != nullptr && l < LAYERS; ++l)
+        NB_CHECK(((uintptr_t)g_layers[l] & 15) == 0, "layers_bwd_params: g_layers[%d] must be 16-byte aligned", l);
+    NB_CUDA(cudaSetDevice(h->device));
+    Plan p;
+    NB_TRY(layers_plan(B, N, &p));
+    NB_CHECK(saved_bytes >= SAVED_RECORD_BYTES, "layers_bwd_params: saved buffer too small");
+    cudaStream_t st = (cudaStream_t)stream;
+    SavedRecord rec;
+    NB_CUDA(cudaMemcpyAsync(&rec, saved_dev, sizeof(rec), cudaMemcpyDeviceToHost, st));
+    NB_CUDA(cudaStreamSynchronize(st));
+    NB_CHECK(rec.magic == SAVED_MAGIC && rec.B == B && rec.N == (int64_t)N,
+             "layers_bwd_params: the saved buffer is not from a nomad_b200_layers_fwd_save(_ex) of this B x N");
+    NB_CHECK(grads_dev == nullptr || (rec.flags & NOMAD_B200_SAVE_PARAMS),
+             "layers_bwd_params: parameter gradients need a forward saved with NOMAD_B200_SAVE_PARAMS");
+    NB_CHECK(conv_grads_dev == nullptr || (rec.flags & NOMAD_B200_SAVE_CONV),
+             "layers_bwd_params: conv encoder gradients need a forward saved with NOMAD_B200_SAVE_CONV");
+    const size_t need_saved = carve_saved(p, rec.flags, nullptr, nullptr, nullptr);
+    NB_CHECK(saved_bytes >= need_saved, "layers_bwd_params: saved buffer too small (%zu < %zu bytes)", saved_bytes, need_saved);
+    return layers_backward(h, p, rec.flags, rec.head, saved_dev, wav_dev, N, g_layers, g_emb, feature_grad_mult, d_wav_dev,
+                           grads_dev, conv_grads_dev, grad_scale_dev, workspace_dev, workspace_bytes, st);
 }
 
 }  // extern "C"

@@ -60,6 +60,14 @@ class Engine:
         self._ws: Optional[torch.Tensor] = None
         self._pinned: Optional[torch.Tensor] = None
         self._pinned_out: Optional[torch.Tensor] = None
+        # bumped by every weight refresh: an autograd graph recorded under an older generation cannot be differentiated
+        self.weight_generation = 0
+        # called before every call that runs the network (Nomad's parameter store: push edited parameters to the device)
+        self.sync_hook = None
+
+    def sync_weights(self):
+        if self.sync_hook is not None:
+            self.sync_hook()
 
     def close(self):
         if getattr(self, "handle", None):
@@ -111,6 +119,7 @@ class Engine:
         with torch.cuda.device(self.device):
             fn = "nomad_b200_refresh_conv_weights" if conv else "nomad_b200_refresh_weights"
             _lib.check(getattr(self.lib, fn)(self.handle, tens, len(names), _stream_ptr()), fn)
+        self.weight_generation += 1
 
     def set_loss_head(self, weight: torch.Tensor, bias: torch.Tensor):
         w = np.ascontiguousarray(weight.detach().to(torch.float32).cpu().numpy())
@@ -141,6 +150,7 @@ class Engine:
     # ------------------------------------------------------------------ scoring
     def embed_packed(self, wav: torch.Tensor, offsets: np.ndarray, out: Optional[torch.Tensor] = None) -> torch.Tensor:
         """``wav``: 1-D fp32 CUDA tensor holding the utterances back to back; ``offsets``: B+1 int64 (host)."""
+        self.sync_weights()
         assert wav.is_cuda and wav.dtype == torch.float32 and wav.is_contiguous()
         B = len(offsets) - 1
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
@@ -166,6 +176,7 @@ class Engine:
 
     def embed_host(self, wav_host: np.ndarray, offsets: np.ndarray, emb_host: Optional[np.ndarray] = None) -> np.ndarray:
         """HOST buffers in and out through ``nomad_b200_embed_host`` (H2D + compute + D2H + sync inside)."""
+        self.sync_weights()
         B = len(offsets) - 1
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
         off_p = offsets.ctypes.data_as(C.POINTER(C.c_int64))
@@ -186,6 +197,7 @@ class Engine:
 
     def score_packed(self, wav: torch.Tensor, offsets: np.ndarray, nmr: torch.Tensor, want_matrix: bool = True):
         """One batch of ``Nomad.predict`` on device-resident data: -> (emb (B, 256), dm (B, m) | None, mean (B,) fp64)."""
+        self.sync_weights()
         assert wav.is_cuda and wav.dtype == torch.float32 and wav.is_contiguous()
         assert nmr.is_cuda and nmr.dtype == torch.float32 and nmr.is_contiguous() and nmr.shape[1] == EMB_DIM
         B, m = len(offsets) - 1, nmr.shape[0]
@@ -206,6 +218,7 @@ class Engine:
     def score_host(self, wav_host: np.ndarray, offsets: np.ndarray, nmr: torch.Tensor, emb_host: Optional[np.ndarray],
                    dm_host: Optional[np.ndarray], mean_host: np.ndarray):
         """Same with HOST waveforms in and HOST results out (H2D + compute + D2H + sync inside the C call)."""
+        self.sync_weights()
         assert wav_host.dtype == np.float32 and wav_host.flags.c_contiguous and mean_host.dtype == np.float64
         assert nmr.is_cuda and nmr.dtype == torch.float32 and nmr.is_contiguous() and nmr.shape[1] == EMB_DIM
         B, m = len(offsets) - 1, nmr.shape[0]
@@ -312,6 +325,7 @@ class Engine:
 
     def layers(self, wav: torch.Tensor, want_layers: bool = True, want_emb: bool = True):
         """``LossNetLayers.forward`` for a (B, N) or (B, 1, N) CUDA batch -> ((12, B, T, 768) | None, (B, 256) | None)."""
+        self.sync_weights()
         if wav.dim() == 3:
             wav = wav.squeeze(1)
         wav = wav.to(self.device, torch.float32).contiguous()
@@ -329,14 +343,16 @@ class Engine:
                                                       _stream_ptr()), "nomad_b200_layers_fwd")
         return layers, emb
 
-    def layers_fwd_save(self, wav: torch.Tensor, head: int, want_layers: bool = True):
+    def layers_fwd_save(self, wav: torch.Tensor, head: int, want_layers: bool = True, flags: int = 0):
         """Save-mode forward of a (B, N) CUDA batch for autograd (``nomad_b200_layers_fwd_save``; fp16 operands whatever
         the engine's precision).  ``head``: 0 = NOMAD head, 1 = loss head.  -> ((12, B, T, 768) | None, (B, 256), saved):
-        ``saved`` is a uint8 CUDA tensor owned by the caller that :meth:`layers_bwd` needs; keep it until then."""
+        ``saved`` is a uint8 CUDA tensor owned by the caller that :meth:`layers_bwd` needs; keep it until then.
+        ``flags`` (``_lib.SAVE_*``, ``nomad_b200_layers_fwd_save_ex``): also save for :meth:`layers_bwd_params`."""
+        self.sync_weights()
         wav = wav.to(self.device, torch.float32).contiguous()
         B, N = wav.shape
         T = self.num_frames(N)
-        nbytes = self.lib.nomad_b200_layers_saved_bytes(B, N)
+        nbytes = self.lib.nomad_b200_layers_saved_bytes_ex(B, N, int(flags))
         if nbytes == 0:
             raise _lib.NomadB200Error(self.lib.nomad_b200_last_error().decode())
         saved = torch.empty(nbytes + 1024, dtype=torch.uint8, device=self.device)
@@ -344,8 +360,13 @@ class Engine:
         layers = torch.empty((NUM_LAYERS, B, T, SSL_OUT_DIM), dtype=torch.float32, device=self.device) if want_layers else None
         emb = torch.empty((B, EMB_DIM), dtype=torch.float32, device=self.device)
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.nomad_b200_layers_fwd_save(self.handle, _ptr(wav), B, N, int(head), _ptr(layers), _ptr(emb),
-                                                           sp, sbytes, _stream_ptr()), "nomad_b200_layers_fwd_save")
+            if flags:
+                _lib.check(self.lib.nomad_b200_layers_fwd_save_ex(self.handle, _ptr(wav), B, N, int(head), _ptr(layers),
+                                                                  _ptr(emb), sp, sbytes, int(flags), _stream_ptr()),
+                           "nomad_b200_layers_fwd_save_ex")
+            else:
+                _lib.check(self.lib.nomad_b200_layers_fwd_save(self.handle, _ptr(wav), B, N, int(head), _ptr(layers),
+                                                               _ptr(emb), sp, sbytes, _stream_ptr()), "nomad_b200_layers_fwd_save")
         return layers, emb, saved
 
     def layers_bwd(self, saved: torch.Tensor, wav: torch.Tensor, g_layers: Sequence[Optional[torch.Tensor]],
@@ -355,14 +376,8 @@ class Engine:
         wav = wav.to(self.device, torch.float32).contiguous()
         B, N = wav.shape
 
-        def dev(g):  # fp32, contiguous, 16-byte aligned (the kernels read rows as float4)
-            if g is None:
-                return None
-            g = g.to(self.device, torch.float32).contiguous()
-            return g if g.data_ptr() % 16 == 0 else g.clone()
-
-        gl = [dev(g) for g in g_layers]
-        ge = dev(g_emb)
+        gl = [self._grad_in(g) for g in g_layers]
+        ge = self._grad_in(g_emb)
         need = self.lib.nomad_b200_layers_bwd_workspace_bytes(B, N)
         if need == 0:
             raise _lib.NomadB200Error(self.lib.nomad_b200_last_error().decode())
@@ -376,7 +391,42 @@ class Engine:
                        "nomad_b200_layers_bwd")
         return d_wav
 
+    def _grad_in(self, g):  # fp32, contiguous, 16-byte aligned (the kernels read rows as float4)
+        if g is None:
+            return None
+        g = g.to(self.device, torch.float32).contiguous()
+        return g if g.data_ptr() % 16 == 0 else g.clone()
+
+    def layers_bwd_params(self, saved: torch.Tensor, wav: torch.Tensor, g_layers: Sequence[Optional[torch.Tensor]],
+                          g_emb: Optional[torch.Tensor], feature_grad_mult: float, flags: int, want_wav: bool,
+                          want_params: bool, want_conv: bool):
+        """:meth:`layers_bwd` plus the parameter gradients (``nomad_b200_layers_bwd_params``) for a forward saved with
+        ``flags``.  -> (d_wav (B, N) | None, grads (flat, ``triplet.grad_segments()`` layout) | None, conv_grads (flat,
+        ``grad_segments(conv=True)``) | None, S (0-dim CUDA tensor)): every result is multiplied by S."""
+        wav = wav.to(self.device, torch.float32).contiguous()
+        B, N = wav.shape
+        gl = [self._grad_in(g) for g in g_layers]
+        ge = self._grad_in(g_emb)
+        need = self.lib.nomad_b200_layers_bwd_params_workspace_bytes(B, N, int(flags))
+        if need == 0:
+            raise _lib.NomadB200Error(self.lib.nomad_b200_last_error().decode())
+        wp, wbytes = self._aligned(self.workspace(need))
+        sp, sbytes = self._aligned(saved)
+        ptrs = (C.c_void_p * NUM_LAYERS)(*[None if g is None else g.data_ptr() for g in gl])
+        f32 = dict(dtype=torch.float32, device=self.device)
+        d_wav = torch.empty((B, N), **f32) if want_wav else None
+        grads = torch.empty((int(self.lib.nomad_b200_triplet_grad_floats()),), **f32) if want_params else None
+        conv = torch.empty((int(self.lib.nomad_b200_triplet_conv_grad_floats()),), **f32) if want_conv else None
+        scale = torch.empty((), **f32)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.nomad_b200_layers_bwd_params(self.handle, sp, sbytes, _ptr(wav), B, N, ptrs, _ptr(ge),
+                                                             C.c_float(feature_grad_mult), _ptr(d_wav), _ptr(grads), _ptr(conv),
+                                                             _ptr(scale), wp, wbytes, _stream_ptr()),
+                       "nomad_b200_layers_bwd_params")
+        return d_wav, grads, conv, scale
+
     def loss_fwd_bwd(self, est: torch.Tensor, clean: torch.Tensor, feature_grad_mult: float, with_grad: bool = True):
+        self.sync_weights()
         if est.dim() == 3:
             est = est.squeeze(1)
         if clean.dim() == 3:

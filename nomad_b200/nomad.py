@@ -9,14 +9,18 @@ backward) runs in ``libnomad_b200.so`` on a B200.  Differences that are delibera
 * there is no CPU path: ``device='cpu'`` raises;
 * weights come from ``pt-models/nomad_best_model.pt`` (or ``$NOMAD_B200_CHECKPOINT``) when present,
   else seeded random-init of the identical architecture -- nothing is downloaded at import;
-* gradients reach the input waveforms only (dgrad chain, wheel 0.0.8 semantics: the NOMAD network's own
-  parameters receive no ``.grad``);
+* the network's parameters start frozen, as in wheel 0.0.8: gradients reach the input waveforms only until
+  ``nomad.model.requires_grad_()`` (or ``requires_grad`` on single tensors of ``nomad.model.parameters()``, which needs
+  ``keep_state_dict=True``); then ``model``, ``lossnet_layers`` and ``forward`` give ``.grad`` to those parameters from
+  any use of their outputs, and edits to them (an optimiser step) reach the device before the next call that runs the
+  network;
 * the differentiable calls (``model``, ``lossnet_layers`` and ``forward`` with grad on) always run fp16 tensor-core
   operands: with ``precision='fp32'`` only the no-grad path is fp32-class.
 """
 from __future__ import annotations
 
 import os
+from collections import OrderedDict
 from datetime import datetime
 from typing import List, Optional, Sequence
 
@@ -26,8 +30,9 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
-from . import audio
+from . import _lib, audio
 from .engine import Engine, MIN_SAMPLES
+from .triplet import POS_G, POS_V, grads_by_name
 from .weights import EMB_DIM, NUM_LAYERS, SSL_OUT_DIM, load_state_dict
 
 w2v_path = 'pt-models/wav2vec_small.pt'        # kept for API compatibility (nomad.py:21); unused
@@ -51,27 +56,114 @@ def plan_batches(lengths: Sequence[int], max_samples: int) -> List[List[int]]:
     return batches
 
 
+CONV_PREFIX = "ssl_model.feature_extractor."
+
+
+class _ParamStore:
+    """The network's parameters as fp32 ``nn.Parameter``s on the engine's device, keyed by checkpoint names: every
+    ``ssl_model.*`` tensor and the NOMAD head ``embedding_layer.*``.  Built on first use from ``Nomad.state_dict_ref``;
+    all start with ``requires_grad=False`` and ``mask_emb`` is never trainable.  Once built, every call that runs the
+    network first compares each parameter's ``_version`` / ``data_ptr`` with the last sync and rebuilds the kernel-ready
+    weights that changed (``Engine.refresh_weights`` / ``refresh_conv_weights``)."""
+
+    def __init__(self, nomad):
+        self._nomad = nomad
+        self.params: Optional["OrderedDict[str, nn.Parameter]"] = None
+        self._seen = None
+
+    def build(self) -> "OrderedDict[str, nn.Parameter]":
+        if self.params is None:
+            sd = self._nomad.state_dict_ref
+            if sd is None:
+                raise ValueError("the network's parameters need the Nomad to be built with keep_state_dict=True")
+            dev = self._nomad.engine.device
+            self.params = OrderedDict(
+                (k, nn.Parameter(v.detach().to(dev, torch.float32).clone(), requires_grad=False)) for k, v in sd.items()
+                if torch.is_tensor(v) and (k.startswith("ssl_model.") or k.startswith("embedding_layer.")))
+            self._seen = self._keys()
+            self._nomad.engine.sync_hook = self.sync
+        return self.params
+
+    def _keys(self):
+        return [(p._version, p.data_ptr()) for p in self.params.values()]
+
+    def sync(self):
+        keys = self._keys()
+        if keys == self._seen:
+            return
+        changed = [k for k, a, b in zip(self.params, keys, self._seen) if a != b]
+        dev = {k: p.detach().contiguous() for k, p in self.params.items()}
+        engine = self._nomad.engine
+        if any(not k.startswith(CONV_PREFIX) for k in changed):
+            engine.refresh_weights(dev)
+        if any(k.startswith(CONV_PREFIX) for k in changed):
+            engine.refresh_conv_weights(dev)
+        self._seen = keys
+
+    def trainable(self, head: int):
+        """[(name, parameter)] that require grad and lie on the path of ``head`` (1: not the NOMAD head)."""
+        if self.params is None:
+            return []
+        return [(k, p) for k, p in self.params.items() if p.requires_grad and not k.endswith("mask_emb")
+                and not (head == 1 and k.startswith("embedding_layer."))]
+
+
 class _NetworkFn(torch.autograd.Function):
     """The network as an autograd node: save-mode forward (``nomad_b200_layers_fwd_save``) of a (B, N) batch, backward
-    from whichever outputs were used (``nomad_b200_layers_bwd``; unused outputs reach it as NULL).  ``head``: 0 = NOMAD
-    head, outputs (emb,); 1 = loss head, outputs (12 layer outputs..., emb).  Only ``wav`` gets a gradient."""
+    from whichever outputs were used (unused outputs reach it as NULL).  ``head``: 0 = NOMAD head, outputs (emb,); 1 =
+    loss head, outputs (12 layer outputs..., emb).  ``params``: the trainable parameters of the store (names in
+    ``names``); with none, only ``wav`` gets a gradient (``nomad_b200_layers_bwd``), else the forward saves for the
+    parameter gradients too and the backward is ``nomad_b200_layers_bwd_params``, with the waveform gradient only when
+    ``wav`` needs one and the conv encoder's gradients only when one of its tensors is trainable."""
 
     @staticmethod
-    def forward(ctx, wav, engine, head, feature_grad_mult):
+    def forward(ctx, wav, engine, head, feature_grad_mult, store, names, *params):
         ctx.set_materialize_grads(False)
-        ctx.engine, ctx.fgm, ctx.want_layers = engine, float(feature_grad_mult), head == 1
+        ctx.engine, ctx.fgm, ctx.want_layers, ctx.store, ctx.names = engine, float(feature_grad_mult), head == 1, store, names
         ctx.in_shape, ctx.in_device, ctx.in_dtype = wav.shape, wav.device, wav.dtype
+        ctx.conv = any(k.startswith(CONV_PREFIX) for k in names)
+        ctx.flags = (_lib.SAVE_PARAMS if names else 0) | (_lib.SAVE_CONV if ctx.conv else 0)
+        # the weight-norm backward of the positional conv needs the values this forward runs with
+        by_name = dict(zip(names, params))
+        ctx.pos_wn = (by_name[POS_V].detach().clone(), by_name[POS_G].detach().clone()) \
+            if (POS_V in by_name or POS_G in by_name) else None
         flat = wav.detach().reshape(-1, wav.shape[-1]).to(engine.device, torch.float32).contiguous()
-        layers, emb, saved = engine.layers_fwd_save(flat, head, want_layers=ctx.want_layers)
+        layers, emb, saved = engine.layers_fwd_save(flat, head, want_layers=ctx.want_layers, flags=ctx.flags)
+        ctx.generation = engine.weight_generation
         ctx.save_for_backward(flat, saved)  # released after the backward (unless the graph is retained)
         return (*layers.unbind(0), emb) if ctx.want_layers else emb
 
     @staticmethod
     def backward(ctx, *grads):
+        if ctx.engine.weight_generation != ctx.generation:
+            raise RuntimeError("the network's weights changed between this forward and its backward (an optimiser step "
+                               "reached the device through a later call): run the forward again")
         flat, saved = ctx.saved_tensors
         g_layers = list(grads[:-1]) if ctx.want_layers else [None] * NUM_LAYERS
-        d = ctx.engine.layers_bwd(saved, flat, g_layers, grads[-1], ctx.fgm)
-        return d.reshape(ctx.in_shape).to(ctx.in_device, ctx.in_dtype), None, None, None
+        want_wav = ctx.needs_input_grad[0]
+        if not ctx.names:
+            d = ctx.engine.layers_bwd(saved, flat, g_layers, grads[-1], ctx.fgm)
+            return d.reshape(ctx.in_shape).to(ctx.in_device, ctx.in_dtype), None, None, None, None, None
+        d, flat_g, conv_g, scale = ctx.engine.layers_bwd_params(saved, flat, g_layers, grads[-1], ctx.fgm, ctx.flags,
+                                                                want_wav, True, ctx.conv)
+        params = ctx.store.params
+        v, g = ctx.pos_wn if ctx.pos_wn is not None else (params[POS_V], params[POS_G])
+        named = grads_by_name(flat_g, scale, v, g, conv_g,
+                              {k: p.shape for k, p in params.items() if k.startswith(CONV_PREFIX)} if ctx.conv else None)
+        d_wav = (d / scale).reshape(ctx.in_shape).to(ctx.in_device, ctx.in_dtype) if want_wav else None
+        return (d_wav, None, None, None, None, None, *[named[k].reshape(params[k].shape) for k in ctx.names])
+
+
+def _network(wav, engine, head, feature_grad_mult, store):
+    """The differentiable call when grad is enabled and ``wav`` or a parameter on this head's path requires grad, else
+    None (the caller runs the no-grad path)."""
+    if not torch.is_grad_enabled():
+        return None
+    trainable = store.trainable(head) if store is not None else []
+    if not (wav.requires_grad or trainable):
+        return None
+    names = tuple(k for k, _ in trainable)
+    return _NetworkFn.apply(wav, engine, head, feature_grad_mult, store, names, *[p for _, p in trainable])
 
 
 def _differentiable(wav) -> bool:
@@ -83,13 +175,39 @@ class TripletModel:
     and ``wav.requires_grad`` the call is differentiable wrt ``wav`` (fp16 operands, fairseq's GradMultiply of
     ``feature_grad_mult()`` on the conv features)."""
 
-    def __init__(self, engine: Engine, feature_grad_mult=lambda: 0.1):
+    def __init__(self, engine: Engine, feature_grad_mult=lambda: 0.1, store: Optional[_ParamStore] = None):
         self.engine = engine
         self.ssl_features = SSL_OUT_DIM
         self.feature_grad_mult = feature_grad_mult  # zero-argument callable, read at each differentiable call
+        self._store = store
 
     def eval(self):
         return self
+
+    def _params(self) -> "OrderedDict[str, nn.Parameter]":
+        if self._store is None:
+            raise ValueError("the network's parameters need the Nomad to be built with keep_state_dict=True")
+        return self._store.build()
+
+    def named_parameters(self):
+        """(checkpoint name, fp32 ``nn.Parameter`` on the engine's device): every ``ssl_model.*`` tensor and the head
+        ``embedding_layer.1.*``, shared with ``lossnet_layers``.  Needs ``keep_state_dict=True``."""
+        return iter(self._params().items())
+
+    def parameters(self):
+        return iter(self._params().values())
+
+    def requires_grad_(self, requires_grad: bool = True):
+        """Train (or freeze) every parameter except ``mask_emb``.  Freeze the conv feature encoder afterwards with
+        ``requires_grad_(False)`` on the ``ssl_model.feature_extractor.*`` tensors."""
+        for k, p in self._params().items():
+            if not k.endswith("mask_emb"):
+                p.requires_grad_(requires_grad)
+        return self
+
+    def state_dict(self) -> "OrderedDict[str, torch.Tensor]":
+        """The parameters, detached: ``Nomad(state_dict=nomad.model.state_dict())`` rebuilds this network."""
+        return OrderedDict((k, p.detach()) for k, p in self._params().items())
 
     def to(self, *_a, **_k):
         return self
@@ -102,8 +220,10 @@ class TripletModel:
             wav = wav.squeeze(1)  # nomad.py:225
         if wav.dim() == 1:
             wav = wav.unsqueeze(0)
-        if _differentiable(wav):
-            return _NetworkFn.apply(wav, self.engine, 0, self.feature_grad_mult())
+        if torch.is_tensor(wav):
+            out = _network(wav, self.engine, 0, self.feature_grad_mult(), self._store)
+            if out is not None:
+                return out
         with torch.no_grad():
             B, N = wav.shape
             flat = wav.to(self.engine.device, torch.float32).contiguous().reshape(-1)
@@ -116,10 +236,11 @@ class LossNetLayers:
     fairseq's GradMultiply of ``feature_grad_mult()`` on the conv features); the backward uses the head as it was at
     the forward."""
 
-    def __init__(self, engine: Engine, feature_grad_mult=lambda: 0.1):
+    def __init__(self, engine: Engine, feature_grad_mult=lambda: 0.1, store: Optional[_ParamStore] = None):
         self.engine = engine
         self.ssl_features = SSL_OUT_DIM
         self.feature_grad_mult = feature_grad_mult  # zero-argument callable, read at each differentiable call
+        self._store = store  # the network's parameters, shared with TripletModel (the loss head below is separate)
         # freshly initialised head, exactly like the reference (nomad.py:238-241)
         self.embedding_layer = nn.Sequential(nn.ReLU(), nn.Linear(SSL_OUT_DIM, EMB_DIM))
         self._synced = None
@@ -139,8 +260,10 @@ class LossNetLayers:
 
     def forward(self, wav: torch.Tensor) -> List[torch.Tensor]:
         self.sync_head()
-        if _differentiable(wav):
-            return list(_NetworkFn.apply(wav, self.engine, 1, self.feature_grad_mult()))
+        if torch.is_tensor(wav):
+            out = _network(wav, self.engine, 1, self.feature_grad_mult(), self._store)
+            if out is not None:
+                return list(out)
         with torch.no_grad():
             layers, emb = self.engine.layers(wav)
             return [layers[i] for i in range(layers.shape[0])] + [emb]
@@ -212,9 +335,10 @@ class Nomad():
         self.precision = precision or os.environ.get("NOMAD_B200_PRECISION", "fp16")
         self.engine = Engine(state_dict, index, self.precision)
         self.state_dict_ref = state_dict if keep_state_dict else None   # fine-tuning (triplet.py) needs the fp32 tensors
-        self.model = TripletModel(self.engine, lambda: self.feature_grad_mult)
+        self._store = _ParamStore(self)
+        self.model = TripletModel(self.engine, lambda: self.feature_grad_mult, self._store)
         # NOMAD loss model shares the same network (nomad.py:70-72)
-        self.lossnet_layers = LossNetLayers(self.engine, lambda: self.feature_grad_mult)
+        self.lossnet_layers = LossNetLayers(self.engine, lambda: self.feature_grad_mult, self._store)
         self.nomad_loss = NomadLoss()
         # fairseq applies GradMultiply(feature_grad_mult) to the conv features (wav2vec 2.0 base: 0.1)
         self.feature_grad_mult = float(feature_grad_mult)
@@ -304,9 +428,9 @@ class Nomad():
 
     def forward(self, estimate, clean):
         """Differentiable NOMAD loss (``nomad.py:142-146``): 0-dim tensor, grad flows to ``estimate``.  When ``clean``
-        requires grad too (grad enabled), the reference's own composition runs instead of the fused CUDA-graph step,
-        so both inputs get their gradient."""
-        if _differentiable(clean):
+        requires grad too, or a network parameter does (grad enabled), the reference's own composition runs instead of
+        the fused CUDA-graph step, so both inputs and the parameters get their gradient."""
+        if _differentiable(clean) or (torch.is_grad_enabled() and self._store.trainable(1)):
             return self.nomad_loss(self.lossnet_layers(clean), self.lossnet_layers(estimate))
         self.lossnet_layers.sync_head()
         return _NomadLossFn.apply(estimate, clean, self)

@@ -17,8 +17,9 @@ stochastic).
 from __future__ import annotations
 
 import ctypes as C
+import functools
 from collections import OrderedDict
-from typing import Dict, Tuple
+from typing import Dict, Optional, Tuple
 
 import torch
 
@@ -26,6 +27,7 @@ from . import _lib
 from .engine import Engine, _ptr, _stream_ptr
 
 
+@functools.lru_cache(maxsize=None)
 def grad_segments(conv: bool = False):
     """[(name, offset, numel)] of the flat gradient buffer (``conv``: of the conv-encoder buffer), as the library lays it
     out."""
@@ -60,6 +62,49 @@ SHAPES = {"qkv.weight": (2304, 768), "self_attn.out_proj.weight": (768, 768), "f
           "fc2.weight": (768, 3072), "post_extract_proj.weight": (768, 512), "embedding_layer.1.weight": (256, 768)}
 
 
+POS_V, POS_G = "ssl_model.encoder.pos_conv.0.weight_v", "ssl_model.encoder.pos_conv.0.weight_g"
+
+
+def grads_by_name(flat: torch.Tensor, scale, weight_v: torch.Tensor, weight_g: torch.Tensor,
+                  conv_flat: Optional[torch.Tensor] = None, conv_shapes=None) -> "OrderedDict[str, torch.Tensor]":
+    """The library's flat gradient buffers (``grad_segments()`` and, when ``conv_flat`` is given, ``grad_segments(conv=
+    True)``; both times the scale S: a float or a 0-dim tensor on their device) -> {state_dict key: gradient}.  The fused
+    q|k|v rows are split (q carries the kernel's head_dim^-0.5), the positional conv's folded-weight gradient goes through
+    the weight-norm backward to ``weight_v`` / ``weight_g`` (the values the forward used), ``conv_shapes`` gives the
+    checkpoint shapes of the conv tensors."""
+    flat = flat / scale
+    grads: "OrderedDict[str, torch.Tensor]" = OrderedDict()
+    for name, off, cnt in grad_segments():
+        g = flat[off:off + cnt]
+        leaf = next((k for k in SHAPES if name.endswith(k)), None)
+        if leaf is not None:
+            g = g.view(SHAPES[leaf])
+        if name.endswith("qkv.weight") or name.endswith("qkv.bias"):
+            base = name[: -len("qkv.weight")] if name.endswith("weight") else name[: -len("qkv.bias")]
+            kind = "weight" if name.endswith("weight") else "bias"
+            q, k, v = g[:768], g[768:1536], g[1536:]
+            grads[base + f"self_attn.q_proj.{kind}"] = q * 0.125   # the kernel's q rows carry head_dim^-0.5
+            grads[base + f"self_attn.k_proj.{kind}"] = k
+            grads[base + f"self_attn.v_proj.{kind}"] = v
+        elif name.endswith("pos_conv.0.folded_weight"):
+            # [g][n][tap][c] -> (out = g * 48 + n, in = c, tap); then through weight_norm(dim=2): w = g * v / ||v||
+            dw = g.view(16, 48, 128, 48).permute(0, 1, 3, 2).reshape(768, 48, 128)
+            with torch.enable_grad():
+                v = weight_v.detach().to(flat.device, torch.float32).requires_grad_(True)
+                gg = weight_g.detach().to(flat.device, torch.float32).requires_grad_(True)
+                w = gg * v / v.pow(2).sum(dim=(0, 1), keepdim=True).sqrt()
+                gv, ggr = torch.autograd.grad(w, (v, gg), dw)
+            grads[POS_V] = gv
+            grads[POS_G] = ggr
+        else:
+            grads[name] = g
+    if conv_flat is not None:
+        conv_flat = conv_flat / scale
+        for name, off, cnt in grad_segments(conv=True):   # already in the checkpoint's (out, in, tap) order
+            grads[name] = conv_flat[off:off + cnt].view(conv_shapes[name])
+    return grads
+
+
 def triplet_loss_and_grads(engine: Engine, state_dict, anchor: torch.Tensor, positive: torch.Tensor, negative: torch.Tensor,
                            margin: float = 0.2, freeze_convnet: bool = True,
                            feature_grad_mult: float = 0.1) -> Tuple[torch.Tensor, "OrderedDict[str, torch.Tensor]"]:
@@ -68,6 +113,7 @@ def triplet_loss_and_grads(engine: Engine, state_dict, anchor: torch.Tensor, pos
     ``feature_grad_mult`` on the conv features (the frozen step has no gradient below the conv features for it to scale).
     ``anchor`` / ``positive`` / ``negative``: (B, N) or (B, 1, N) waveforms of one common length."""
     lib = engine.lib
+    engine.sync_weights()
     sq = lambda t: (t.squeeze(1) if t.dim() == 3 else t).to(engine.device, torch.float32)
     wav = torch.cat([sq(anchor), sq(positive), sq(negative)]).contiguous()
     B, N = wav.shape[0] // 3, wav.shape[1]
@@ -89,35 +135,9 @@ def triplet_loss_and_grads(engine: Engine, state_dict, anchor: torch.Tensor, pos
                                                            C.c_float(feature_grad_mult), _ptr(loss), _ptr(flat), _ptr(conv_flat),
                                                            C.byref(scale), wp, wbytes, _stream_ptr()),
                        "nomad_b200_triplet_conv_fwd_bwd")
-    flat = flat / scale.value
-    grads: "OrderedDict[str, torch.Tensor]" = OrderedDict()
-    for name, off, cnt in grad_segments():
-        g = flat[off:off + cnt]
-        leaf = next((k for k in SHAPES if name.endswith(k)), None)
-        if leaf is not None:
-            g = g.view(SHAPES[leaf])
-        if name.endswith("qkv.weight") or name.endswith("qkv.bias"):
-            base = name[: -len("qkv.weight")] if name.endswith("weight") else name[: -len("qkv.bias")]
-            kind = "weight" if name.endswith("weight") else "bias"
-            q, k, v = g[:768], g[768:1536], g[1536:]
-            grads[base + f"self_attn.q_proj.{kind}"] = q * 0.125   # the kernel's q rows carry head_dim^-0.5
-            grads[base + f"self_attn.k_proj.{kind}"] = k
-            grads[base + f"self_attn.v_proj.{kind}"] = v
-        elif name.endswith("pos_conv.0.folded_weight"):
-            # [g][n][tap][c] -> (out = g * 48 + n, in = c, tap); then through weight_norm(dim=2): w = g * v / ||v||
-            dw = g.view(16, 48, 128, 48).permute(0, 1, 3, 2).reshape(768, 48, 128)
-            v = _device_copy(engine, state_dict, "ssl_model.encoder.pos_conv.0.weight_v").requires_grad_(True)
-            gg = _device_copy(engine, state_dict, "ssl_model.encoder.pos_conv.0.weight_g").requires_grad_(True)
-            w = gg * v / v.pow(2).sum(dim=(0, 1), keepdim=True).sqrt()
-            w.backward(dw)
-            grads["ssl_model.encoder.pos_conv.0.weight_v"] = v.grad
-            grads["ssl_model.encoder.pos_conv.0.weight_g"] = gg.grad
-        else:
-            grads[name] = g
-    if not freeze_convnet:
-        conv_flat = conv_flat / scale.value
-        for name, off, cnt in grad_segments(conv=True):   # already in the checkpoint's (out, in, tap) order
-            grads[name] = conv_flat[off:off + cnt].view(state_dict[name].shape)
+    conv_shapes = None if freeze_convnet else {k: state_dict[k].shape for k, _, _ in grad_segments(conv=True)}
+    grads = grads_by_name(flat, scale.value, _device_copy(engine, state_dict, POS_V), _device_copy(engine, state_dict, POS_G),
+                          None if freeze_convnet else conv_flat, conv_shapes)
     return loss, grads
 
 
