@@ -71,7 +71,10 @@ NOMAD_B200_API int nomad_b200_create(nomad_b200_handle** out, const nomad_b200_t
                                      int precision_mode, int device);
 /* Switch a handle created with NOMAD_B200_PRECISION_FP32 between the two arithmetic classes (a handle created with
  * NOMAD_B200_PRECISION_FP16 holds the fp16 weights only).  The scoring entry points (embed, score, layers_fwd and
- * their _host variants) honour the mode; the loss path always runs fp16 operands. */
+ * their _host variants) and the waveform-gradient entry points (loss_fwd_bwd, layers_fwd_save / _ex with flags 0,
+ * layers_bwd) honour the mode.  Parameter gradients (NOMAD_B200_SAVE_* forwards, layers_bwd_params, the triplet steps)
+ * run fp16 operands in either mode.  An FP32 handle also keeps the transposed hi + lo weight planes of the fp32-class
+ * backward (~0.38 GB beside the ~0.38 GB of forward planes). */
 NOMAD_B200_API int nomad_b200_set_precision(nomad_b200_handle* h, int precision_mode);
 NOMAD_B200_API int nomad_b200_get_precision(nomad_b200_handle* h);
 NOMAD_B200_API int nomad_b200_destroy(nomad_b200_handle* h);
@@ -103,6 +106,10 @@ NOMAD_B200_API int nomad_b200_embed_host(nomad_b200_handle* h, const float* wav_
  * d_est: B x N fp32 device = d loss / d estimate (already including ``feature_grad_mult``), or NULL
  * for forward only.  Weight gradients are not produced (wheel 0.0.8 semantics, see DESIGN.md). */
 NOMAD_B200_API size_t nomad_b200_loss_workspace_bytes(int B, int64_t N, int with_grad);
+/* The workspace a handle in `precision_mode` needs (mode 0: exactly nomad_b200_loss_workspace_bytes).  In FP32 mode the
+ * step runs the fp32-class save-mode forward of both halves and the fp32-class backward of the estimates (hi + lo
+ * operand planes, fp32 LayerNorm / softmax / GELU; see DESIGN.md section 5e), eagerly; a smaller workspace is refused. */
+NOMAD_B200_API size_t nomad_b200_loss_workspace_bytes_mode(int B, int64_t N, int with_grad, int precision_mode);
 NOMAD_B200_API int nomad_b200_loss_fwd_bwd(nomad_b200_handle* h, const float* est_dev, const float* clean_dev, int B, int64_t N,
                             float feature_grad_mult, float* loss_dev, float* d_est_dev, void* workspace_dev,
                             size_t workspace_bytes, void* stream);
@@ -116,13 +123,16 @@ NOMAD_B200_API int nomad_b200_layers_fwd(nomad_b200_handle* h, const float* wav_
                           float* emb_dev, void* workspace_dev, size_t workspace_bytes, void* stream);
 
 /* ---- autograd through ``LossNetLayers`` / ``TripletModel`` (nomad.py:224-258 are plain nn.Modules) ------------------
- * Save-mode forward of the network for B utterances of N samples (fp16 operands, like the loss path).  Writes the 12
+ * Save-mode forward of the network for B utterances of N samples, in the handle's precision_mode.  Writes the 12
  * post-LayerNorm layer outputs (12 x B x T x 768 fp32, layer major, may be NULL) and the head output (B x 256, may be
  * NULL).  head: 0 = the NOMAD head (TripletModel), 1 = the loss head set by nomad_b200_set_loss_head (LossNetLayers).
  * Everything the backward needs goes into ``saved`` (caller-owned, 1024-byte aligned, nomad_b200_layers_saved_bytes
  * bytes, alive and untouched until the last backward that uses it): the save-mode activations, the pooled features and
  * a snapshot of the chosen head, so a later nomad_b200_set_loss_head does not change the backward. */
 NOMAD_B200_API size_t nomad_b200_layers_saved_bytes(int B, int64_t N);
+/* Saved-buffer size for a forward in `precision_mode` (mode 0: exactly nomad_b200_layers_saved_bytes).  The buffer's
+ * record stores the mode of the forward that wrote it. */
+NOMAD_B200_API size_t nomad_b200_layers_saved_bytes_mode(int B, int64_t N, int precision_mode);
 NOMAD_B200_API int nomad_b200_layers_fwd_save(nomad_b200_handle* h, const float* wav_dev, int B, int64_t N, int head,
                                               float* layers_dev, float* emb_dev, void* saved_dev, size_t saved_bytes,
                                               void* stream);
@@ -131,8 +141,13 @@ NOMAD_B200_API int nomad_b200_layers_fwd_save(nomad_b200_handle* h, const float*
  * each, 16-byte aligned, NULL = zero gradient) or NULL; g_emb: B x 256 fp32 device or NULL.  ``saved`` comes from
  * nomad_b200_layers_fwd_save with the same B and N, wav_dev is the waveform given to it.  The power-of-two scale that
  * keeps the 16-bit gradients in range is chosen on the device from max|g|.  The saved buffer is only read: one forward
- * may be differentiated more than once.  No weight gradients; no host synchronisation. */
+ * may be differentiated more than once.  No weight gradients.  The backward runs in the mode the forward was saved in,
+ * which must be the handle's current mode (a buffer saved before a nomad_b200_set_precision is refused); on a handle
+ * created with NOMAD_B200_PRECISION_FP32 the call reads the buffer's record back first (one stream synchronisation),
+ * otherwise it does not synchronise.  Workspace: nomad_b200_layers_bwd_workspace_bytes_mode with the handle's mode
+ * (mode 0: exactly nomad_b200_layers_bwd_workspace_bytes). */
 NOMAD_B200_API size_t nomad_b200_layers_bwd_workspace_bytes(int B, int64_t N);
+NOMAD_B200_API size_t nomad_b200_layers_bwd_workspace_bytes_mode(int B, int64_t N, int precision_mode);
 NOMAD_B200_API int nomad_b200_layers_bwd(nomad_b200_handle* h, const void* saved_dev, size_t saved_bytes, const float* wav_dev,
                                          int B, int64_t N, const float* const* g_layers, const float* g_emb,
                                          float feature_grad_mult, float* d_wav_dev, void* workspace_dev,
@@ -143,14 +158,16 @@ NOMAD_B200_API int nomad_b200_layers_bwd(nomad_b200_handle* h, const void* saved
  * weight gradients need (each layer's GELU(fc1) activations); NOMAD_B200_SAVE_CONV saves the conv0 GELU gradient without
  * the GroupNorm gamma * rstd factor, as the conv-encoder gradients need it.  The flags are recorded in the saved buffer
  * (size: nomad_b200_layers_saved_bytes_ex; flags 0 = nomad_b200_layers_saved_bytes).  A buffer saved with flags != 0 goes
- * to nomad_b200_layers_bwd_params only.
+ * to nomad_b200_layers_bwd_params only.  Everything in this block runs fp16 operands whatever the handle's precision_mode
+ * (fine-tuning runs in mode 0: nomad_b200_refresh_weights refuses an FP32-mode handle); a flags-0 forward saved in FP32
+ * mode is refused by nomad_b200_layers_bwd_params.
  * nomad_b200_layers_bwd_params: from the same g_layers / g_emb as nomad_b200_layers_bwd, the waveform gradient (d_wav,
  * B x N, or NULL) and the gradient of every trainable parameter: grads (NULL, or nomad_b200_triplet_grad_floats() fp32
  * values laid out as nomad_b200_triplet_grad_segment enumerates; needs SAVE_PARAMS), conv_grads (NULL = conv encoder
  * frozen, or nomad_b200_triplet_conv_grad_floats() values as nomad_b200_triplet_conv_grad_segment; needs SAVE_CONV and
  * grads).  The embedding-head slots hold the NOMAD head's gradient for a head-0 forward and zeros for head 1.  Every
  * output is multiplied by the power-of-two scale S chosen on the device, which is written to *grad_scale_dev (device
- * float): divide it out on the device.  The call reads the saved buffer's 16-byte record back before launching anything
+ * float): divide it out on the device.  The call reads the saved buffer's record back before launching anything
  * (one stream synchronisation) and refuses gradients the forward did not save for.  With d_wav NULL and the conv
  * encoder frozen the conv-stack backward is skipped.  Workspace: nomad_b200_layers_bwd_params_workspace_bytes with the
  * forward's flags.  grads / conv_grads / g_emb / g_layers[l]: 16-byte aligned. */

@@ -51,14 +51,17 @@ PROTOTYPES = {
     "nomad_b200_embed": (C.c_int, [c_vp, c_vp, C.POINTER(c_i64), C.c_int, c_vp, c_vp, C.c_size_t, c_vp]),
     "nomad_b200_embed_host": (C.c_int, [c_vp, c_vp, C.POINTER(c_i64), C.c_int, c_vp, c_vp, C.c_size_t, c_vp]),
     "nomad_b200_loss_workspace_bytes": (C.c_size_t, [C.c_int, c_i64, C.c_int]),
+    "nomad_b200_loss_workspace_bytes_mode": (C.c_size_t, [C.c_int, c_i64, C.c_int, C.c_int]),
     "nomad_b200_loss_fwd_bwd": (C.c_int, [c_vp, c_vp, c_vp, C.c_int, c_i64, C.c_float, c_vp, c_vp, c_vp,
                                           C.c_size_t, c_vp]),
     "nomad_b200_layers_workspace_bytes": (C.c_size_t, [C.c_int, c_i64]),
     "nomad_b200_num_frames": (c_i64, [c_i64]),
     "nomad_b200_layers_fwd": (C.c_int, [c_vp, c_vp, C.c_int, c_i64, c_vp, c_vp, c_vp, C.c_size_t, c_vp]),
     "nomad_b200_layers_saved_bytes": (C.c_size_t, [C.c_int, c_i64]),
+    "nomad_b200_layers_saved_bytes_mode": (C.c_size_t, [C.c_int, c_i64, C.c_int]),
     "nomad_b200_layers_fwd_save": (C.c_int, [c_vp, c_vp, C.c_int, c_i64, C.c_int, c_vp, c_vp, c_vp, C.c_size_t, c_vp]),
     "nomad_b200_layers_bwd_workspace_bytes": (C.c_size_t, [C.c_int, c_i64]),
+    "nomad_b200_layers_bwd_workspace_bytes_mode": (C.c_size_t, [C.c_int, c_i64, C.c_int]),
     "nomad_b200_layers_bwd": (C.c_int, [c_vp, c_vp, C.c_size_t, c_vp, C.c_int, c_i64, C.POINTER(c_vp), c_vp, C.c_float, c_vp,
                                         c_vp, C.c_size_t, c_vp]),
     "nomad_b200_layers_saved_bytes_ex": (C.c_size_t, [C.c_int, c_i64, C.c_int]),

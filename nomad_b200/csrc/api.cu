@@ -402,6 +402,16 @@ static int upload_split(Handle* h, const std::vector<float>& w, SplitW* out) {
     return 0;
 }
 
+static std::vector<float> transpose_f32(const float* w, size_t rows, size_t cols) {
+    std::vector<float> t(rows * cols);
+    for (size_t r = 0; r < rows; ++r)
+        for (size_t c = 0; c < cols; ++c) t[c * rows + r] = w[r * cols + c];
+    return t;
+}
+
+// The transposed planes (the *_t members, for the dgrad GEMMs of the fp32-class waveform backward) take as much device
+// memory as the forward planes: ~0.38 GB more per FP32 handle.  Their max |w| and so their power-of-two scale equal the
+// forward tensor's, so the hi / lo values are the forward planes' values, transposed.
 static int build_weights_precise(Handle* h, TensorTable& tt) {
     PreciseWeights& pw = h->pw;
     const std::string P = "ssl_model.";
@@ -413,9 +423,24 @@ static int build_weights_precise(Handle* h, TensorTable& tt) {
             for (int c = 0; c < 512; ++c)
                 for (int j = 0; j < k; ++j) fw[(size_t)o * (k * 512) + (size_t)j * 512 + c] = cw[((size_t)o * 512 + c) * k + j];
         NB_TRY(upload_split(h, fw, &pw.conv[l]));
+        std::vector<float> bw((size_t)512 * 512 * k);  // dgrad: per tap [cin][cout]
+        for (int o = 0; o < 512; ++o)
+            for (int c = 0; c < 512; ++c)
+                for (int j = 0; j < k; ++j) bw[((size_t)j * 512 + c) * 512 + o] = cw[((size_t)o * 512 + c) * k + j];
+        NB_TRY(upload_split(h, bw, &pw.conv_t[l]));
+        if (k == 3) {  // even input rows: [cin][tap 2: cout | tap 0: cout]
+            std::vector<float> ew((size_t)512 * 1024);
+            for (int c = 0; c < 512; ++c)
+                for (int o = 0; o < 512; ++o) {
+                    ew[(size_t)c * 1024 + o] = cw[((size_t)o * 512 + c) * 3 + 2];
+                    ew[(size_t)c * 1024 + 512 + o] = cw[((size_t)o * 512 + c) * 3 + 0];
+                }
+            NB_TRY(upload_split(h, ew, &pw.conv_te[l]));
+        }
     }
     GET(pwt, P + "post_extract_proj.weight", 768LL * 512);
     NB_TRY(upload_split(h, std::vector<float>(pwt, pwt + 768 * 512), &pw.proj));
+    NB_TRY(upload_split(h, transpose_f32(pwt, 768, 512), &pw.proj_t));
     GET(pv, P + "encoder.pos_conv.0.weight_v", 768LL * POS_GC * POS_K);
     GET(pg, P + "encoder.pos_conv.0.weight_g", POS_K);
     {
@@ -423,14 +448,18 @@ static int build_weights_precise(Handle* h, TensorTable& tt) {
         for (size_t i = 0; i < (size_t)768 * POS_GC; ++i)
             for (int k = 0; k < POS_K; ++k) nrm[k] += (double)pv[i * POS_K + k] * pv[i * POS_K + k];
         for (int k = 0; k < POS_K; ++k) nrm[k] = (double)pg[k] / std::sqrt(nrm[k]);
-        std::vector<float> fw((size_t)POS_G * POS_GC * POS_K * POS_GC);  // [g][n][tap * 48 + c]
+        // forward [g][n][tap * 48 + c]; dgrad [g][c][tap' * 48 + n] with tap' = 127 - tap (as Weights::pos_wt)
+        std::vector<float> fw((size_t)POS_G * POS_GC * POS_K * POS_GC), bw(fw.size());
         for (int g = 0; g < POS_G; ++g)
             for (int n = 0; n < POS_GC; ++n)
                 for (int c = 0; c < POS_GC; ++c)
-                    for (int k = 0; k < POS_K; ++k)
-                        fw[((size_t)(g * POS_GC + n)) * (POS_K * POS_GC) + (size_t)k * POS_GC + c] =
-                            (float)((double)pv[((size_t)(g * POS_GC + n) * POS_GC + c) * POS_K + k] * nrm[k]);
+                    for (int k = 0; k < POS_K; ++k) {
+                        const float v = (float)((double)pv[((size_t)(g * POS_GC + n) * POS_GC + c) * POS_K + k] * nrm[k]);
+                        fw[((size_t)(g * POS_GC + n)) * (POS_K * POS_GC) + (size_t)k * POS_GC + c] = v;
+                        bw[((size_t)(g * POS_GC + c)) * (POS_K * POS_GC) + (size_t)(POS_K - 1 - k) * POS_GC + n] = v;
+                    }
         NB_TRY(upload_split(h, fw, &pw.pos));
+        NB_TRY(upload_split(h, bw, &pw.pos_t));
     }
     for (int l = 0; l < LAYERS; ++l) {
         const std::string Q = P + "encoder.layers." + std::to_string(l) + ".";
@@ -444,12 +473,16 @@ static int build_weights_precise(Handle* h, TensorTable& tt) {
             v[(size_t)2 * 768 * 768 + i] = wv[i];
         }
         NB_TRY(upload_split(h, v, &pw.qkv[l]));
+        NB_TRY(upload_split(h, transpose_f32(v.data(), 2304, 768), &pw.qkv_t[l]));
         GET(wo, Q + "self_attn.out_proj.weight", 768LL * 768);
         GET(w1, Q + "fc1.weight", 3072LL * 768);
         GET(w2, Q + "fc2.weight", 768LL * 3072);
         NB_TRY(upload_split(h, std::vector<float>(wo, wo + 768 * 768), &pw.o[l]));
         NB_TRY(upload_split(h, std::vector<float>(w1, w1 + (size_t)3072 * 768), &pw.fc1[l]));
         NB_TRY(upload_split(h, std::vector<float>(w2, w2 + (size_t)768 * 3072), &pw.fc2[l]));
+        NB_TRY(upload_split(h, transpose_f32(wo, 768, 768), &pw.o_t[l]));
+        NB_TRY(upload_split(h, transpose_f32(w1, 3072, 768), &pw.fc1_t[l]));
+        NB_TRY(upload_split(h, transpose_f32(w2, 768, 3072), &pw.fc2_t[l]));
     }
     pw.built = true;
     return 0;

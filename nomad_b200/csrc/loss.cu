@@ -11,7 +11,7 @@
 #include <cstring>
 
 #include "../../include/nomad_b200.h"
-#include "kernels.cuh"
+#include "precise.cuh"
 
 namespace nb {
 
@@ -702,6 +702,21 @@ size_t nomad_b200_loss_workspace_bytes(int B, int64_t N, int with_grad) {
     if (core == 0) return 0;
     // + estimate / clean / gradient / loss staging: the step is replayed as a CUDA graph over fixed addresses
     return (core + 1023) / 1024 * 1024 + loss_stage_bytes(B, N);
+}
+
+// fp32-class step: [save-mode forward of the 2B utterances | L1 sums, pooled features, head gradient | backward scratch]
+static size_t loss_precise_bytes(const Plan& p, int B, bool with_grad, size_t* fwd, size_t* mid) {
+    *fwd = carve_precise(p, nullptr, nullptr, true);
+    *mid = carve_loss(p, B, 0, 0, 0, false, nullptr, nullptr);
+    return *fwd + *mid + (with_grad ? precise_bwd_bytes(p, B) : 0);
+}
+
+size_t nomad_b200_loss_workspace_bytes_mode(int B, int64_t N, int with_grad, int precision_mode) {
+    if (precision_mode != NOMAD_B200_PRECISION_FP32) return nomad_b200_loss_workspace_bytes(B, N, with_grad);
+    Plan p;
+    if (loss_plan(B, N, &p)) return 0;
+    size_t fwd, mid;
+    return loss_precise_bytes(p, B, with_grad != 0, &fwd, &mid);
 }
 
 }  // extern "C"
@@ -1625,6 +1640,58 @@ static int loss_run(nomad_b200_handle* hh, const float* est_dev, const float* cl
     return backward_chain(h, ws, L, B, Fe, R0e, pos_rows_e, T, seed_layer, feature_grad_mult, S, est_dev, N, d_est_dev, st, nullptr);
 }
 
+// The fused loss step on a handle in NOMAD_B200_PRECISION_FP32: the fp32-class save-mode forward of both halves, the same
+// L1 / head kernels as loss_run on its pre-LayerNorm sums and residual stream, and the fp32-class waveform backward of
+// the estimate half.  Always eager (the step is dominated by its split-operand GEMMs, not by launch gaps).
+static int loss_run_precise(Handle* h, const float* est_dev, const float* clean_dev, int B, int64_t N, float feature_grad_mult,
+                            float* loss_dev, float* d_est_dev, void* workspace_dev, size_t workspace_bytes, cudaStream_t st) {
+    const bool with_grad = d_est_dev != nullptr;
+    const Weights& w = h->w;
+    Plan p;
+    NB_TRY(loss_plan(B, N, &p));
+    const long long clean_off = (long long)(((intptr_t)clean_dev - (intptr_t)est_dev) / 4);
+    for (int b = 0; b < B; ++b) {
+        p.utt[b].wav_off = (long long)b * N;
+        p.utt[B + b].wav_off = clean_off + (long long)b * N;
+    }
+    size_t fwd, mid;
+    const size_t need = loss_precise_bytes(p, B, with_grad, &fwd, &mid);
+    NB_CHECK(workspace_bytes >= need, "loss (fp32 mode): workspace too small (%zu < %zu bytes); size it with "
+             "nomad_b200_loss_workspace_bytes_mode", workspace_bytes, need);
+    char* base = (char*)workspace_dev;
+    PWorkspace ws;
+    carve_precise(p, base, &ws, true);
+    LossBufs L;
+    carve_loss(p, B, 0, 0, 0, false, base + fwd, &L);
+    const long long Fe = p.frames / 2;
+    const int T = p.max_T;
+    NB_CUDA(cudaMemsetAsync(L.acc, 0, sizeof(double) * 16, st));
+    NB_TRY(embed_precise_save(h, p, base, fwd, est_dev, st, nullptr, 0));
+    NB_TRY(launch_pool_head(st, ws.x, ws.meta, p.B, w.loss_head_wt, w.loss_head_b, L.emb, L.pooled));
+    const unsigned row_blocks = (unsigned)((Fe + 7) / 8);
+    for (int l = 0; l < LAYERS; ++l) {
+        l1_layer_kernel<<<row_blocks, 256, 0, st>>>(ws.pre2[l], ws.meta, B, Fe, w.layer[l].ln2_g, L.acc + l);
+        NB_LAUNCHED();
+    }
+    const double numel = (double)B * T * EMBED;
+    const float S = with_grad ? (float)std::exp2(std::ceil(std::log2(numel))) : 0.f;
+    head_bwd_kernel<<<B, 256, 0, st>>>(L.pooled, ws.meta, B, w.loss_head_wt, w.loss_head_w, w.loss_head_b,
+                                       (float)(S / ((double)B * EMB)), L.acc + LAYERS, L.g_pool);
+    NB_LAUNCHED();
+    loss_finalize_kernel<<<1, 1, 0, st>>>(L.acc, 1.0 / numel, 1.0 / ((double)B * EMB), loss_dev);
+    NB_LAUNCHED();
+    if (!with_grad) return 0;
+    PBwdArgs a;
+    memset(&a, 0, sizeof(a));
+    a.B_bwd = B;
+    a.top = LAYERS - 1;
+    a.g_pool = L.g_pool;
+    a.seed_layer = (float)(S / numel);
+    a.out_scale = 1.0f / S;
+    a.feature_grad_mult = feature_grad_mult;
+    return backward_precise(h, p, base, a, est_dev, N, d_est_dev, base + fwd + mid, workspace_bytes - fwd - mid, st);
+}
+
 extern "C" {
 
 // The step is ~250 small launches for B = 32 x 2 s (profiles/r02_loss_trace_before.log: 8 % of the step was launch gaps):
@@ -1642,6 +1709,8 @@ int nomad_b200_loss_fwd_bwd(nomad_b200_handle* hh, const float* est_dev, const f
     NB_CHECK(((uintptr_t)workspace_dev & 1023) == 0, "loss: workspace must be 1024-byte aligned");
     NB_CUDA(cudaSetDevice(h->device));
     cudaStream_t st = (cudaStream_t)stream;
+    if (h->precision == NOMAD_B200_PRECISION_FP32)
+        return loss_run_precise(h, est_dev, clean_dev, B, N, feature_grad_mult, loss_dev, d_est_dev, workspace_dev, workspace_bytes, st);
     const int with_grad = d_est_dev != nullptr ? 1 : 0;
     static const int use_graph = getenv("NOMAD_B200_LOSS_GRAPH") ? atoi(getenv("NOMAD_B200_LOSS_GRAPH")) : 1;
     const size_t core = (loss_core_bytes(B, N, with_grad) + 1023) / 1024 * 1024;
@@ -1660,14 +1729,16 @@ int nomad_b200_loss_fwd_bwd(nomad_b200_handle* hh, const float* est_dev, const f
     NB_CUDA(cudaMemcpyAsync(s_clean, clean_dev, bn * 4, cudaMemcpyDeviceToDevice, st));
     LossGraphEntry* ent = nullptr;
     for (auto& e : h->loss_graphs)
-        if (e.B == B && e.N == N && e.with_grad == with_grad && e.fgm == feature_grad_mult && e.ws == workspace_dev) ent = &e;
+        if (e.mode == h->precision && e.B == B && e.N == N && e.with_grad == with_grad && e.fgm == feature_grad_mult &&
+            e.ws == workspace_dev)
+            ent = &e;
     if (ent == nullptr) {  // first call with this shape: eager (also performs the one-off per-kernel attribute set-up)
         if (h->loss_graphs.size() >= 8) {
             for (auto& e : h->loss_graphs)
                 if (e.exec) cudaGraphExecDestroy(e.exec);
             h->loss_graphs.clear();
         }
-        h->loss_graphs.push_back(LossGraphEntry{B, (long long)N, with_grad, feature_grad_mult, workspace_dev, nullptr, 0, false});
+        h->loss_graphs.push_back(LossGraphEntry{h->precision, B, (long long)N, with_grad, feature_grad_mult, workspace_dev, nullptr, 0, false});
         NB_TRY(loss_run(hh, s_est, s_clean, B, N, feature_grad_mult, s_loss, with_grad ? s_grad : nullptr, workspace_dev, core, st, 0));
     } else if (ent->exec == nullptr && !ent->failed) {  // second call: capture on the handle's own stream, then launch
         if (!h->graph_stream) NB_CUDA(cudaStreamCreateWithFlags(&h->graph_stream, cudaStreamNonBlocking));
@@ -1911,6 +1982,7 @@ struct SavedRecord {
     uint32_t magic;
     int32_t flags, head, B;
     int64_t N;
+    int32_t mode;  // precision_mode of the forward: 1 = the fp32-class layout of precise.cu (flags 0 only)
 };
 static constexpr uint32_t SAVED_MAGIC = 0x4e425356u;
 static constexpr size_t SAVED_RECORD_BYTES = 1024;
@@ -1925,10 +1997,15 @@ static int layers_plan(int B, int64_t N, Plan* p) {
     return make_plan(off.data(), B, p);
 }
 
-static size_t carve_saved(const Plan& p, int flags, void* base, Workspace* ws, SavedTail* tail) {
-    size_t o = SAVED_RECORD_BYTES + carve_workspace(p, base ? (char*)base + SAVED_RECORD_BYTES : nullptr, ws, true,
-                                                    (flags & NOMAD_B200_SAVE_PARAMS) != 0);
-    if (ws) ws->aux0_raw = (flags & NOMAD_B200_SAVE_CONV) != 0;
+// mode 1: [record | fp32-class save-mode forward (carve_precise) | tail]; `ws` is then not filled
+static size_t carve_saved(const Plan& p, int flags, void* base, Workspace* ws, SavedTail* tail, int mode = 0) {
+    size_t o = SAVED_RECORD_BYTES;
+    if (mode == NOMAD_B200_PRECISION_FP32) {
+        o += carve_precise(p, nullptr, nullptr, true);
+    } else {
+        o += carve_workspace(p, base ? (char*)base + SAVED_RECORD_BYTES : nullptr, ws, true, (flags & NOMAD_B200_SAVE_PARAMS) != 0);
+        if (ws) ws->aux0_raw = (flags & NOMAD_B200_SAVE_CONV) != 0;
+    }
     auto take = [&](size_t bytes) {
         size_t at = o;
         o = (o + bytes + 1023) / 1024 * 1024;
@@ -1972,6 +2049,19 @@ static size_t carve_params_bwd(const Plan& p, int flags, void* base, LossBufs* L
     return lb + extra + conv;
 }
 
+// fp32-class backward scratch: [backward_precise scratch | g_pool B x 768 | gy B x 256 | scale state]
+static size_t carve_layers_bwd_precise(const Plan& p, void* base, float** g_pool, float** gy, unsigned** state, size_t* bwd) {
+    auto al = [](size_t v) { return (v + 1023) / 1024 * 1024; };
+    const size_t b = precise_bwd_bytes(p, p.B), gp = al(4ull * EMBED * p.B), gyb = al(4ull * EMB * p.B);
+    if (base) {
+        *bwd = b;
+        *g_pool = (float*)((char*)base + b);
+        *gy = (float*)((char*)base + b + gp);
+        *state = (unsigned*)((char*)base + b + gp + gyb);
+    }
+    return b + gp + gyb + 1024;
+}
+
 extern "C" {
 
 size_t nomad_b200_layers_saved_bytes(int B, int64_t N) { return nomad_b200_layers_saved_bytes_ex(B, N, 0); }
@@ -1986,6 +2076,19 @@ size_t nomad_b200_layers_bwd_workspace_bytes(int B, int64_t N) {
     Plan p;
     if (layers_plan(B, N, &p)) return 0;
     return carve_layers_bwd(p, nullptr, nullptr, nullptr, nullptr);
+}
+
+size_t nomad_b200_layers_saved_bytes_mode(int B, int64_t N, int precision_mode) {
+    Plan p;
+    if (layers_plan(B, N, &p)) return 0;
+    return carve_saved(p, 0, nullptr, nullptr, nullptr, precision_mode == NOMAD_B200_PRECISION_FP32 ? 1 : 0);
+}
+
+size_t nomad_b200_layers_bwd_workspace_bytes_mode(int B, int64_t N, int precision_mode) {
+    Plan p;
+    if (layers_plan(B, N, &p)) return 0;
+    if (precision_mode != NOMAD_B200_PRECISION_FP32) return carve_layers_bwd(p, nullptr, nullptr, nullptr, nullptr);
+    return carve_layers_bwd_precise(p, nullptr, nullptr, nullptr, nullptr, nullptr);
 }
 
 size_t nomad_b200_layers_bwd_params_workspace_bytes(int B, int64_t N, int flags) {
@@ -2012,17 +2115,27 @@ int nomad_b200_layers_fwd_save_ex(nomad_b200_handle* hh, const float* wav_dev, i
     NB_CUDA(cudaSetDevice(h->device));
     Plan p;
     NB_TRY(layers_plan(B, N, &p));
+    // parameter gradients (flags != 0) keep the fp16-operand arithmetic in either mode
+    const int mode = flags == 0 && h->precision == NOMAD_B200_PRECISION_FP32 ? NOMAD_B200_PRECISION_FP32 : NOMAD_B200_PRECISION_FP16;
     Workspace ws;
     SavedTail t;
-    const size_t need = carve_saved(p, flags, saved_dev, &ws, &t);
-    NB_CHECK(saved_bytes >= need, "layers_fwd_save: saved buffer too small (%zu < %zu bytes)", saved_bytes, need);
+    const size_t need = carve_saved(p, flags, saved_dev, &ws, &t, mode);
+    NB_CHECK(saved_bytes >= need, "layers_fwd_save: saved buffer too small (%zu < %zu bytes)%s", saved_bytes, need,
+             mode ? "; the handle is in fp32 mode: size it with nomad_b200_layers_saved_bytes_mode" : "");
     cudaStream_t st = (cudaStream_t)stream;
     const Weights& w = h->w;
     // pageable source: staged by the call itself, nothing to keep alive
-    const SavedRecord rec{SAVED_MAGIC, flags, head, B, (int64_t)N};
+    const SavedRecord rec{SAVED_MAGIC, flags, head, B, (int64_t)N, mode};
     NB_CUDA(cudaMemcpyAsync(saved_dev, &rec, sizeof(rec), cudaMemcpyHostToDevice, st));
     NB_CUDA(cudaMemcpyAsync(t.head_wt, head ? w.loss_head_wt : w.head_wt, 4ull * EMBED * EMB, cudaMemcpyDeviceToDevice, st));
     NB_CUDA(cudaMemcpyAsync(t.head_b, head ? w.loss_head_b : w.head_b, 4ull * EMB, cudaMemcpyDeviceToDevice, st));
+    if (mode == NOMAD_B200_PRECISION_FP32) {
+        char* fwd = (char*)saved_dev + SAVED_RECORD_BYTES;
+        NB_TRY(embed_precise_save(h, p, fwd, carve_precise(p, nullptr, nullptr, true), wav_dev, st, layers_dev, p.max_T));
+        PWorkspace pws;
+        carve_precise(p, fwd, &pws, true);
+        return launch_pool_head(st, pws.x, pws.meta, p.B, t.head_wt, t.head_b, emb_dev ? emb_dev : t.emb, t.pooled);
+    }
     NB_TRY(upload_meta(h, p, ws, st));
     NB_TRY(forward_encoder(h, p, ws, wav_dev, st, layers_dev, p.max_T));
     NB_TRY(launch_pool_head(st, ws.x, ws.meta, p.B, t.head_wt, t.head_b, emb_dev ? emb_dev : t.emb, t.pooled));
@@ -2109,6 +2222,59 @@ static int layers_backward(Handle* h, const Plan& p, int flags, int head, const 
                           d_wav_dev, st, params ? &tc : nullptr, &ug);
 }
 
+// The same for a buffer saved in fp32 mode: head and gradient scale as above, then backward_precise.
+static int layers_backward_precise(Handle* h, const Plan& p, const void* saved_dev, const float* wav_dev, int64_t N,
+                                   const float* const* g_layers, const float* g_emb, float feature_grad_mult, float* d_wav_dev,
+                                   void* workspace_dev, size_t workspace_bytes, cudaStream_t st) {
+    const int B = p.B;
+    SavedTail t;
+    carve_saved(p, 0, (void*)saved_dev, nullptr, &t, NOMAD_B200_PRECISION_FP32);
+    void* fwd = (char*)saved_dev + SAVED_RECORD_BYTES;
+    PWorkspace ws;
+    carve_precise(p, fwd, &ws, true);
+    float *g_pool = nullptr, *gy = nullptr;
+    unsigned* state = nullptr;
+    size_t bwd = 0;
+    const size_t need = carve_layers_bwd_precise(p, workspace_dev, &g_pool, &gy, &state, &bwd);
+    NB_CHECK(workspace_bytes >= need, "layers_bwd (fp32 mode): workspace too small (%zu < %zu bytes); size it with "
+             "nomad_b200_layers_bwd_workspace_bytes_mode", workspace_bytes, need);
+    PBwdArgs a;
+    memset(&a, 0, sizeof(a));
+    a.B_bwd = B;
+    a.top = -1;
+    a.user_T = p.max_T;
+    a.feature_grad_mult = feature_grad_mult;
+    ScaleSources src;
+    memset(&src, 0, sizeof(src));
+    for (int l = 0; l < LAYERS; ++l) {
+        a.g_layers[l] = g_layers != nullptr ? g_layers[l] : nullptr;
+        src.p[l] = a.g_layers[l];
+        src.n[l] = (long long)B * p.max_T * EMBED;
+        if (a.g_layers[l] != nullptr) a.top = l;
+    }
+    if (a.top < 0 && g_emb == nullptr) {  // no output is used: the gradient is zero
+        NB_CUDA(cudaMemsetAsync(d_wav_dev, 0, 4ull * B * N, st));
+        return 0;
+    }
+    if (g_emb != nullptr) {
+        head_emb_bwd_kernel<<<B, 256, 0, st>>>(t.pooled, t.head_wt, t.head_b, g_emb, gy);
+        NB_LAUNCHED();
+        head_pool_grad_kernel<<<B, 256, 0, st>>>(gy, t.pooled, ws.meta, t.head_wt, g_pool);
+        NB_LAUNCHED();
+        a.g_pool = g_pool;
+        a.top = LAYERS - 1;
+        src.p[LAYERS] = g_pool;
+        src.n[LAYERS] = (long long)B * EMBED;
+    }
+    float* scale = (float*)(state + 2);
+    NB_CUDA(cudaMemsetAsync(state, 0, 2 * sizeof(unsigned), st));
+    grad_scale_kernel<<<2 * 148, 256, 0, st>>>(src, state, scale);
+    NB_LAUNCHED();
+    a.scale_dev = scale;
+    a.out_scale = 1.f;
+    return backward_precise(h, p, fwd, a, wav_dev, N, d_wav_dev, workspace_dev, bwd, st);
+}
+
 extern "C" {
 
 int nomad_b200_layers_bwd(nomad_b200_handle* hh, const void* saved_dev, size_t saved_bytes, const float* wav_dev, int B,
@@ -2126,11 +2292,28 @@ int nomad_b200_layers_bwd(nomad_b200_handle* hh, const void* saved_dev, size_t s
     NB_CUDA(cudaSetDevice(h->device));
     Plan p;
     NB_TRY(layers_plan(B, N, &p));
-    const size_t need_saved = carve_saved(p, 0, nullptr, nullptr, nullptr);
+    cudaStream_t st = (cudaStream_t)stream;
+    int mode = NOMAD_B200_PRECISION_FP16;
+    if (h->pw.built) {  // the handle can save either layout: read the record back (one stream synchronisation)
+        NB_CHECK(saved_bytes >= SAVED_RECORD_BYTES, "layers_bwd: saved buffer too small");
+        SavedRecord rec;
+        NB_CUDA(cudaMemcpyAsync(&rec, saved_dev, sizeof(rec), cudaMemcpyDeviceToHost, st));
+        NB_CUDA(cudaStreamSynchronize(st));
+        NB_CHECK(rec.magic == SAVED_MAGIC && rec.B == B && rec.N == (int64_t)N,
+                 "layers_bwd: the saved buffer is not from a nomad_b200_layers_fwd_save of this B x N");
+        NB_CHECK(rec.mode == h->precision,
+                 "layers_bwd: the saved buffer was written in precision_mode %d but the handle is now in mode %d; switch "
+                 "back with nomad_b200_set_precision before the backward, or run the forward again", rec.mode, h->precision);
+        mode = rec.mode;
+    }
+    const size_t need_saved = carve_saved(p, 0, nullptr, nullptr, nullptr, mode);
     NB_CHECK(saved_bytes >= need_saved, "layers_bwd: saved buffer too small (%zu < %zu bytes): not from a forward of this B x N?",
              saved_bytes, need_saved);
+    if (mode == NOMAD_B200_PRECISION_FP32)
+        return layers_backward_precise(h, p, saved_dev, wav_dev, N, g_layers, g_emb, feature_grad_mult, d_wav_dev, workspace_dev,
+                                       workspace_bytes, st);
     return layers_backward(h, p, 0, 0, saved_dev, wav_dev, N, g_layers, g_emb, feature_grad_mult, d_wav_dev, nullptr, nullptr,
-                           nullptr, workspace_dev, workspace_bytes, (cudaStream_t)stream);
+                           nullptr, workspace_dev, workspace_bytes, st);
 }
 
 int nomad_b200_layers_bwd_params(nomad_b200_handle* hh, const void* saved_dev, size_t saved_bytes, const float* wav_dev, int B,
@@ -2160,6 +2343,9 @@ int nomad_b200_layers_bwd_params(nomad_b200_handle* hh, const void* saved_dev, s
     NB_CUDA(cudaStreamSynchronize(st));
     NB_CHECK(rec.magic == SAVED_MAGIC && rec.B == B && rec.N == (int64_t)N,
              "layers_bwd_params: the saved buffer is not from a nomad_b200_layers_fwd_save(_ex) of this B x N");
+    NB_CHECK(rec.mode == NOMAD_B200_PRECISION_FP16,
+             "layers_bwd_params: the buffer holds an fp32-class forward (parameter gradients run the fp16-operand path: save "
+             "with NOMAD_B200_SAVE_PARAMS, or use nomad_b200_layers_bwd for the waveform gradient)");
     NB_CHECK(grads_dev == nullptr || (rec.flags & NOMAD_B200_SAVE_PARAMS),
              "layers_bwd_params: parameter gradients need a forward saved with NOMAD_B200_SAVE_PARAMS");
     NB_CHECK(conv_grads_dev == nullptr || (rec.flags & NOMAD_B200_SAVE_CONV),

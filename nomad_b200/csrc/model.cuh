@@ -87,6 +87,11 @@ struct PreciseWeights {
     SplitW conv[7]{};   // l = 1..6, same layout as Weights::conv_w
     SplitW proj{}, pos{};
     SplitW qkv[LAYERS]{}, o[LAYERS]{}, fc1[LAYERS]{}, fc2[LAYERS]{};
+    // transposed planes for the dgrad GEMMs of the fp32-class waveform backward (precise_bwd.cu), in the layouts of
+    // Weights::conv_wt / conv_wte / proj_wt / pos_wt / wt_*: the same hi / lo values, the same inv_scale
+    SplitW conv_t[7]{}, conv_te[7]{};
+    SplitW proj_t{}, pos_t{};
+    SplitW qkv_t[LAYERS]{}, o_t[LAYERS]{}, fc1_t[LAYERS]{}, fc2_t[LAYERS]{};
 };
 
 struct Plan {
@@ -144,6 +149,7 @@ struct Workspace {
 
 // one captured loss step (loss.cu): replayed while shape, gradient request and workspace stay the same
 struct LossGraphEntry {
+    int mode;  // precision_mode the step was recorded in
     int B;
     long long N;
     int with_grad;

@@ -13,42 +13,19 @@
 #include <cmath>
 #include <cstring>
 
-#include "kernels.cuh"
+#include "precise.cuh"
 
 namespace nb {
 
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
-// ------------------------------------------------------------------------------------------------ small helpers
-// 8 fp32 values -> 8 hi + 8 lo halves (16 bytes each)
-__device__ __forceinline__ void split_store8(const float* v, op_t* hi, op_t* lo) {
-    uint32_t h[4], l[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        h[i] = pack_op(v[2 * i], v[2 * i + 1]);
-        const float2 f = unpack_op(h[i]);
-        l[i] = pack_op(v[2 * i] - f.x, v[2 * i + 1] - f.y);
-    }
-    *reinterpret_cast<uint4*>(hi) = make_uint4(h[0], h[1], h[2], h[3]);
-    *reinterpret_cast<uint4*>(lo) = make_uint4(l[0], l[1], l[2], l[3]);
-}
-__device__ __forceinline__ void split_load8(const op_t* hi, const op_t* lo, float* v) {
-    const uint4 h = __ldg(reinterpret_cast<const uint4*>(hi)), l = __ldg(reinterpret_cast<const uint4*>(lo));
-    const uint32_t hh[4] = {h.x, h.y, h.z, h.w}, ll[4] = {l.x, l.y, l.z, l.w};
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        const float2 a = unpack_op(hh[i]), b = unpack_op(ll[i]);
-        v[2 * i] = a.x + b.x;
-        v[2 * i + 1] = a.y + b.y;
-    }
-}
-
 // ------------------------------------------------------------------------------------------------ conv0
 // out[row][c] = GELU(sum_j fold[c][j] x[5 t + j] + shift[c]) with the GroupNorm folded into the taps (frontend.cu),
-// fp32 FMAs, libdevice erff, stored as hi + lo planes; zeros for the padding rows t >= T0.
+// fp32 FMAs, libdevice erff, stored as hi + lo planes; zeros for the padding rows t >= T0.  pre_out (save mode, may be
+// null): the GELU input, fp32.
 __global__ void __launch_bounds__(256) conv0_precise_kernel(const float* __restrict__ wav, const UttMeta* __restrict__ meta,
                                                             int B, const float* __restrict__ fold, op_t* __restrict__ out_hi,
-                                                            op_t* __restrict__ out_lo) {
+                                                            op_t* __restrict__ out_lo, float* __restrict__ pre_out) {
     const int blk = blockIdx.x;
     const int row_base = blk * 64;
     const int b = find_utt_by_frame(meta, B, blk);
@@ -81,6 +58,8 @@ __global__ void __launch_bounds__(256) conv0_precise_kernel(const float* __restr
                 y0 = fmaf(w0[j], xv, y0);
                 y1 = fmaf(w1[j], xv, y1);
             }
+            if (pre_out != nullptr)
+                *reinterpret_cast<float2*>(pre_out + (long long)(row_base + t) * CONV_DIM + c) = make_float2(y0, y1);
             y0 = gelu_erf_exact(y0);
             y1 = gelu_erf_exact(y1);
             ph = pack_op(y0, y1);
@@ -89,7 +68,30 @@ __global__ void __launch_bounds__(256) conv0_precise_kernel(const float* __restr
         }
         oh[(long long)t * (CONV_DIM / 2)] = ph;
         ol[(long long)t * (CONV_DIM / 2)] = pl;
+        if (pre_out != nullptr && t >= valid)
+            *reinterpret_cast<float2*>(pre_out + (long long)(row_base + t) * CONV_DIM + c) = make_float2(0.f, 0.f);
     }
+}
+
+// save mode: GELU of the fp32 pre-activations `in` (n values, n % 8 == 0) to hi + lo planes and / or fp32 `out`
+__global__ void __launch_bounds__(256) gelu_precise_kernel(const float* __restrict__ in, long long n, op_t* __restrict__ hi,
+                                                           op_t* __restrict__ lo, float* __restrict__ out) {
+    const long long i = ((long long)blockIdx.x * blockDim.x + threadIdx.x) * 8;
+    if (i >= n) return;
+    const float4 a = __ldg(reinterpret_cast<const float4*>(in + i)), b = __ldg(reinterpret_cast<const float4*>(in + i + 4));
+    float v[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+#pragma unroll
+    for (int j = 0; j < 8; ++j) v[j] = gelu_erf_exact(v[j]);
+    if (hi != nullptr) split_store8(v, hi + i, lo + i);
+    if (out != nullptr) {
+        *reinterpret_cast<float4*>(out + i) = make_float4(v[0], v[1], v[2], v[3]);
+        *reinterpret_cast<float4*>(out + i + 4) = make_float4(v[4], v[5], v[6], v[7]);
+    }
+}
+static int launch_gelu_precise(cudaStream_t st, const float* in, long long n, op_t* hi, op_t* lo, float* out) {
+    gelu_precise_kernel<<<(unsigned)((n / 8 + 255) / 256), 256, 0, st>>>(in, n, hi, lo, out);
+    NB_LAUNCHED();
+    return 0;
 }
 
 // ------------------------------------------------------------------------------------------------ LayerNorm(512)
@@ -247,12 +249,14 @@ __global__ void __launch_bounds__(256) ln768_precise_kernel(const float* __restr
 // softmax(Q K^T) V per (utterance, head) on the fp32 cores: one CTA = 64 queries x one head, streaming 64-key tiles with
 // an online softmax.  Thread (ty, tx) of the 16 x 16 layout owns queries 4 ty .. 4 ty + 3 and, in the two products,
 // keys / output columns 4 tx .. 4 tx + 3 (4 x 4 register tiles fed by float4 shared loads).  q is already scaled by
-// head_dim^-0.5 (folded into the QKV weights).  Output goes out as hi + lo planes (the out-projection's A operand).
+// head_dim^-0.5 (folded into the QKV weights).  Output goes out as hi + lo planes (the out-projection's A operand);
+// lse (save mode, may be null): frames x 12 log-sum-exp of the softmax rows.
 static constexpr int PA_T = 64, PA_P = 68;  // tile edge, shared-memory row pitch (floats)
 static constexpr int PA_SMEM = 4 * PA_T * PA_P * 4;
 
 __global__ void __launch_bounds__(256) attention_precise_kernel(const float* __restrict__ qkv, const UttMeta* __restrict__ meta,
-                                                                op_t* __restrict__ out_hi, op_t* __restrict__ out_lo) {
+                                                                op_t* __restrict__ out_hi, op_t* __restrict__ out_lo,
+                                                                float* __restrict__ lse) {
     const int b = blockIdx.z, h = blockIdx.y, q0 = blockIdx.x * PA_T;
     const int T = meta[b].T;
     if (q0 >= T) return;
@@ -363,27 +367,12 @@ __global__ void __launch_bounds__(256) attention_precise_kernel(const float* __r
         const long long off = (f0 + q) * EMBED + h * HEAD_DIM + 4 * tx;
         *reinterpret_cast<uint2*>(out_hi + off) = make_uint2(h0, h1);
         *reinterpret_cast<uint2*>(out_lo + off) = make_uint2(pack_op(r0 - f0v.x, r1 - f0v.y), pack_op(r2 - f1v.x, r3 - f1v.y));
+        if (lse != nullptr && tx == 0) lse[(f0 + q) * HEADS + h] = m_run[i] + logf(l_run[i]);
     }
 }
 
 // ------------------------------------------------------------------------------------------------ workspace
-struct PWorkspace {
-    UttMeta* meta;
-    double* stat_part;
-    float* c0_fold;
-    op_t *y_hi[2], *y_lo[2];    // conv levels ping-pong: even levels in [0], odd levels in [1]
-    op_t *ln0_hi, *ln0_lo;      // alias y[1] (level 6 lives in y[0])
-    float *x0, *x, *pre;
-    op_t *xh_hi, *xh_lo;
-    op_t *posg_hi, *posg_lo;
-    float* pos_y;
-    float* qkv;
-    op_t *attn_hi, *attn_lo;
-    op_t *ffn_hi, *ffn_lo;
-    size_t bytes;
-};
-
-static size_t carve_precise(const Plan& p, void* base, PWorkspace* out) {
+size_t carve_precise(const Plan& p, void* base, PWorkspace* out, bool save) {
     size_t o = 0;
     auto take = [&](size_t bytes) {
         size_t at = o;
@@ -405,23 +394,45 @@ static size_t carve_precise(const Plan& p, void* base, PWorkspace* out) {
     w.ln0_lo = w.y_lo[1];
     w.x0 = (float*)take(4ull * EMBED * F);
     w.x = (float*)take(4ull * EMBED * F);
-    w.pre = (float*)take(4ull * EMBED * F);
+    float* pre = (float*)take(4ull * EMBED * F);
     w.xh_hi = (op_t*)take(2ull * EMBED * F);
     w.xh_lo = (op_t*)take(2ull * EMBED * F);
     w.posg_hi = (op_t*)take(2ull * POS_G * POS_GC * (p.pos_rows + POS_K));
     w.posg_lo = (op_t*)take(2ull * POS_G * POS_GC * (p.pos_rows + POS_K));
     w.pos_y = (float*)take(4ull * EMBED * p.pos_rows);
-    w.qkv = (float*)take(4ull * 3 * EMBED * F);
-    w.attn_hi = (op_t*)take(2ull * EMBED * F);
-    w.attn_lo = (op_t*)take(2ull * EMBED * F);
+    float* qkv = (float*)take(4ull * 3 * EMBED * F);
+    op_t* attn_hi = (op_t*)take(2ull * EMBED * F);
+    op_t* attn_lo = (op_t*)take(2ull * EMBED * F);
     w.ffn_hi = (op_t*)take(2ull * FFN * F);
     w.ffn_lo = (op_t*)take(2ull * FFN * F);
+    for (int l = 0; l < LAYERS; ++l) {
+        w.qkv[l] = qkv;
+        w.attn_hi[l] = attn_hi;
+        w.attn_lo[l] = attn_lo;
+        w.pre1[l] = w.pre2[l] = pre;
+    }
+    if (save) {
+        w.gn_stat = (float*)take(4ull * 2 * CONV_DIM * p.B);
+        for (int l = 0; l < 7; ++l) w.u[l] = (float*)take(4ull * CONV_DIM * (size_t)(p.rows0 >> l));
+        w.pos_pre = (float*)take(4ull * EMBED * p.pos_rows);
+        for (int l = 0; l < LAYERS; ++l) {
+            if (l > 0) {
+                w.qkv[l] = (float*)take(4ull * 3 * EMBED * F);
+                w.attn_hi[l] = (op_t*)take(2ull * EMBED * F);
+                w.attn_lo[l] = (op_t*)take(2ull * EMBED * F);
+                w.pre1[l] = (float*)take(4ull * EMBED * F);
+            }
+            w.pre2[l] = (float*)take(4ull * EMBED * F);
+            w.lse[l] = (float*)take(4ull * HEADS * F);
+            w.fc1_pre[l] = (float*)take(4ull * FFN * F);
+        }
+    }
     w.bytes = o;
     if (out) *out = w;
     return o;
 }
 
-size_t precise_workspace_bytes(const Plan& p) { return carve_precise(p, nullptr, nullptr); }
+size_t precise_workspace_bytes(const Plan& p) { return carve_precise(p, nullptr, nullptr, false); }
 
 // ------------------------------------------------------------------------------------------------ forward
 static GemmEpilogue epi_precise(int flags, const SplitW& w, const float* bias, const float* resid, float* out_f, op_t* out_h,
@@ -432,14 +443,10 @@ static GemmEpilogue epi_precise(int flags, const SplitW& w, const float* bias, c
     return e;
 }
 
-// wav (device, packed) -> embeddings, every utterance exactly as if alone (same masking rules as the fp16 path)
-int embed_precise(Handle* h, const Plan& p, void* workspace, size_t workspace_bytes, const float* wav, cudaStream_t st,
-                  float* layers_out, int layer_T, const float* head_wt, const float* head_b, float* emb_dev) {
-    NB_CHECK(h->pw.built, "this handle was created without the fp32-class weights (precision_mode 1)");
-    NB_CHECK(p.B <= 65535, "embed (fp32 mode): at most 65535 utterances per call (got %d); split the batch", p.B);
-    PWorkspace ws;
-    const size_t need = carve_precise(p, workspace, &ws);
-    NB_CHECK(workspace_bytes >= need, "embed (fp32 mode): workspace too small (%zu < %zu bytes)", workspace_bytes, need);
+// wav (device, packed) -> residual stream after the 12th layer (ws.x), every utterance exactly as if alone (same masking
+// rules as the fp16 path).  save: also keep what the waveform backward reads (PWorkspace); the arithmetic is the same.
+static int forward_precise(Handle* h, const Plan& p, const PWorkspace& ws, const float* wav, cudaStream_t st, float* layers_out,
+                           int layer_T, bool save) {
     const Weights& w = h->w;
     const PreciseWeights& pw = h->pw;
     const long long F = p.frames;
@@ -460,16 +467,22 @@ int embed_precise(Handle* h, const Plan& p, void* workspace, size_t workspace_by
         }
     }
     NB_TRY(launch_wave_stats(st, wav, ws.meta, 0, p.B, p.max_chunks, ws.stat_part));
-    NB_TRY(launch_gn_fold(st, ws.stat_part, ws.meta, 0, p.B, p.max_chunks, w.conv0_w, w.gn_g, w.gn_b, ws.c0_fold, nullptr, nullptr));
-    conv0_precise_kernel<<<(unsigned)(p.rows0 / 64), 256, 0, st>>>(wav, ws.meta, p.B, ws.c0_fold, ws.y_hi[0], ws.y_lo[0]);
+    NB_TRY(launch_gn_fold(st, ws.stat_part, ws.meta, 0, p.B, p.max_chunks, w.conv0_w, w.gn_g, w.gn_b, ws.c0_fold, ws.gn_stat, nullptr));
+    conv0_precise_kernel<<<(unsigned)(p.rows0 / 64), 256, 0, st>>>(wav, ws.meta, p.B, ws.c0_fold, ws.y_hi[0], ws.y_lo[0], ws.u[0]);
     NB_LAUNCHED();
     for (int l = 1; l < 7; ++l) {
         const long long M = p.rows0 >> l;
         const int in = (l - 1) & 1, ot = l & 1;
         GemmOperand A{ws.y_hi[in], M, 2 * CONV_DIM, 0, 0, ws.y_lo[in]};
         GemmOperand Bw{pw.conv[l].hi, CONV_DIM, (long long)CONV_KERNEL[l] * CONV_DIM, 0, 0, pw.conv[l].lo};
-        GemmEpilogue e = epi_precise(EPI_GELU | EPI_OUT_H16, pw.conv[l], nullptr, nullptr, nullptr, ws.y_hi[ot], ws.y_lo[ot], CONV_DIM);
-        NB_TRY(gemm_h16(st, A, Bw, (int)M, CONV_DIM, CONV_KERNEL[l] * CONV_DIM, 1, e, 0));
+        if (save) {  // pre-activation kept for the backward, GELU applied by a separate pass (same bits as the epilogue's)
+            GemmEpilogue e = epi_precise(EPI_OUT_F32, pw.conv[l], nullptr, nullptr, ws.u[l], nullptr, nullptr, CONV_DIM);
+            NB_TRY(gemm_h16(st, A, Bw, (int)M, CONV_DIM, CONV_KERNEL[l] * CONV_DIM, 1, e, 0));
+            NB_TRY(launch_gelu_precise(st, ws.u[l], M * CONV_DIM, ws.y_hi[ot], ws.y_lo[ot], nullptr));
+        } else {
+            GemmEpilogue e = epi_precise(EPI_GELU | EPI_OUT_H16, pw.conv[l], nullptr, nullptr, nullptr, ws.y_hi[ot], ws.y_lo[ot], CONV_DIM);
+            NB_TRY(gemm_h16(st, A, Bw, (int)M, CONV_DIM, CONV_KERNEL[l] * CONV_DIM, 1, e, 0));
+        }
     }
     ln512_precise_kernel<<<(unsigned)((F + 7) / 8), 256, 0, st>>>(ws.y_hi[0], ws.y_lo[0], F, w.ln0_g, w.ln0_b, ws.ln0_hi, ws.ln0_lo);
     NB_LAUNCHED();
@@ -487,16 +500,20 @@ int embed_precise(Handle* h, const Plan& p, void* workspace, size_t workspace_by
         NB_LAUNCHED();
         GemmOperand A{ws.posg_hi, p.pos_rows, POS_GC, rows_alloc * POS_GC, 0, ws.posg_lo};
         GemmOperand Bw{pw.pos.hi, POS_GC, (long long)POS_K * POS_GC, (long long)POS_GC * POS_K * POS_GC, 0, pw.pos.lo};
-        GemmEpilogue e = epi_precise(EPI_BIAS | EPI_GELU | EPI_OUT_F32, pw.pos, w.pos_b, nullptr, ws.pos_y, nullptr, nullptr, EMBED);
+        GemmEpilogue e = epi_precise(save ? EPI_BIAS | EPI_OUT_F32 : EPI_BIAS | EPI_GELU | EPI_OUT_F32, pw.pos, w.pos_b, nullptr,
+                                     save ? ws.pos_pre : ws.pos_y, nullptr, nullptr, EMBED);
         e.bias_bstride = POS_GC;
         e.out_bstride = POS_GC;
         NB_TRY(gemm_h16(st, A, Bw, (int)p.pos_rows, POS_GC, POS_K * POS_GC, POS_G, e, 0));
+        if (save) NB_TRY(launch_gelu_precise(st, ws.pos_pre, p.pos_rows * EMBED, nullptr, nullptr, ws.pos_y));
         pos_finish_ln_precise_kernel<<<(unsigned)((F + 7) / 8), 256, 0, st>>>(ws.x0, ws.pos_y, ws.meta, p.B, F, w.lne_g, w.lne_b,
                                                                               ws.x, ws.xh_hi, ws.xh_lo);
         NB_LAUNCHED();
     }
-    NB_CUDA(cudaMemsetAsync(ws.attn_hi, 0, 2ull * EMBED * F, st));  // padded rows stay finite
-    NB_CUDA(cudaMemsetAsync(ws.attn_lo, 0, 2ull * EMBED * F, st));
+    for (int l = 0; l < (save ? LAYERS : 1); ++l) {  // padded rows stay finite
+        NB_CUDA(cudaMemsetAsync(ws.attn_hi[l], 0, 2ull * EMBED * F, st));
+        NB_CUDA(cudaMemsetAsync(ws.attn_lo[l], 0, 2ull * EMBED * F, st));
+    }
     static bool attr_set[64] = {false};
     if (bool* flag = device_once_flag(attr_set)) {
         NB_CUDA(cudaFuncSetAttribute(attention_precise_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PA_SMEM));
@@ -507,42 +524,69 @@ int embed_precise(Handle* h, const Plan& p, void* workspace, size_t workspace_by
         {
             GemmOperand A{ws.xh_hi, F, EMBED, 0, 0, ws.xh_lo};
             GemmOperand Bw{pw.qkv[l].hi, 3 * EMBED, EMBED, 0, 0, pw.qkv[l].lo};
-            GemmEpilogue e = epi_precise(EPI_BIAS | EPI_OUT_F32, pw.qkv[l], L.b_qkv, nullptr, ws.qkv, nullptr, nullptr, 3 * EMBED);
+            GemmEpilogue e = epi_precise(EPI_BIAS | EPI_OUT_F32, pw.qkv[l], L.b_qkv, nullptr, ws.qkv[l], nullptr, nullptr, 3 * EMBED);
             NB_TRY(gemm_h16(st, A, Bw, (int)F, 3 * EMBED, EMBED, 1, e, 0));
         }
         {
             dim3 grid((p.max_T + PA_T - 1) / PA_T, HEADS, p.B);
-            attention_precise_kernel<<<grid, 256, PA_SMEM, st>>>(ws.qkv, ws.meta, ws.attn_hi, ws.attn_lo);
+            attention_precise_kernel<<<grid, 256, PA_SMEM, st>>>(ws.qkv[l], ws.meta, ws.attn_hi[l], ws.attn_lo[l], ws.lse[l]);
             NB_LAUNCHED();
         }
         {
-            GemmOperand A{ws.attn_hi, F, EMBED, 0, 0, ws.attn_lo};
+            GemmOperand A{ws.attn_hi[l], F, EMBED, 0, 0, ws.attn_lo[l]};
             GemmOperand Bw{pw.o[l].hi, EMBED, EMBED, 0, 0, pw.o[l].lo};
-            GemmEpilogue e = epi_precise(EPI_BIAS | EPI_RESID | EPI_OUT_F32, pw.o[l], L.b_o, ws.x, ws.pre, nullptr, nullptr, EMBED);
+            GemmEpilogue e = epi_precise(EPI_BIAS | EPI_RESID | EPI_OUT_F32, pw.o[l], L.b_o, ws.x, ws.pre1[l], nullptr, nullptr, EMBED);
             NB_TRY(gemm_h16(st, A, Bw, (int)F, EMBED, EMBED, 1, e, 0));
         }
-        ln768_precise_kernel<<<(unsigned)((F + 7) / 8), 256, 0, st>>>(ws.pre, ws.meta, p.B, F, L.ln1_g, L.ln1_b, ws.x, ws.xh_hi,
+        ln768_precise_kernel<<<(unsigned)((F + 7) / 8), 256, 0, st>>>(ws.pre1[l], ws.meta, p.B, F, L.ln1_g, L.ln1_b, ws.x, ws.xh_hi,
                                                                       ws.xh_lo, nullptr, 0);
         NB_LAUNCHED();
         {
             GemmOperand A{ws.xh_hi, F, EMBED, 0, 0, ws.xh_lo};
             GemmOperand Bw{pw.fc1[l].hi, FFN, EMBED, 0, 0, pw.fc1[l].lo};
-            GemmEpilogue e = epi_precise(EPI_BIAS | EPI_GELU | EPI_OUT_H16, pw.fc1[l], L.b_fc1, nullptr, nullptr, ws.ffn_hi, ws.ffn_lo, FFN);
-            NB_TRY(gemm_h16(st, A, Bw, (int)F, FFN, EMBED, 1, e, 0));
+            if (save) {
+                GemmEpilogue e = epi_precise(EPI_BIAS | EPI_OUT_F32, pw.fc1[l], L.b_fc1, nullptr, ws.fc1_pre[l], nullptr, nullptr, FFN);
+                NB_TRY(gemm_h16(st, A, Bw, (int)F, FFN, EMBED, 1, e, 0));
+                NB_TRY(launch_gelu_precise(st, ws.fc1_pre[l], F * FFN, ws.ffn_hi, ws.ffn_lo, nullptr));
+            } else {
+                GemmEpilogue e = epi_precise(EPI_BIAS | EPI_GELU | EPI_OUT_H16, pw.fc1[l], L.b_fc1, nullptr, nullptr, ws.ffn_hi, ws.ffn_lo, FFN);
+                NB_TRY(gemm_h16(st, A, Bw, (int)F, FFN, EMBED, 1, e, 0));
+            }
         }
         {
             GemmOperand A{ws.ffn_hi, F, FFN, 0, 0, ws.ffn_lo};
             GemmOperand Bw{pw.fc2[l].hi, EMBED, FFN, 0, 0, pw.fc2[l].lo};
-            GemmEpilogue e = epi_precise(EPI_BIAS | EPI_RESID | EPI_OUT_F32, pw.fc2[l], L.b_fc2, ws.x, ws.pre, nullptr, nullptr, EMBED);
+            GemmEpilogue e = epi_precise(EPI_BIAS | EPI_RESID | EPI_OUT_F32, pw.fc2[l], L.b_fc2, ws.x, ws.pre2[l], nullptr, nullptr, EMBED);
             NB_TRY(gemm_h16(st, A, Bw, (int)F, EMBED, FFN, 1, e, 0));
         }
         float* lo = layers_out ? layers_out + (size_t)l * p.B * layer_T * EMBED : nullptr;
-        ln768_precise_kernel<<<(unsigned)((F + 7) / 8), 256, 0, st>>>(ws.pre, ws.meta, p.B, F, L.ln2_g, L.ln2_b, ws.x, ws.xh_hi,
+        ln768_precise_kernel<<<(unsigned)((F + 7) / 8), 256, 0, st>>>(ws.pre2[l], ws.meta, p.B, F, L.ln2_g, L.ln2_b, ws.x, ws.xh_hi,
                                                                       ws.xh_lo, lo, layer_T);
         NB_LAUNCHED();
     }
+    return 0;
+}
+
+int embed_precise(Handle* h, const Plan& p, void* workspace, size_t workspace_bytes, const float* wav, cudaStream_t st,
+                  float* layers_out, int layer_T, const float* head_wt, const float* head_b, float* emb_dev) {
+    NB_CHECK(h->pw.built, "this handle was created without the fp32-class weights (precision_mode 1)");
+    NB_CHECK(p.B <= 65535, "embed (fp32 mode): at most 65535 utterances per call (got %d); split the batch", p.B);
+    PWorkspace ws;
+    const size_t need = carve_precise(p, workspace, &ws, false);
+    NB_CHECK(workspace_bytes >= need, "embed (fp32 mode): workspace too small (%zu < %zu bytes)", workspace_bytes, need);
+    NB_TRY(forward_precise(h, p, ws, wav, st, layers_out, layer_T, false));
     if (emb_dev != nullptr) NB_TRY(launch_pool_head(st, ws.x, ws.meta, p.B, head_wt, head_b, emb_dev, nullptr));
     return 0;
+}
+
+int embed_precise_save(Handle* h, const Plan& p, void* saved, size_t saved_bytes, const float* wav, cudaStream_t st,
+                       float* layers_out, int layer_T) {
+    NB_CHECK(h->pw.built, "this handle was created without the fp32-class weights (precision_mode 1)");
+    NB_CHECK(p.B <= 65535, "save-mode forward (fp32 mode): at most 65535 utterances per call (got %d)", p.B);
+    PWorkspace ws;
+    const size_t need = carve_precise(p, saved, &ws, true);
+    NB_CHECK(saved_bytes >= need, "save-mode forward (fp32 mode): buffer too small (%zu < %zu bytes)", saved_bytes, need);
+    return forward_precise(h, p, ws, wav, st, layers_out, layer_T, true);
 }
 
 }  // namespace nb

@@ -344,15 +344,16 @@ class Engine:
         return layers, emb
 
     def layers_fwd_save(self, wav: torch.Tensor, head: int, want_layers: bool = True, flags: int = 0):
-        """Save-mode forward of a (B, N) CUDA batch for autograd (``nomad_b200_layers_fwd_save``; fp16 operands whatever
-        the engine's precision).  ``head``: 0 = NOMAD head, 1 = loss head.  -> ((12, B, T, 768) | None, (B, 256), saved):
+        """Save-mode forward of a (B, N) CUDA batch for autograd (``nomad_b200_layers_fwd_save``, in the engine's precision;
+        with ``flags`` fp16 operands whatever the precision).  ``head``: 0 = NOMAD head, 1 = loss head.  -> ((12, B, T, 768) | None, (B, 256), saved):
         ``saved`` is a uint8 CUDA tensor owned by the caller that :meth:`layers_bwd` needs; keep it until then.
         ``flags`` (``_lib.SAVE_*``, ``nomad_b200_layers_fwd_save_ex``): also save for :meth:`layers_bwd_params`."""
         self.sync_weights()
         wav = wav.to(self.device, torch.float32).contiguous()
         B, N = wav.shape
         T = self.num_frames(N)
-        nbytes = self.lib.nomad_b200_layers_saved_bytes_ex(B, N, int(flags))
+        nbytes = (self.lib.nomad_b200_layers_saved_bytes_ex(B, N, int(flags)) if flags
+                  else self.lib.nomad_b200_layers_saved_bytes_mode(B, N, self._mode))
         if nbytes == 0:
             raise _lib.NomadB200Error(self.lib.nomad_b200_last_error().decode())
         saved = torch.empty(nbytes + 1024, dtype=torch.uint8, device=self.device)
@@ -372,13 +373,14 @@ class Engine:
     def layers_bwd(self, saved: torch.Tensor, wav: torch.Tensor, g_layers: Sequence[Optional[torch.Tensor]],
                    g_emb: Optional[torch.Tensor], feature_grad_mult: float) -> torch.Tensor:
         """d(<g_layers, layers> + <g_emb, emb>) / d wav for the forward that filled ``saved`` (``nomad_b200_layers_bwd``):
-        ``g_layers``: 12 entries of (B, T, 768) or None, ``g_emb``: (B, 256) or None.  -> (B, N) fp32 CUDA tensor."""
+        ``g_layers``: 12 entries of (B, T, 768) or None, ``g_emb``: (B, 256) or None.  -> (B, N) fp32 CUDA tensor.  Runs
+        in the precision the forward was saved in, which must still be the engine's (the library refuses otherwise)."""
         wav = wav.to(self.device, torch.float32).contiguous()
         B, N = wav.shape
 
         gl = [self._grad_in(g) for g in g_layers]
         ge = self._grad_in(g_emb)
-        need = self.lib.nomad_b200_layers_bwd_workspace_bytes(B, N)
+        need = self.lib.nomad_b200_layers_bwd_workspace_bytes_mode(B, N, self._mode)
         if need == 0:
             raise _lib.NomadB200Error(self.lib.nomad_b200_last_error().decode())
         wp, wbytes = self._aligned(self.workspace(need))
@@ -435,7 +437,7 @@ class Engine:
         clean = clean.detach().to(self.device, torch.float32).contiguous()
         assert est.shape == clean.shape
         B, N = est.shape
-        need = self.lib.nomad_b200_loss_workspace_bytes(B, N, 1 if with_grad else 0)
+        need = self.lib.nomad_b200_loss_workspace_bytes_mode(B, N, 1 if with_grad else 0, self._mode)
         if need == 0:
             raise _lib.NomadB200Error(self.lib.nomad_b200_last_error().decode())
         ws = self.workspace(need)

@@ -14,8 +14,9 @@ backward) runs in ``libnomad_b200.so`` on a B200.  Differences that are delibera
   ``keep_state_dict=True``); then ``model``, ``lossnet_layers`` and ``forward`` give ``.grad`` to those parameters from
   any use of their outputs, and edits to them (an optimiser step) reach the device before the next call that runs the
   network;
-* the differentiable calls (``model``, ``lossnet_layers`` and ``forward`` with grad on) always run fp16 tensor-core
-  operands: with ``precision='fp32'`` only the no-grad path is fp32-class.
+* with ``precision='fp32'`` the waveform gradients (``forward`` with grad on, and ``model`` / ``lossnet_layers`` with a
+  waveform that requires grad) are fp32-class like the no-grad path; parameter gradients always run fp16 tensor-core
+  operands (fine-tuning needs ``precision='fp16'``).
 """
 from __future__ import annotations
 
@@ -331,7 +332,8 @@ class Nomad():
         else:
             self.weights_source = "state_dict"
         # arithmetic class of the scoring path: "fp16" (tensor-core operands in fp16, scores within 1e-3 of the
-        # reference's fp32 arithmetic) or "fp32" (split operands, within 1e-5); the loss path always runs "fp16"
+        # reference's fp32 arithmetic) or "fp32" (split operands, within 1e-5); the waveform gradients follow it, parameter
+        # gradients always run "fp16"
         self.precision = precision or os.environ.get("NOMAD_B200_PRECISION", "fp16")
         self.engine = Engine(state_dict, index, self.precision)
         self.state_dict_ref = state_dict if keep_state_dict else None   # fine-tuning (triplet.py) needs the fp32 tensors
